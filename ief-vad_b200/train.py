@@ -4,10 +4,11 @@
 The reference's loop builds its loss in the CALLER from `outputs['logits']` (through CLAS2) and from
 `outputs['image_mu' / 'event_mu' / 'image_logvar' / 'event_logvar']` (cosine / norm regulariser, KL term), so the drop-in
 contract is: the forward's outputs carry a grad_fn, and backward turns the gradients of those outputs into gradients of
-the 78 parameters.  `ForwardFn` is that autograd node.  Its forward is the model composed from the library's stand-alone
-operators (tcgen05 GEMMs with the 3-term bf16 split - gradients need fp32's exponent range, fp16 operands would flush
-them - the 3xTF32 tensor-core training attention of csrc/train_attn_mma.cu, fp32 LayerNorm / fusion kernels) keeping what
-the backward needs; its backward runs entirely in
+the 78 parameters and, when the image / event features require grad, of those inputs (the gradient reaching each
+modality's first attention layer; fp32, cast by autograd to the input's dtype).  `ForwardFn` is that autograd node.
+Its forward is the model composed from the library's stand-alone operators (tcgen05 GEMMs with the 3-term bf16 split -
+gradients need fp32's exponent range, fp16 operands would flush them - the 3xTF32 tensor-core training attention of
+csrc/train_attn_mma.cu, fp32 LayerNorm / fusion kernels) keeping what the backward needs; its backward runs entirely in
 libiefvad.so kernels too: dgrad = linear(dY, W^T), wgrad = linear(dY^T, X^T) on the same tcgen05 GEMM, attention /
 LayerNorm / fusion / ReLU backward kernels of csrc/train.cu.  torch only owns the buffers and the autograd graph.
 
@@ -152,6 +153,7 @@ class ForwardFn(torch.autograd.Function):
         d_mu_i, d_mu_e, d_lv_i, d_lv_e = ops.fuse_bwd(mu_i, mu_e, lv_i, lv_e, dx, g_wi, g_we, g_mu_i, g_mu_e, g_lv_i, g_lv_e,
                                                      cfg["noise_model"], cfg["nu"], cfg["epsilon"])
         # ---- heads, whitening LN and the attention stacks, event modality first (reverse of the forward)
+        d_in = [None, None]                            # gradients of img / ev
         for mi in (1, 0):
             d_mu, d_lv = (d_mu_i, d_lv_i) if mi == 0 else (d_mu_e, d_lv_e)
             base = mi * (6 * L + 6)
@@ -175,9 +177,11 @@ class ForwardFn(torch.autograd.Function):
                 grads[p0] = _wgrad(dqkv, x)
                 grads[p0 + 1] = ops.colsum(dqkv)
                 dxm = _dgrad(dqkv, w_in, resid=dy)     # residual path + attention path
+            if ctx.needs_input_grad[1 + mi]:
+                d_in[mi] = dxm.view(B, T, D)           # fp32; autograd casts it to the input's dtype
         assert not saved
         grads = [g.view_as(p) if g is not None else None for g, p in zip(grads, params)]
-        return (None, None, None, *grads)
+        return (None, *d_in, *grads)
 
 
 class Clas2Fn(torch.autograd.Function):

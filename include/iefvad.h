@@ -319,8 +319,9 @@ int iefvad_bench_gemm(int64_t M, int N, int K, int nsplit, int tile_n, int stage
  * torch/nn/functional.py:6643-6647): out = dropout(softmax(q k^T / sqrt(head_dim))) v per (batch element, head).
  * qkv [B*T, 3*heads*head_dim] (in-projection output, bias added, q unscaled); out [B*T, heads*head_dim]; lse [B, heads, T]
  * = log-sum-exp of the scores (saved for the backward).  The dropout mask is a pure function of (seed, head, query, key):
- * Philox4x32-10 with key = seed and counter = (key >> 2, query, b * heads + h, 0), word (key & 3), dropped when the word
- * < p_drop * 2^32, kept weights scaled by 1 / (1 - p_drop) - NOT PyTorch's generator stream (no kernel can reproduce that),
+ * Philox4x32-10 with key = (seed & 0xffffffff, seed >> 32) and counter = (key >> 2, query, b * heads + h, 0), word (key & 3),
+ * dropped when the word < uint32(double(p_drop) * 2^32), kept weights scaled by 1.f / (1.f - p_drop) (restated in
+ * oracle/iefvad_oracle.py: attention_keep) - NOT PyTorch's generator stream (no kernel can reproduce that),
  * so train-mode parity with the reference is statistical; p_drop = 0 gives the eval-mode arithmetic. */
 int iefvad_attention_train_fwd(const float* qkv, int64_t B, int64_t T, int heads, int head_dim, float p_drop, uint64_t seed,
                                float* out, float* lse, void* stream);

@@ -90,6 +90,44 @@ def multihead_self_attention(x, in_w, in_b, out_w, out_b, heads: int,
 
 
 # --------------------------------------------------------------------------
+# N3: the attention-dropout mask of the training step
+# --------------------------------------------------------------------------
+
+_M32 = np.uint64(0xFFFFFFFF)
+
+
+def philox4x32_10(ctr, key) -> Tuple[np.ndarray, np.ndarray, np.ndarray, np.ndarray]:
+    """Philox4x32-10 (Salmon et al., SC'11; Random123's philox4x32 with 10 rounds) on uint64 arrays holding uint32
+    words.  ctr: four broadcastable integer arrays, key: two integers -> the four output words."""
+    c0, c1, c2, c3 = (np.asarray(c, dtype=np.uint64) & _M32 for c in ctr)
+    k0, k1 = (np.uint64(int(k) & 0xFFFFFFFF) for k in key)
+    for _ in range(10):
+        p0 = np.uint64(0xD2511F53) * c0                          # exact: both factors < 2^32
+        p1 = np.uint64(0xCD9E8D57) * c2
+        c0, c1, c2, c3 = (p1 >> np.uint64(32)) ^ c1 ^ k0, p1 & _M32, (p0 >> np.uint64(32)) ^ c3 ^ k1, p0 & _M32
+        k0 = (k0 + np.uint64(0x9E3779B9)) & _M32
+        k1 = (k1 + np.uint64(0xBB67AE85)) & _M32
+    return c0, c1, c2, c3
+
+
+def attention_keep(seed: int, B: int, H: int, T: int, p: float) -> np.ndarray:
+    """Multiplier of the attention weights under the training step's dropout (include/iefvad.h,
+    iefvad_attention_train_fwd) -> float64 [B, H, T, T] indexed (b, h, query, key): Philox4x32-10 with counter
+    (key >> 2, query, b * H + h, 0) and key (seed & 0xffffffff, seed >> 32), word key & 3; the weight is dropped when
+    that word < uint32(double(float32(p)) * 2^32), kept weights are scaled by 1 / (1 - p) in float32 arithmetic."""
+    seed = int(seed)
+    q = np.arange(T, dtype=np.uint64)[None, :, None]
+    k = np.arange(T, dtype=np.uint64)[None, None, :]
+    bh = np.arange(B * H, dtype=np.uint64)[:, None, None]
+    words = np.stack(np.broadcast_arrays(*philox4x32_10((k >> np.uint64(2), q, bh, 0), (seed, seed >> 32))))
+    word = np.take_along_axis(words, np.broadcast_to(k & np.uint64(3), words.shape[1:])[None].astype(np.int64), 0)[0]
+    pf = np.float32(p)
+    thresh = int(np.float64(pf) * 4294967296.0) if pf > 0 else 0
+    scale = np.float64(np.float32(1) / (np.float32(1) - pf))
+    return np.where(word >= np.uint64(thresh), scale, 0.0).reshape(B, H, T, T)
+
+
+# --------------------------------------------------------------------------
 # A1-A6, A9: the MMFMIL forward
 # --------------------------------------------------------------------------
 
