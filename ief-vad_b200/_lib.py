@@ -22,7 +22,7 @@ if not os.path.exists(LIB_PATH):
 
 lib = C.CDLL(LIB_PATH)
 
-_vp, _i, _i64, _f = C.c_void_p, C.c_int, C.c_int64, C.c_float
+_vp, _i, _i64, _f, _d = C.c_void_p, C.c_int, C.c_int64, C.c_float, C.c_double
 
 _SIGS = {
     "iefvad_abi_version": (_i, []),
@@ -75,6 +75,10 @@ _SIGS = {
     "iefvad_wgrad": (_i, [_vp, _vp, _i64, _i, _i, _f, _vp, _vp]),
     "iefvad_transpose": (_i, [_vp, _i64, _i, _vp, _i64, _vp]),
     "iefvad_clas2_bwd": (_i, [_vp, _vp, _vp, _i64, _vp, _i64, _i64, _i, _vp, _vp, _vp]),
+    "iefvad_train_loss_fwd": (_i, [_vp, _vp, _i64, _vp, _i64, _i64] + [_vp] * 4 + [_i, _d, _d, _d, _vp, _vp, _i]
+                              + [_vp] * 6),
+    "iefvad_train_loss_bwd": (_i, [_vp, _vp, _vp, _i64, _vp, _i64, _i64, _i] + [_vp] * 4 + [_i, _vp, _d, _d, _d]
+                              + [_vp] * 10),
     "iefvad_locmap_proposals": (_i, [_vp, _vp, _vp, _i64, _i, _i] + [_vp] * 5),
     "iefvad_locmap_match": (_i, [_vp, _vp, _vp, _i64, _i, _vp, _vp, _i64, C.c_double, _vp, _vp, _vp]),
     "iefvad_bench_gemm": (_i, [_i64, _i, _i, _i, _i, _i, _i, _i, _vp]),

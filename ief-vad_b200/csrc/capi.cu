@@ -873,6 +873,57 @@ int iefvad_clas2_bwd(const float* logits, const float* means, const float* label
   return clas2_bwd(logits, means, labels, label_stride, idx, int(B), int(T), kmax, g_loss, dlogits, static_cast<cudaStream_t>(stream));
 }
 
+static int train_loss_check(const char* fn, const float* logits, const float* labels, const int32_t* idx, int64_t B, int64_t T,
+                            int kmax, const float* const* wide, int D, double nu) {
+  IEF_CHECK(logits && labels && idx && wide[0] && wide[1] && wide[2] && wide[3], "%s: null argument", fn);
+  IEF_CHECK(B >= 1 && T >= 1 && T <= 16384 && B * T < (1LL << 31), "%s: B=%lld, T=%lld out of range", fn, (long long)B,
+            (long long)T);
+  IEF_CHECK(kmax == int(T / 16 + 1), "%s: kmax must be T / 16 + 1 = %d, got %d", fn, int(T / 16 + 1), kmax);
+  IEF_CHECK(D >= 4 && D % 4 == 0, "%s: D=%d must be a positive multiple of 4", fn, D);
+  for (int i = 0; i < 4; ++i)
+    IEF_CHECK(reinterpret_cast<uintptr_t>(wide[i]) % 16 == 0, "%s: the [B, T, D] tensors must be 16-byte aligned", fn);
+  IEF_CHECK(nu > 0.0, "%s: nu=%g must be positive", fn, nu);
+  return IEFVAD_OK;
+}
+
+int iefvad_train_loss_fwd(const float* logits, const float* labels, int64_t label_stride, const int64_t* lengths, int64_t B,
+                          int64_t T, const float* mu_i, const float* mu_e, const float* logvar_i, const float* logvar_e, int D,
+                          double nu, double reg_weight, double kl_weight, float* means, int32_t* idx, int kmax, double* record,
+                          float* total, float* loss_cls, float* loss_reg, float* loss_kl, void* stream) {
+  const float* wide[4] = {mu_i, mu_e, logvar_i, logvar_e};
+  IEF_TRY(train_loss_check("iefvad_train_loss_fwd", logits, labels, idx, B, T, kmax, wide, D, nu));
+  IEF_CHECK(lengths && means && record && total && loss_cls && loss_reg && loss_kl, "iefvad_train_loss_fwd: null argument");
+  IEF_CHECK(reinterpret_cast<uintptr_t>(record) % 32 == 0, "iefvad_train_loss_fwd: record must be 32-byte aligned");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  Scratch sc(st);
+  void* slabs = nullptr;
+  IEF_TRY(sc.get(&slabs, size_t(2) * train_loss_slabs(B * T) * sizeof(double)));
+  return train_loss_fwd(logits, labels, label_stride, reinterpret_cast<const long long*>(lengths), int(B), int(T), mu_i, mu_e,
+                        logvar_i, logvar_e, D, nu, reg_weight, kl_weight, means, idx, kmax, record, static_cast<double*>(slabs),
+                        total, loss_cls, loss_reg, loss_kl, st);
+}
+
+int iefvad_train_loss_bwd(const float* logits, const float* means, const float* labels, int64_t label_stride, const int32_t* idx,
+                          int64_t B, int64_t T, int kmax, const float* mu_i, const float* mu_e, const float* logvar_i,
+                          const float* logvar_e, int D, const double* record, double nu, double reg_weight, double kl_weight,
+                          const float* g_total, const float* g_cls, const float* g_reg, const float* g_kl, float* d_logits,
+                          float* d_mu_i, float* d_mu_e, float* d_logvar_i, float* d_logvar_e, void* stream) {
+  const float* wide[4] = {mu_i, mu_e, logvar_i, logvar_e};
+  IEF_TRY(train_loss_check("iefvad_train_loss_bwd", logits, labels, idx, B, T, kmax, wide, D, nu));
+  IEF_CHECK(means && record && d_logits && d_mu_i && d_mu_e && d_logvar_i && d_logvar_e, "iefvad_train_loss_bwd: null argument");
+  const float* outs[4] = {d_mu_i, d_mu_e, d_logvar_i, d_logvar_e};
+  for (int i = 0; i < 4; ++i)
+    IEF_CHECK(reinterpret_cast<uintptr_t>(outs[i]) % 16 == 0, "iefvad_train_loss_bwd: the gradients must be 16-byte aligned");
+  IEF_CHECK(reinterpret_cast<uintptr_t>(record) % 32 == 0, "iefvad_train_loss_bwd: record must be 32-byte aligned");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  Scratch sc(st);
+  void* g_cls_total = nullptr;
+  IEF_TRY(sc.get(&g_cls_total, sizeof(float)));
+  return train_loss_bwd(logits, means, labels, label_stride, idx, int(B), int(T), kmax, mu_i, mu_e, logvar_i, logvar_e, D, record,
+                        nu, reg_weight, kl_weight, g_total, g_cls, g_reg, g_kl, static_cast<float*>(g_cls_total), d_logits,
+                        d_mu_i, d_mu_e, d_logvar_i, d_logvar_e, st);
+}
+
 // ------------------------------------------------------------------------------------------------ localisation mAP (N5)
 
 int iefvad_locmap_proposals(const float* pred, const int64_t* vid_off, const int32_t* vid_len, int64_t num_videos,

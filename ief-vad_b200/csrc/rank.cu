@@ -469,10 +469,10 @@ int mil_topk_mean(const float* x, const long long* lengths, long long B, long lo
 }
 
 int clas2(const float* logits, const float* labels, long long label_stride, const long long* lengths, long long B,
-          long long T, float* means, float* loss, cudaStream_t stream) {
+          long long T, float* means, float* loss, cudaStream_t stream, int* idx, int kmax) {
   IEF_CHECK(logits && labels && lengths && means && loss, "clas2: null argument");
   IEF_CHECK(B >= 1, "clas2: empty batch");
-  IEF_TRY(mil_topk_mean(logits, lengths, B, T, 1, means, nullptr, 0, stream));
+  IEF_TRY(mil_topk_mean(logits, lengths, B, T, 1, means, idx, kmax, stream));
   bce_kernel<<<1, 256, 0, stream>>>(means, labels, label_stride, int(B), loss);
   count_launches(1);
   IEF_CUDA(cudaGetLastError());

@@ -8,9 +8,10 @@ namespace iefvad {
 int mil_topk_mean(const float* x, const long long* lengths, long long B, long long T, int apply_sigmoid, float* mean,
                   int* idx, int kmax, cudaStream_t stream);
 
-// train/loss.py:18-30 (CLAS2): per-row means + scalar BCE loss against 1 - labels[:, 0]
+// train/loss.py:18-30 (CLAS2): per-row means + scalar BCE loss against 1 - labels[:, 0]; idx (optional, [B, kmax]):
+// the top-k positions as in mil_topk_mean, for the backward
 int clas2(const float* logits, const float* labels, long long label_stride, const long long* lengths, long long B,
-          long long T, float* means, float* loss, cudaStream_t stream);
+          long long T, float* means, float* loss, cudaStream_t stream, int* idx = nullptr, int kmax = 0);
 
 // stable descending argsort of fp32 scores (== np.argsort(-s, kind="stable")); keys_sorted optional
 int sort_scores(const float* scores, long long n, int* order, uint32_t* keys_sorted, cudaStream_t stream);

@@ -39,4 +39,18 @@ int transpose_split(const float* src, long long rows, int cols, bf16* dst_hi, bf
 int clas2_bwd(const float* logits, const float* means, const float* labels, long long label_stride, const int* idx, int B, int T,
               int kmax, const float* g_loss, float* dlogits, cudaStream_t stream);
 
+// Training objective of train/ucf_train.py:73-102 (train_loss.cu): CLAS2 + cosine / norm regulariser + StudentT KL.
+// record: [B*T, 4] float64 for the backward; slab_scratch: 2 * train_loss_slabs(B*T) doubles; D % 4 == 0, 16-byte aligned rows.
+int train_loss_slabs(long long rows);
+int train_loss_fwd(const float* logits, const float* labels, long long label_stride, const long long* lengths, int B, int T,
+                   const float* mu_i, const float* mu_e, const float* lv_i, const float* lv_e, int D, double nu, double reg_w,
+                   double kl_w, float* means, int* idx, int kmax, double* record, double* slab_scratch, float* total,
+                   float* loss_cls, float* loss_reg, float* loss_kl, cudaStream_t stream);
+// g_*: device scalars, null = 0; g_cls_scratch: one device float (CLAS2's coefficient g_total + g_cls)
+int train_loss_bwd(const float* logits, const float* means, const float* labels, long long label_stride, const int* idx, int B,
+                   int T, int kmax, const float* mu_i, const float* mu_e, const float* lv_i, const float* lv_e, int D,
+                   const double* record, double nu, double reg_w, double kl_w, const float* g_total, const float* g_cls,
+                   const float* g_reg, const float* g_kl, float* g_cls_scratch, float* d_logits, float* d_mu_i, float* d_mu_e,
+                   float* d_lv_i, float* d_lv_e, cudaStream_t stream);
+
 }  // namespace iefvad

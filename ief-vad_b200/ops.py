@@ -330,3 +330,65 @@ def clas2_bwd(logits, means, labels, idx, g_loss=None):
         _lib.check(_lib.lib.iefvad_clas2_bwd(x.data_ptr(), means.data_ptr(), labels.data_ptr(), labels.stride(0),
                                              idx.data_ptr(), B, T, idx.shape[1], _lib.ptr(g), out.data_ptr(), _stream(x)))
     return out
+
+
+def _check_objective_inputs(logits, labels, lengths, wide):
+    for name, t in zip(("logits", "labels", "lengths", "image_mu", "event_mu", "image_logvar", "event_logvar"),
+                       (logits, labels, lengths, *wide)):
+        if not t.is_cuda:
+            raise RuntimeError(f"train_loss: {name} must be a CUDA tensor (the B200 path has no CPU fallback), got {t.device}")
+    shape = wide[0].shape
+    if wide[0].dim() != 3 or any(t.shape != shape for t in wide[1:]):
+        raise RuntimeError("train_loss: image_mu, event_mu, image_logvar and event_logvar must share one [B, T, D] shape, "
+                           f"got {[tuple(t.shape) for t in wide]}")
+    if tuple(logits.shape) != (shape[0], shape[1], 1):
+        raise RuntimeError(f"train_loss: logits must be [B, T, 1] = {[shape[0], shape[1], 1]}, got {list(logits.shape)}")
+    if labels.dim() != 2 or labels.shape[0] != shape[0] or lengths.numel() != shape[0]:
+        raise RuntimeError(f"train_loss: labels must be [B, C] and lengths [B] with B = {shape[0]}, "
+                           f"got {list(labels.shape)} and {list(lengths.shape)}")
+
+
+def train_loss_fwd(logits, labels, lengths, mu_i, mu_e, lv_i, lv_e, nu: float, reg_weight: float = 1.0,
+                   kl_weight: float = 1.0):
+    """Loss of train/ucf_train.py:73-102 (CLAS2 + cosine / norm regulariser + StudentT KL, iefvad_train_loss_fwd).
+    logits [B, T, 1], mu_* / lv_* [B, T, D], labels [B, C], lengths [B] -> (total, classification, regulariser, kl) as
+    0-dim fp32 device tensors, and (means, idx, record), what train_loss_bwd needs."""
+    _check_objective_inputs(logits, labels, lengths, (mu_i, mu_e, lv_i, lv_e))
+    B, T, D = mu_i.shape
+    x = _f32c(logits, "train_loss").reshape(B, T)
+    labels = _f32c(labels, "train_loss")
+    lengths = lengths.to(dtype=torch.int64).contiguous()
+    wide = [_f32c(t, "train_loss") for t in (mu_i, mu_e, lv_i, lv_e)]
+    kmax = T // 16 + 1
+    dev = x.device
+    means = torch.empty(B, dtype=torch.float32, device=dev)
+    idx = torch.empty((B, kmax), dtype=torch.int32, device=dev)
+    record = torch.empty((B * T, 4), dtype=torch.float64, device=dev)
+    scalars = [torch.empty((), dtype=torch.float32, device=dev) for _ in range(4)]
+    with torch.cuda.device(dev):
+        _lib.check(_lib.lib.iefvad_train_loss_fwd(x.data_ptr(), labels.data_ptr(), labels.stride(0), lengths.data_ptr(), B, T,
+                                                  *[t.data_ptr() for t in wide], D, float(nu), float(reg_weight),
+                                                  float(kl_weight), means.data_ptr(), idx.data_ptr(), kmax, record.data_ptr(),
+                                                  *[t.data_ptr() for t in scalars], _stream(x)))
+    return tuple(scalars), (means, idx, record)
+
+
+def train_loss_bwd(logits, labels, mu_i, mu_e, lv_i, lv_e, saved, nu: float, reg_weight: float = 1.0, kl_weight: float = 1.0,
+                   g_total=None, g_cls=None, g_reg=None, g_kl=None):
+    """Backward of train_loss_fwd: gradients of g_total total + g_cls classification + g_reg regulariser + g_kl kl
+    (device scalars, None = 0) -> (d_logits [B, T, 1], d_mu_i, d_mu_e, d_lv_i, d_lv_e [B, T, D]), fp32."""
+    means, idx, record = saved
+    B, T, D = mu_i.shape
+    x = _f32c(logits, "train_loss_bwd").reshape(B, T)
+    labels = _f32c(labels, "train_loss_bwd")
+    wide = [_f32c(t, "train_loss_bwd") for t in (mu_i, mu_e, lv_i, lv_e)]
+    gs = [_f32c(g, "train_loss_bwd").reshape(()) if g is not None else None for g in (g_total, g_cls, g_reg, g_kl)]
+    d_logits = torch.empty((B, T, 1), dtype=torch.float32, device=x.device)
+    outs = [torch.empty((B, T, D), dtype=torch.float32, device=x.device) for _ in range(4)]
+    with torch.cuda.device(x.device):
+        _lib.check(_lib.lib.iefvad_train_loss_bwd(x.data_ptr(), means.data_ptr(), labels.data_ptr(), labels.stride(0),
+                                                  idx.data_ptr(), B, T, idx.shape[1], *[t.data_ptr() for t in wide], D,
+                                                  record.data_ptr(), float(nu), float(reg_weight), float(kl_weight),
+                                                  *[_lib.ptr(g) for g in gs], d_logits.data_ptr(),
+                                                  *[t.data_ptr() for t in outs], _stream(x)))
+    return (d_logits, *outs)

@@ -199,3 +199,24 @@ class Clas2Fn(torch.autograd.Function):
         logits, means, labels, idx = ctx.saved_tensors
         d = ops.clas2_bwd(logits, means, labels, idx, g_loss)
         return d.view_as(logits), None, None
+
+
+class TrainLossFn(torch.autograd.Function):
+    """train/ucf_train.py:73-102 with a gradient: (logits, image_mu, event_mu, image_logvar, event_logvar, labels, lengths,
+    nu, reg_weight, kl_weight) -> (total, classification, regulariser, kl), 0-dim fp32 device tensors.  Forward and backward
+    are the kernels of csrc/train_loss.cu plus CLAS2's; the gradients of the five tensor inputs go on to
+    ForwardFn.backward unchanged."""
+
+    @staticmethod
+    def forward(ctx, logits, mu_i, mu_e, lv_i, lv_e, labels, lengths, nu, reg_weight, kl_weight):
+        scalars, saved = ops.train_loss_fwd(logits, labels, lengths, mu_i, mu_e, lv_i, lv_e, nu, reg_weight, kl_weight)
+        ctx.save_for_backward(logits, mu_i, mu_e, lv_i, lv_e, labels, *saved)
+        ctx.consts = (nu, reg_weight, kl_weight)
+        ctx.set_materialize_grads(False)          # an unused output's gradient stays None: the kernel reads NULL as 0
+        return scalars
+
+    @staticmethod
+    def backward(ctx, g_total, g_cls, g_reg, g_kl):
+        logits, mu_i, mu_e, lv_i, lv_e, labels, *saved = ctx.saved_tensors
+        grads = ops.train_loss_bwd(logits, labels, mu_i, mu_e, lv_i, lv_e, saved, *ctx.consts, g_total, g_cls, g_reg, g_kl)
+        return (*grads, None, None, None, None, None)

@@ -353,6 +353,32 @@ int iefvad_transpose(const float* src, int64_t rows, int cols, float* dst, int64
  * per-row means of iefvad_mil_topk_mean(apply_sigmoid = 1); g_loss: device scalar (NULL = 1). */
 int iefvad_clas2_bwd(const float* logits, const float* means, const float* labels, int64_t label_stride, const int32_t* idx,
                      int64_t B, int64_t T, int kmax, const float* g_loss, float* dlogits, void* stream);
+/* Training objective of the reference's loop (train/ucf_train.py:73-102, the loss it builds from the module's outputs), with
+ * mu_i, mu_e, lv_i, lv_e the [B, T, D] fp32 outputs image_mu, event_mu, image_logvar, event_logvar:
+ *   loss_cls = CLAS2(logits, labels, lengths)                               (train/loss.py:18-30, as iefvad_clas2)
+ *   cos      = cosine_similarity(normalize(mu_i), normalize(mu_e)) per row  (:75-82)
+ *   loss_reg = mean(1 - cos) + mean |norm(mu_i) - norm(mu_e)|               (:75-82)
+ *   c = log(nu / (nu + 1)), eli = lv_i + c, ele = lv_e + c                  (:93-98)
+ *   loss_kl  = -0.5 mean(1 + eli - mu_i^2 - exp(eli)) - 0.5 mean(1 + ele - mu_e^2 - exp(ele))
+ *   total    = loss_cls + reg_weight loss_reg + kl_weight loss_kl
+ * The means run over all B*T rows (B*T*D elements for the KL term), pad rows beyond `lengths` included, as in the loop.
+ * torch's edge rules hold: normalize divides by max(|x|, 1e-12), cosine_similarity by max(|x|, 1e-8) per factor; the
+ * gradients of |x| at 0 and of a norm at the zero vector are 0; exp overflows to +inf as fp32 does.  Reductions are in
+ * float64 in a fixed order (run-to-run identical, independent of the device's SM count).  D % 4 == 0, the wide tensors
+ * 16-byte aligned, kmax = T / 16 + 1.
+ * Forward: means [B], idx [B, kmax] (top-k positions, as iefvad_mil_topk_mean) and record [B*T, 4] (float64, 32-byte
+ * aligned) are kept for the backward; total, loss_cls, loss_reg, loss_kl are device scalars.  4 kernel launches. */
+int iefvad_train_loss_fwd(const float* logits, const float* labels, int64_t label_stride, const int64_t* lengths, int64_t B,
+                          int64_t T, const float* mu_i, const float* mu_e, const float* logvar_i, const float* logvar_e, int D,
+                          double nu, double reg_weight, double kl_weight, float* means, int32_t* idx, int kmax, double* record,
+                          float* total, float* loss_cls, float* loss_reg, float* loss_kl, void* stream);
+/* Backward: d_logits [B, T] and d_mu_i, d_mu_e, d_logvar_i, d_logvar_e [B*T, D] (fp32) of
+ * g_total total + g_cls loss_cls + g_reg loss_reg + g_kl loss_kl; each g_* is a device scalar, NULL = 0.  2 launches. */
+int iefvad_train_loss_bwd(const float* logits, const float* means, const float* labels, int64_t label_stride, const int32_t* idx,
+                          int64_t B, int64_t T, int kmax, const float* mu_i, const float* mu_e, const float* logvar_i,
+                          const float* logvar_e, int D, const double* record, double nu, double reg_weight, double kl_weight,
+                          const float* g_total, const float* g_cls, const float* g_reg, const float* g_kl, float* d_logits,
+                          float* d_mu_i, float* d_mu_e, float* d_logvar_i, float* d_logvar_e, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Temporal-localisation mAP (SURVEY 8f row N5) - replaces getDetectionMAP / getLocMAP / nms, train/metrics.py:19-136
