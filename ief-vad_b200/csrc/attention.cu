@@ -2,15 +2,13 @@
 // no mask, keys = all T rows of the batch element including zero pads; q pre-scaled by d_h^-1/2,
 // torch/nn/functional.py:6632) - softmax(Q K^T) V without ever materialising the [B,H,T,T] scores.
 //
-// attn_tc : tcgen05 flash-style kernel.  One CTA = 128 query rows of one (batch, head); key blocks of 128
-//           stream through a 2-stage TMA ring; S = Q.K^T lands in one of two 128-column TMEM buffers, the
+// attn_tc : tcgen05 flash-style kernel.  One CTA = 128 query rows of one (batch, head); key blocks of 64
+//           stream through a 2-stage TMA ring; S = Q.K^T lands in one of two 64-column TMEM buffers, the
 //           four softmax warps (thread == query row, so row max / sum need no shuffles) turn it into bf16 P in
 //           128B-swizzled smem, P.V^T-major accumulates a per-block O in TMEM which the same threads fold into
 //           fp32 registers with the online-softmax rescale.  Optional additive mask / key-padding mask serve
 //           the model/module.py block (D4).
 // attn_simt : fp32 reference plan (one warp per query row), same math in IEEE fp32.
-#include <cstdlib>
-
 #include "attention.cuh"
 #include "common.cuh"
 #include "tensormap.cuh"
@@ -20,6 +18,10 @@ namespace iefvad {
 namespace {
 
 constexpr int QB = 128;   // query rows per CTA
+// Keys per block.  64 rather than 128 halves every per-CTA resource (104 KB smem, 256 TMEM columns) so that TWO CTAs
+// share an SM and one CTA's softmax overlaps the other's MMAs / loads (T_c = 256 has only two 128-key blocks to
+// pipeline within a CTA); two CTAs per SM measured faster at every T (7.75 vs 7.95 ms on config 5).
+constexpr int KB = 64;
 constexpr float kLog2e = 1.4426950408889634f;
 
 // 2^x on the SFU in one instruction (ex2.approx.ftz: 2 ulp, flushes denormal results - they vanish in the 16-bit P)
@@ -29,10 +31,7 @@ __device__ __forceinline__ float fast_exp2(float x) {
   return y;
 }
 
-// KB = keys per block.  KB = 64 halves every per-CTA resource (104 KB smem, 256 TMEM columns) so that TWO CTAs share
-// an SM and one CTA's softmax overlaps the other's MMAs / loads - the short-sequence configuration (T_c = 256 has
-// only two 128-key blocks to pipeline within a CTA); KB = 128 halves the per-key synchronisation for long T.
-template <int DH, int DHP, int KB>
+template <int DH, int DHP>
 struct AttnCfg {
   static constexpr uint32_t kQBytes = QB * DHP * 2;
   static constexpr uint32_t kKBytes = KB * DHP * 2;
@@ -45,18 +44,18 @@ struct AttnCfg {
   static constexpr uint32_t kOffBar = kOffP + kPBytes;
   static constexpr size_t kSmemBytes = 1024 + kOffBar + 256;
   static constexpr uint32_t kOffO = 2 * KB;              // TMEM: S0 [0,KB) S1 [KB,2KB) O [2KB, 2KB+DH)
-  static constexpr uint32_t kTmemCols = (2 * KB + 128 <= 256) ? 256 : 512;
-  static constexpr int kCtasPerSm = (KB == 64) ? 2 : 1;
+  static constexpr uint32_t kTmemCols = 256;
+  static_assert(kOffO + DH <= kTmemCols, "S0, S1 and O fit the TMEM allocation");
 };
 
-template <int DH, int DHP, int KB>
-__global__ void __launch_bounds__(192, AttnCfg<DH, DHP, KB>::kCtasPerSm)
+template <int DH, int DHP>
+__global__ void __launch_bounds__(192, 2)
 attn_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                const __grid_constant__ CUtensorMap tmVt, bf16* __restrict__ out, int ldo, int T, int H,
                const float* __restrict__ attn_mask /* [T,T] additive or null */,
                const uint8_t* __restrict__ key_pad /* [B,T] 1 = ignore, or null */, int fp16, int out_fp16,
                const int* __restrict__ row_out) {
-  using Cfg = AttnCfg<DH, DHP, KB>;
+  using Cfg = AttnCfg<DH, DHP>;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + Cfg::kOffBar);
@@ -310,12 +309,12 @@ attn_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ 
   }
 }
 
-template <int DH, int DHP, int KB>
+template <int DH, int DHP>
 int launch_attn_tc(const AttnTcArgs& a, cudaStream_t stream) {
-  using Cfg = AttnCfg<DH, DHP, KB>;
+  using Cfg = AttnCfg<DH, DHP>;
   static bool attr_set = false;
   if (!attr_set) {
-    IEF_CUDA(cudaFuncSetAttribute(attn_tc_kernel<DH, DHP, KB>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    IEF_CUDA(cudaFuncSetAttribute(attn_tc_kernel<DH, DHP>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   static_cast<int>(Cfg::kSmemBytes)));
     attr_set = true;
   }
@@ -325,8 +324,8 @@ int launch_attn_tc(const AttnTcArgs& a, cudaStream_t stream) {
   IEF_TRY(make_tmap_3d(&tk, a.k, DHP, a.T, BH, uint64_t(DHP) * 2, uint64_t(a.T) * DHP * 2, 64, KB, 1));
   IEF_TRY(make_tmap_3d(&tv, a.vt, a.T, DH, BH, uint64_t(a.Tpad) * 2, uint64_t(DH) * a.Tpad * 2, 64, DH, 1));
   dim3 grid((a.T + QB - 1) / QB, a.H, a.B);
-  attn_tc_kernel<DH, DHP, KB><<<grid, 192, Cfg::kSmemBytes, stream>>>(tq, tk, tv, a.out, a.ldo, a.T, a.H, a.attn_mask,
-                                                                  a.key_pad, a.fp16, a.out_fp16, a.row_out);
+  attn_tc_kernel<DH, DHP><<<grid, 192, Cfg::kSmemBytes, stream>>>(tq, tk, tv, a.out, a.ldo, a.T, a.H, a.attn_mask,
+                                                              a.key_pad, a.fp16, a.out_fp16, a.row_out);
   count_launches(1);
   IEF_CUDA(cudaGetLastError());
   return IEFVAD_OK;
@@ -418,12 +417,8 @@ int attn_tc(const AttnTcArgs& a, cudaStream_t stream) {
   if (attn_short_supported(a)) return attn_short(a, stream);
   if (attn_long_supported(a)) return attn_long(a, stream);
   IEF_CHECK(a.B <= 65535 && a.H <= 65535, "attn_tc: B=%d / H=%d exceed the grid limits", a.B, a.H);
-  static const int env_kb = [] { const char* e = getenv("IEFVAD_ATTN_KB"); return e ? atoi(e) : 0; }();   // tuning knob
-  const int kb = a.key_block ? a.key_block : (env_kb ? env_kb : 64);      // two CTAs per SM measured faster at every T (7.75 vs 7.95 ms on config 5)
-  IEF_CHECK(kb == 64 || kb == 128, "attn_tc: key_block must be 64 or 128");
-#define IEF_ATTN(DH_, DHP_)                                                      \
-  if (a.dh == DH_ && a.dhp == DHP_)                                              \
-    return kb == 64 ? launch_attn_tc<DH_, DHP_, 64>(a, stream) : launch_attn_tc<DH_, DHP_, 128>(a, stream);
+#define IEF_ATTN(DH_, DHP_) \
+  if (a.dh == DH_ && a.dhp == DHP_) return launch_attn_tc<DH_, DHP_>(a, stream);
   IEF_ATTN(96, 128)
   IEF_ATTN(64, 64)
   IEF_ATTN(128, 128)

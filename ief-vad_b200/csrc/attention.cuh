@@ -19,19 +19,18 @@ struct AttnTcArgs {
   // {first row, rows (<= 256), valid rows, multiplicity of the last row as a key (0 = none)} for n_chunks row ranges
   const int* items = nullptr;          // device, int4 per chunk
   int n_chunks = 0;
-  int key_block = 0;                   // 0 = heuristic (64 keys per block up to T = 2048, else 128), or 64 / 128
 };
 
 int attn_tc(const AttnTcArgs& a, cudaStream_t stream);
 
 // T <= 256 without masks (every chunk the reference's callers produce): persistent kernel, P kept in TMEM
-// (attention_short.cu).  attn_tc dispatches here when attn_short_supported(a); IEFVAD_ATTN_SHORT=0 disables it.
+// (attention_short.cu).  attn_tc dispatches here when attn_short_supported(a).
 // T > 256 without masks: persistent two-tile kernel, single-pass softmax with integer (power-of-two) maxima, O
-// accumulated in TMEM (attention_long.cu); IEFVAD_ATTN_LONG=0 falls back to the flash-style attn_tc_kernel.
+// accumulated in TMEM (attention_long.cu).  Masked attention, and any other shape neither kernel takes, runs the
+// flash-style attn_tc_kernel.
 bool attn_long_supported(const AttnTcArgs& a);
 int attn_long(const AttnTcArgs& a, cudaStream_t stream);
 bool attn_short_supported(const AttnTcArgs& a);
-bool attn_short_enabled();      // IEFVAD_ATTN_SHORT != 0: the short kernel (and with it unpadded q / k rows) may be used
 int attn_short(const AttnTcArgs& a, cudaStream_t stream);
 
 // fp32 plan: qkv fp32 [B*T, 3*H*dh] (bias added, q unscaled) -> out fp32 [B*T, H*dh]

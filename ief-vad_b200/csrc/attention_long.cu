@@ -348,8 +348,7 @@ int launch_attn_long(const AttnTcArgs& a, int num_sms, cudaStream_t stream) {
 }  // namespace
 
 bool attn_long_supported(const AttnTcArgs& a) {
-  static const int env_off = [] { const char* e = getenv("IEFVAD_ATTN_LONG"); return (e && atoi(e) == 0) ? 1 : 0; }();
-  return !env_off && a.T > 256 && !a.attn_mask && !a.key_pad && !a.items;
+  return a.T > 256 && !a.attn_mask && !a.key_pad && !a.items;
 }
 
 int attn_long(const AttnTcArgs& a, cudaStream_t stream) {

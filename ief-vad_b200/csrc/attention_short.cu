@@ -12,9 +12,6 @@
 // Nothing of P ever touches shared memory; Q / K / V^T buffers are released by tcgen05.commit as soon as their last
 // MMA retires, so the next item's TMA loads overlap this item's softmax.  TMEM columns of tile t (base 256 t):
 //   [0, 64) P keys 0..127 | [64, 64 + DH) O | [192, 256) P keys 128..255    (all inside the dead S columns).
-#include <cstdio>
-#include <cstdlib>
-
 #include "attention.cuh"
 #include "common.cuh"
 #include "tensormap.cuh"
@@ -57,11 +54,8 @@ template <int DH, int DHP>
 __global__ void __launch_bounds__(kThreads, 1)
 attn_short_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                   const __grid_constant__ CUtensorMap tmVt, bf16* __restrict__ out, int ldo, int T, int H, int n_items,
-                  int fp16, int out_fp16, const int* __restrict__ row_out, const int4* __restrict__ items,
-                  long long* __restrict__ trace) {
+                  int fp16, int out_fp16, const int* __restrict__ row_out, const int4* __restrict__ items) {
   using Cfg = ShortCfg<DH, DHP>;
-  // debug timeline (IEFVAD_ATTN_TRACE): CTA 0 records clock64() of pipeline events, 16 slots per item
-  auto mark = [&](int it, int ev) { if (trace && blockIdx.x == 0 && it < 64) trace[it * 16 + ev] = clock64(); };
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + Cfg::kOffBar);
@@ -161,13 +155,11 @@ attn_short_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
         const Item d = get_item(item);
         mbar_wait(&s_full[0], ph);                // S_a(i) retired
         mbar_wait(v_empty, ph ^ 1);               // P.V of item i-1 retired
-        mark(it, 1);
         mbar_arrive_expect_tx(v_full, uint32_t(nv(d)) * Cfg::kVSub);
         for (int c = 0; c < nv(d); ++c)
           tma_load_3d(&tmVt, v_full, smem + Cfg::kOffV + c * Cfg::kVSub, d.row0 + c * 64, 0, d.z);
         if (item + step < n_items) {
           mbar_wait(qk_empty, ph);                // every S MMA of item i retired: Q / K buffers are free
-          mark(it + 1, 0);
           load_qk(get_item(item + step));
           if (item + 2 * step < n_items) prefetch(get_item(item + 2 * step));
         }
@@ -213,14 +205,11 @@ attn_short_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
         const uint32_t ph = it & 1;
         const bool act_b = get_item(item).rows > 128;
         mbar_wait(qk_full, ph);
-        mark(it, 2);
         mbar_wait(&s_empty[0], ph ^ 1);         // tile 0's columns (P and O of the previous item) have been read out
-        mark(it, 3);
         tc_fence_after();
         issue_s(0);
         if (pend_b) {
           mbar_wait(&p_full[1], nb_pv & 1);
-          mark(it - 1, 7);
           tc_fence_after();
           issue_pv(1);                          // previous item, still on the previous V
           tc_commit(v_empty);
@@ -228,16 +217,13 @@ attn_short_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
         }
         if (act_b) {
           mbar_wait(&s_empty[1], (nb_s & 1) ^ 1);
-          mark(it, 4);
           tc_fence_after();
           issue_s(1);
           ++nb_s;
         }
         tc_commit(qk_empty);                    // Q and K may be overwritten once the S MMAs have retired
         mbar_wait(v_full, ph);
-        mark(it, 5);
         mbar_wait(&p_full[0], ph);
-        mark(it, 6);
         tc_fence_after();
         issue_pv(0);
         if (!act_b) tc_commit(v_empty);
@@ -263,9 +249,8 @@ attn_short_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
     // exchange slots: xch[((kind * 2 + parity) * 2 + tile) * 2 + half][row]
     auto slot = [&](int kind, uint32_t ph, int half) { return xch + ((((kind * 2 + int(ph)) * 2 + t) * 2 + half) << 7) + r; };
 
-    int it = 0;
     uint32_t n_mine = 0;                            // items this tile has processed (tile 1 skips the short ones)
-    for (int item = blockIdx.x; item < n_items; item += gridDim.x, ++it) {
+    for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
       const Item d = get_item(item);
       if (t == 1 && d.rows <= 128) continue;
       const uint32_t ph = n_mine & 1;
@@ -276,7 +261,6 @@ attn_short_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
       const float lnm = d.mult > 0 ? __logf(float(d.mult)) : 0.f;
       const int plain_end = padkey >= 0 ? padkey : Tk;   // 32-key chunks that end at or before this key need no masking
       mbar_wait(&s_full[t], ph);
-      if (threadIdx.x == 0 || threadIdx.x == 256) mark(it, 8 + t);
       tc_fence_after();
       // ---- pass 1: row max over this thread's 128 keys.  Only the 32-key chunk that holds the last key needs per-key
       // masking (keys >= Tk are not there; the last key may carry a multiplicity); chunks before it are plain, chunks
@@ -306,7 +290,6 @@ attn_short_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
       named_bar_sync(1 + t, 256);
       mx = fmaxf(mx, *slot(0, ph, hf ^ 1));          // key 0 is always valid, so the row max is finite
       const float mscaled = mx * kLog2e;
-      if (threadIdx.x == 0) mark(it, 10);
       // ---- pass 2: P = exp(S - max) -> packed 16-bit pairs over the S columns already consumed.  Half 0 walks its
       // chunks upwards and packs downwards into [0, 64); half 1 walks downwards and packs into [192, 256).
       float lsum = 0.f;
@@ -350,10 +333,8 @@ attn_short_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
       tmem_st_wait();
       tc_fence_before();
       mbar_arrive(&p_full[t]);
-      if (threadIdx.x == 0) mark(it, 11);
       // ---- O = P.V: this thread normalises and stores columns [hf DH/2, hf DH/2 + DH/2) of its row
       mbar_wait(&o_full[t], ph);
-      if (threadIdx.x == 0 || threadIdx.x == 256) mark(it, 12 + t);
       tc_fence_after();
       named_bar_sync(1 + t, 256);
       const float inv = 1.f / (lsum + *slot(1, ph, hf ^ 1));
@@ -363,7 +344,6 @@ attn_short_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
       tmem_ld_wait();
       tc_fence_before();
       mbar_arrive(&s_empty[t]);
-      if (threadIdx.x == 0) mark(it, 14);
       long long ro = (long long)d.orow0 + tq;
       if (tq < Tk && row_out) ro = __ldg(row_out + ro);
       if (tq < Tk && ro >= 0) {
@@ -407,43 +387,18 @@ int launch_attn_short(const AttnTcArgs& a, int num_sms, cudaStream_t stream) {
   IEF_TRY(make_tmap_3d(&tv, a.vt, a.T, DH, BH, uint64_t(a.Tpad) * 2, uint64_t(DH) * a.Tpad * 2, 64, DH, 1));
   const int n_items = a.items ? a.n_chunks * a.H : int(BH);
   const int grid = n_items < num_sms ? n_items : num_sms;
-  static const bool want_trace = getenv("IEFVAD_ATTN_TRACE") != nullptr;
-  static long long* trace = nullptr;
-  static int traced = 0;
-  if (want_trace && !trace) {
-    IEF_CUDA(cudaMallocManaged(&trace, 64 * 16 * sizeof(long long)));
-    for (int i = 0; i < 64 * 16; ++i) trace[i] = 0;
-  }
   attn_short_kernel<DH, DHP><<<grid, kThreads, Cfg::kSmemBytes, stream>>>(tq, tk, tv, a.out, a.ldo, a.T, a.H, n_items,
-                                                                         a.fp16, a.out_fp16, a.row_out, reinterpret_cast<const int4*>(a.items),
-                                                                         (want_trace && traced < 3) ? trace : nullptr);
+                                                                         a.fp16, a.out_fp16, a.row_out, reinterpret_cast<const int4*>(a.items));
   count_launches(1);
   IEF_CUDA(cudaGetLastError());
-  if (want_trace && traced < 3 && n_items >= 8 * grid) {
-    ++traced;
-    IEF_CUDA(cudaStreamSynchronize(stream));
-    // columns: 0 qk_empty seen (producer) 1 v_empty seen 2 qk_full seen (MMA) 3/4 s_empty[0/1] seen 5 v_full seen
-    // 6/7 p_full[0/1] seen 8/9 s_full[0/1] seen (softmax) 10 row max known 11 P written 12/13 o_full[0/1] seen 14 O read
-    for (int it = 2; it < 8; ++it) {
-      fprintf(stderr, "[attn_short trace] item %d:", it);
-      for (int e = 0; e < 15; ++e) fprintf(stderr, " %lld", trace[it * 16 + e] - trace[2 * 16 + 2]);
-      fprintf(stderr, "\n");
-    }
-  }
   return IEFVAD_OK;
 }
 
 }  // namespace
 
-bool attn_short_enabled() {
-  static const int env_off = [] { const char* e = getenv("IEFVAD_ATTN_SHORT"); return (e && atoi(e) == 0) ? 1 : 0; }();
-  return !env_off;
-}
-
 bool attn_short_supported(const AttnTcArgs& a) {
-  const int env_off = attn_short_enabled() ? 0 : 1;
   if (a.items) return !a.attn_mask && !a.key_pad;      // ragged items exist only here (every item <= 256 rows)
-  return !env_off && a.T <= 256 && !a.attn_mask && !a.key_pad && uint64_t(a.B) * a.H < (1ull << 31);
+  return a.T <= 256 && !a.attn_mask && !a.key_pad && uint64_t(a.B) * a.H < (1ull << 31);
 }
 
 int attn_short(const AttnTcArgs& a, cudaStream_t stream) {

@@ -2,8 +2,6 @@
 #include "../../include/iefvad.h"
 
 #include <cmath>
-#include <cstdio>
-#include <cstdlib>
 #include <new>
 #include <string>
 #include <vector>
@@ -180,15 +178,13 @@ static int forward_from_host(iefvad_model* m, const void* img_host, const void* 
   const int64_t cap_rows = m->impl.max_rows;
   std::vector<int64_t> partsB;
   {
-    static const double env_first = [] { const char* e = getenv("IEFVAD_HOST_PART_FIRST"); return e ? atof(e) : 0.0; }();
-    static const double env_growth = [] { const char* e = getenv("IEFVAD_HOST_PART_GROWTH"); return e ? atof(e) : 0.0; }();
     const bool ragged_in = chunk_start_dev != nullptr;
-    double growth = env_growth > 1.0 ? env_growth : (ragged_in ? 3.0 : 1.4);
-    double want = env_first > 0.0 ? env_first : double(m->host_part_rows) / (ragged_in ? 8.0 : 4.0);
+    double growth = ragged_in ? 3.0 : 1.4;
+    double want = double(m->host_part_rows) / (ragged_in ? 8.0 : 4.0);
     // Back-to-back calls: the previous call's last part is still computing, so this call's copy hides behind it
     // whatever its size - the whole batch then travels as ONE part into the other input buffer (full GEMM grids; a
     // small first part only pays when the device is idle at the call).
-    if (env_first <= 0.0 && m->host_seq > 0 && m->ev_consumed[(m->host_seq - 1) & 1] &&
+    if (m->host_seq > 0 && m->ev_consumed[(m->host_seq - 1) & 1] &&
         cudaEventQuery(m->ev_consumed[(m->host_seq - 1) & 1]) == cudaErrorNotReady) {
       (void)cudaGetLastError();            // cudaErrorNotReady is a status, not a failure: keep it out of the next check
       want = double(B * T);
@@ -204,14 +200,6 @@ static int forward_from_host(iefvad_model* m, const void* img_host, const void* 
       partsB.push_back(pb);
       left -= pb;
       want *= growth;
-    }
-  }
-  {
-    static const bool debug = getenv("IEFVAD_HOST_DEBUG") != nullptr;      // print the part schedule of every call
-    if (debug) {
-      fprintf(stderr, "[iefvad] host forward %lld x %lld rows, parts:", (long long)B, (long long)T);
-      for (int64_t pb : partsB) fprintf(stderr, " %lld", (long long)(pb * T));
-      fprintf(stderr, "\n");
     }
   }
   int64_t maxB = 0;

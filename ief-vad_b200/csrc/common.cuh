@@ -152,12 +152,6 @@ __device__ __forceinline__ void tma_load_3d(const CUtensorMap* m, uint64_t* bar,
 }
 
 // L2 prefetch of a tensor box: the data starts moving from HBM long before a shared-memory buffer is free to take it
-__device__ __forceinline__ void tma_prefetch_2d(const CUtensorMap* m, int c0, int c1) {
-  asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];"
-               :
-               : "l"(reinterpret_cast<uint64_t>(m)), "r"(c0), "r"(c1)
-               : "memory");
-}
 __device__ __forceinline__ void tma_prefetch_3d(const CUtensorMap* m, int c0, int c1, int c2) {
   asm volatile("cp.async.bulk.prefetch.tensor.3d.L2.global.tile [%0, {%1, %2, %3}];"
                :

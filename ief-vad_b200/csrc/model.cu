@@ -322,9 +322,8 @@ int Model::forward(const void* img, const void* ev, int in_dtype, long long B, l
     // Out-projection + residual + LayerNorm(s) as one kernel (outproj_ln.cu) under the all-fp16 plan: y never reaches HBM.
     // Every encoder stage then works in encoder-row space (all rows, or the packed rows of the pad de-duplication); the
     // LAST layer's kernel writes its result through the inverse row map, i.e. directly as compact valid rows.
-    static const bool ln_fused_off = [] { const char* e = getenv("IEFVAD_OUTPROJ_LN"); return e && atoi(e) == 0; }();   // A/B knob
     const bool ln_fused = !fp32_plan && (plan & PLAN_FP16_ATTENTION) && (plan & PLAN_FP16_HEADS) && D == kOutprojLnDim && L >= 1 &&
-                          outproj_ln_mode != 0 && !ln_fused_off &&
+                          outproj_ln_mode != 0 &&
                           (in_dtype == IEFVAD_DT_F16 || !(vr && vr->chunk_start && vr->chunk_valid));
     // Pad de-duplication (valid-rows mode, fp16 inputs, fp16 encoder, chunks of <= 256 rows): the zero-pad rows of a
     // chunk are identical, and stay identical to each other through every row-wise stage and through attention, so
@@ -332,9 +331,8 @@ int Model::forward(const void* img, const void* ev, int in_dtype, long long B, l
     // gets + log mult, which is exactly what mult equal keys contribute to the softmax).  The encoder then works on
     // Me = sum(valid + 1) packed rows instead of B * T; chunks without valid rows vanish.  Same arithmetic as the
     // dense forward up to the rounding of that one key's probability.
-    static const bool dedup_off = [] { const char* e = getenv("IEFVAD_DEDUP"); return e && atoi(e) == 0; }();
     const bool dedup = direct_compact && !fp32_plan && (plan & PLAN_FP16_ATTENTION) && in_dtype == IEFVAD_DT_F16 &&
-                       T <= 256 && T % 32 == 0 && pad_dedup && !dedup_off;
+                       T <= 256 && T % 32 == 0 && pad_dedup;
     long long Me = M;                       // rows the encoder stages before the valid-row cut run on
     if (dedup) {
       items_host.clear();
@@ -384,9 +382,8 @@ int Model::forward(const void* img, const void* ev, int in_dtype, long long B, l
     if (dedup && n_items == 0) continue;                 // no valid row in this slab
     // heads of both modalities + fusion as one kernel (heads_fuse.cu) when the caller keeps neither mu / logvar nor the fusion
     // weights (the evaluation forward) and the refinement chain takes the fp16 pair
-    static const bool heads_fuse_off = [] { const char* e = getenv("IEFVAD_HEADS_FUSE"); return e && atoi(e) == 0; }();   // A/B knob
     const bool hf = ln_fused && vr && heads_outputs_unused && !w_i && !eval_wi_mean && (plan & PLAN_FP16_REFINE) && R > 0 &&
-                    D == kHeadsFuseDim && L >= 2 && heads_fuse_mode != 0 && !heads_fuse_off;
+                    D == kHeadsFuseDim && L >= 2 && heads_fuse_mode != 0;
     if (ln_fused) {
       IEF_TRY(ln_scratch.reserve(outproj_ln_scratch_bytes(Me)));
       if (!ln_ident.p) {
@@ -402,8 +399,7 @@ int Model::forward(const void* img, const void* ev, int in_dtype, long long B, l
     }
     // q / k rows: d_h padded to a multiple of 64 for the 128-byte-swizzled kernels; the short-sequence kernel takes
     // 32-column chunks (64-byte swizzle), so d_h = 96 goes unpadded there (a quarter less q / k traffic)
-    static const bool qk_pad = [] { const char* e = getenv("IEFVAD_QK_PAD"); return e && atoi(e) != 0; }();   // A/B knob
-    const int dhq = (!fp32_plan && T <= 256 && dh % 32 == 0 && attn_short_enabled() && !qk_pad) ? dh : dhp;
+    const int dhq = (!fp32_plan && T <= 256 && dh % 32 == 0) ? dh : dhp;
     for (int m = 0; m < 2; ++m) {
       const bool ragged = vr && vr->chunk_start && vr->chunk_valid;
       const uint8_t* in = static_cast<const uint8_t*>(inputs[m]) + (ragged ? 0 : size_t(row0) * D * in_esize);

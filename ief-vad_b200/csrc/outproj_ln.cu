@@ -28,7 +28,6 @@
 //   mean(u^2), mean(u b1) follow from the sums of w d, w^2 d, w^2 d^2, w b1 d (d = y - shift) gathered in pass 1 once mu
 //   is known.
 // Per-row results do not depend on the tile position or the batch size.
-#include <cstdlib>
 #include <cstring>
 
 #include "outproj_ln.cuh"
@@ -74,7 +73,6 @@ struct LnParams {
   int groups;          // blocks in flight (grid = groups * kNT pairs)
   int stages;
   uint32_t warp_bytes;
-  int dbg;             // IEFVAD_OUTPROJ_LN_DBG bits (timing experiments only): 1 = no residual k-blocks, 2 = no epilogue math, 8 = L2 prefetch
   const int* row_map;
   __half* out_hi;      // row-mapped stores only
 };
@@ -135,7 +133,7 @@ outproj_ln_kernel(const __grid_constant__ CUtensorMap ta, const __grid_constant_
   const int grp = blockIdx.x / kClusterCtas;
   const int n_blk = int(crank >> 1);
   constexpr int kResStages = kKBRes * (1 + RES_LO) / 2;              // two 64-column residual boxes per ring stage
-  const int kKB = (p.dbg & 1) ? kKBMain : kKBMain + kResStages;
+  constexpr int kKB = kKBMain + kResStages;
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&ta);
@@ -181,12 +179,9 @@ outproj_ln_kernel(const __grid_constant__ CUtensorMap ta, const __grid_constant_
           uint8_t* sa = smem + size_t(s) * kStageBytes;
           const uint32_t lead_full = mapa_shared(smem_u32(&full[s]), lead);
           if (rank == 0) mbar_arrive_expect_tx(&full[s], 2 * kStageBytes);
-          const int m_next = m_blk + 2 * p.groups;
-          const bool pf = (p.dbg & 8) && mp + p.groups < p.num_mp;      // A/B knob: L2 prefetch of the next tile's A boxes (measured no gain)
           if (kb < kKBMain) {
             tma_load_2d_cg2(&ta, lead_full, sa, kb * BK, m_blk * BM);
             tma_load_2d_cg2(&tw, lead_full, sa + kABytes, kb * BK, n_blk * BN + int(rank) * (BN / 2));
-            if (pf) tma_prefetch_2d(&ta, kb * BK, m_next * BM);
           } else {
             // residual stage: two A boxes x[rows, tile columns kk * 64 ..] (the W operand is the resident identity)
 #pragma unroll
@@ -195,7 +190,6 @@ outproj_ln_kernel(const __grid_constant__ CUtensorMap ta, const __grid_constant_
               const int kk = kr & (kKBRes - 1);
               const CUtensorMap* tr = (RES_LO && kr >= kKBRes) ? &trl : &trh;
               tma_load_2d_cg2(tr, lead_full, sa + b * kABytes, n_blk * BN + kk * BK, m_blk * BM);
-              if (pf) tma_prefetch_2d(tr, n_blk * BN + kk * BK, m_next * BM);
             }
           }
           if (++s == STAGES) { s = 0; ph ^= 1; }
@@ -314,12 +308,6 @@ outproj_ln_kernel(const __grid_constant__ CUtensorMap ta, const __grid_constant_
       mbar_wait(&tfull[team], aph);
       tc_fence_after();
       float v[32];
-      if (p.dbg & 2) {
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive_cluster(mapa_shared(smem_u32(&tempty[team]), lead));
-        continue;
-      }
 
       // ---- pass 1: y = acc (= ctx . Wo^T + x) + bias, back into TMEM; shifted sums of this thread's 128 columns
       float shift = 0.f, S1 = 0.f, S2 = 0.f, A1 = 0.f, A2 = 0.f, A3 = 0.f, A4 = 0.f;
@@ -535,9 +523,6 @@ int outproj_ln(const OutprojLnArgs& a, int num_sms, cudaStream_t stream) {
   const uint32_t fixed = 1024 + kIBytes + kEpiWarps * p.warp_bytes + kParamBytes + kConstBytes + xch_bytes + kBarBytes;
   p.stages = int((kSmemLimit - fixed) / kStageBytes);
   if (p.stages > kMaxStages) p.stages = kMaxStages;
-  static const int dbg = [] { const char* e = getenv("IEFVAD_OUTPROJ_LN_DBG"); return e ? atoi(e) : 0; }();
-  p.dbg = dbg & 15;
-  if ((dbg >> 4) > 0 && (dbg >> 4) < p.stages) p.stages = dbg >> 4;     // bits 4+: cap on the operand ring depth
   IEF_CHECK(p.stages >= 2, "outproj_ln: no room for the operand ring");
   const size_t smem_bytes = fixed + size_t(p.stages) * kStageBytes;
   p.row_map = a.row_map;

@@ -26,8 +26,6 @@
 //   GEMM2 accumulator: [384, 512)  (= upper half of chunk 2, free once read out); h occupies [0, 384)
 // Warp roles (320 threads): warp 0 = TMA producer, warp 1 = MMA issuer (leader CTA only), warps 2..9 = epilogue, two warps
 // per TMEM lane quarter, each taking half of the columns.
-#include <cstdio>
-#include <cstdlib>
 #include <cstring>
 
 #include "common.cuh"
@@ -134,20 +132,7 @@ struct RefineParams {
   int steps;
   float lambda;
   int num_tiles;           // tiles of 256 rows
-  long long* trace;        // debug (IEFVAD_REFINE_TRACE): cycles CTA 0 spent waiting, per role and barrier
 };
-
-// accumulate the cycles a wait took when tracing (one thread per role)
-#define TWAIT(acc, stmt)                         \
-  do {                                           \
-    if (tr) {                                    \
-      const long long _t0 = clock64();           \
-      stmt;                                      \
-      acc += clock64() - _t0;                    \
-    } else {                                     \
-      stmt;                                      \
-    }                                            \
-  } while (0)
 
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
 refine_chain_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmW1,
@@ -202,9 +187,6 @@ refine_chain_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_consta
   if (warp == 0) {
     // ===================== TMA producer =====================
     if (lane == 0) {
-      const bool tr = p.trace != nullptr && blockIdx.x == 0;
-      long long w_empty = 0, w_flag = 0;
-      const long long t_begin = clock64();
       int st = 0;
       uint32_t ph = 0;
       for (int u = pair; u < units; u += npairs) {
@@ -212,18 +194,16 @@ refine_chain_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_consta
         const int row0 = (t * 2 + int(rank)) * BM;
         if (s > 0) {
           // unit (s - 1, t) - some pair's work ~T units ago - has written this tile's fp16(x): wait for all its 16 warps
-          const long long t0 = tr ? clock64() : 0;
           uint32_t spins = 0;
           while (ld_acquire_gpu(p.done + t) < 16 * s) {
             __nanosleep(64);
             if (++spins > (1u << 24)) __trap();
           }
-          if (tr) w_flag += clock64() - t0;
           fence_proxy_async_all();       // the rows were written by generic stores; the TMA reads below are async-proxy
         }
         for (int c = 0; c < NCH1; ++c)
           for (int kb = 0; kb < NKB; ++kb) {
-            TWAIT(w_empty, mbar_wait(&empty[st], ph ^ 1));
+            mbar_wait(&empty[st], ph ^ 1);
             if (rank == 0) mbar_arrive_expect_tx(&full[st], 2 * kStage);
             uint8_t* dst = smem + size_t(st) * kStage;
             tma_load_2d_cg2(&tmX, lead(&full[st]), dst, kb * BK, row0);
@@ -232,7 +212,7 @@ refine_chain_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_consta
           }
         for (int n = 0; n < NCH2; ++n)
           for (int kq = 0; kq < 3; ++kq) {
-            TWAIT(w_empty, mbar_wait(&empty[st], ph ^ 1));
+            mbar_wait(&empty[st], ph ^ 1);
             if (rank == 0) mbar_arrive_expect_tx(&full[st], 2 * kStage);
             uint8_t* dst = smem + size_t(st) * kStage;
 #pragma unroll
@@ -241,29 +221,24 @@ refine_chain_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_consta
             if (++st == STAGES) { st = 0; ph ^= 1; }
           }
       }
-      if (tr) { p.trace[0] = clock64() - t_begin; p.trace[1] = w_empty; p.trace[2] = w_flag; }
     }
   } else if (warp == 1) {
     // ===================== MMA issuer (leader CTA) =====================
     if (lane == 0 && rank == 0) {
       const uint32_t idesc1 = make_idesc_f16(256, 256);
       const uint32_t idesc2 = make_idesc_f16(256, 128);
-      const bool tr = p.trace != nullptr && blockIdx.x == 0;
-      long long w_up = 0, w_full1 = 0, w_hrdy = 0, w_a2 = 0, w_full2 = 0, t_g1 = 0, t_g2 = 0;
-      const long long t_begin = clock64();
       int st = 0;
       uint32_t ph = 0, n_up = 0, n_a2 = 0;
       int it = 0;
       for (int u = pair; u < units; u += npairs, ++it) {
         // ---- GEMM1: accumulator of chunk c at columns [128 c, 128 c + 256)
-        const long long tg1 = tr ? clock64() : 0;
         for (int c = 0; c < NCH1; ++c) {
-          if (c > 0) { TWAIT(w_up, mbar_wait(upfree, n_up & 1u)); ++n_up; }     // chunk c - 1's upper half is in registers
-          if (c == 2 && it > 0) { TWAIT(w_a2, mbar_wait(a2free, n_a2 & 1u)); ++n_a2; }   // previous unit's last GEMM2 chunk too
+          if (c > 0) { mbar_wait(upfree, n_up & 1u); ++n_up; }     // chunk c - 1's upper half is in registers
+          if (c == 2 && it > 0) { mbar_wait(a2free, n_a2 & 1u); ++n_a2; }   // previous unit's last GEMM2 chunk too
           tc_fence_after();
           const uint32_t d_tmem = tmem_base + uint32_t(128 * c);
           for (int kb = 0; kb < NKB; ++kb) {
-            TWAIT(w_full1, mbar_wait(&full[st], ph));
+            mbar_wait(&full[st], ph);
             tc_fence_after();
             const uint32_t sa = smem_u32(smem + size_t(st) * kStage);
             const uint64_t da = make_smem_desc_sw128(sa), db = make_smem_desc_sw128(sa + kABox);
@@ -276,17 +251,15 @@ refine_chain_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_consta
           tc_commit_cg2(accfull, 3);
         }
         // ---- GEMM2: accumulator at [384, 512) (chunk 2's upper half), A = h chunk kq at columns [128 kq, 128 kq + 128)
-        const long long tg2 = tr ? clock64() : 0;
-        t_g1 += tg2 - tg1;
-        TWAIT(w_up, mbar_wait(upfree, n_up & 1u));
+        mbar_wait(upfree, n_up & 1u);
         ++n_up;
         const uint32_t d2 = tmem_base + 384u;
         for (int n = 0; n < NCH2; ++n) {
-          if (n > 0) { TWAIT(w_a2, mbar_wait(a2free, n_a2 & 1u)); ++n_a2; }
+          if (n > 0) { mbar_wait(a2free, n_a2 & 1u); ++n_a2; }
           tc_fence_after();
           for (int kq = 0; kq < 3; ++kq) {
-            TWAIT(w_full2, mbar_wait(&full[st], ph));
-            if (n == 0) TWAIT(w_hrdy, mbar_wait(&hrdy[kq], uint32_t(it) & 1u));
+            mbar_wait(&full[st], ph);
+            if (n == 0) mbar_wait(&hrdy[kq], uint32_t(it) & 1u);
             tc_fence_after();
             const uint32_t sb = smem_u32(smem + size_t(st) * kStage);
 #pragma unroll
@@ -300,11 +273,6 @@ refine_chain_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_consta
           }
           tc_commit_cg2(a2full, 3);
         }
-        if (tr) t_g2 += clock64() - tg2;
-      }
-      if (tr) {
-        p.trace[4] = clock64() - t_begin; p.trace[5] = w_up; p.trace[6] = w_full1; p.trace[7] = w_hrdy; p.trace[8] = w_a2;
-        p.trace[9] = w_full2; p.trace[10] = t_g1; p.trace[11] = t_g2;
       }
     }
   } else {
@@ -316,9 +284,6 @@ refine_chain_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_consta
     const float nlam = -p.lambda;
     const uint32_t Hb = smem_u32(smem + kOffStageBuf + size_t(warp - 2) * kWarpStage);      // shared-space addresses
     const uint32_t Lb = Hb + 4096;
-    const bool tr = p.trace != nullptr && blockIdx.x == 0 && warp == 2;
-    long long w_acc = 0, w_a2f = 0;
-    const long long t_begin = clock64();
     uint32_t n_acc = 0, n_a2 = 0;
     int publish_t = -1;                           // tile whose step this warp has finished but not yet published
     auto publish = [&]() {                        // this warp's share of a step of tile publish_t is in global memory
@@ -361,7 +326,7 @@ refine_chain_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_consta
       const float* b1 = p.b1[s];
 #pragma unroll 1
       for (int c = 0; c < NCH1; ++c) {
-        TWAIT(w_acc, mbar_wait(accfull, n_acc & 1u));
+        mbar_wait(accfull, n_acc & 1u);
         ++n_acc;
         tc_fence_after();
         float v[64];
@@ -410,7 +375,7 @@ refine_chain_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_consta
       for (int n = 0; n < NCH2; ++n) {
         const int col0 = n * 128 + 64 * hf;
         // the accumulator first: the tensor pipe idles until every warp of the pair has read it out
-        TWAIT(w_a2f, mbar_wait(a2full, n_a2 & 1u));
+        mbar_wait(a2full, n_a2 & 1u);
         ++n_a2;
         tc_fence_after();
         float v[64];
@@ -497,7 +462,6 @@ refine_chain_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_consta
     }
     publish();
     if (lane == 0) bulk_wait_all<0>();            // Ob must outlive the last stores
-    if (tr && lane == 0) { p.trace[12] = clock64() - t_begin; p.trace[13] = w_acc; p.trace[14] = w_a2f; }
   }
 
   tc_fence_before();
@@ -513,9 +477,6 @@ refine_chain_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_consta
 size_t refine_chain_scratch_bytes(long long M) { return size_t((M + 255) / 256) * sizeof(int) + 16; }
 
 bool refine_chain_preferred(long long M, int num_sms) {
-  static const int mode = [] { const char* e = getenv("IEFVAD_REFINE_FUSED"); return e ? atoi(e) : -1; }();
-  if (mode == 0) return false;
-  if (mode == 1) return true;
   // a unit (256 rows, one step) keeps one CTA pair busy: enough tiles to give every pair work within a step
   return (M + 255) / 256 >= num_sms / 2;
 }
@@ -551,14 +512,6 @@ int refine_chain(const RefineChainArgs& a, int num_sms, cudaStream_t stream) {
   const int pairs = num_sms / 2;
   const long long units = (long long)p.num_tiles * a.steps;
   const int grid = int(units < pairs ? units : pairs) * 2;
-  static const bool want_trace = getenv("IEFVAD_REFINE_TRACE") != nullptr;
-  static long long* trace = nullptr;
-  static int traced = 0;
-  if (want_trace && !trace) {
-    IEF_CUDA(cudaMallocManaged(&trace, 32 * sizeof(long long)));
-    for (int i = 0; i < 32; ++i) trace[i] = 0;
-  }
-  p.trace = (want_trace && traced < 3) ? trace : nullptr;
   static bool attr_set = false;
   if (!attr_set) {
     IEF_CUDA(cudaFuncSetAttribute(refine_chain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(kSmemBytes)));
@@ -567,14 +520,6 @@ int refine_chain(const RefineChainArgs& a, int num_sms, cudaStream_t stream) {
   refine_chain_kernel<<<grid, kThreads, kSmemBytes, stream>>>(tx, tw1, tw2, tsh, tsl, tso, p);
   IEF_CUDA(cudaGetLastError());
   count_launches(1);
-  if (p.trace) {
-    ++traced;
-    IEF_CUDA(cudaStreamSynchronize(stream));
-    fprintf(stderr, "[refine trace] M=%lld tiles=%d grid=%d | producer: total %lld, wait empty %lld, wait step flag %lld | mma: total %lld, "
-            "wait upfree %lld full(gemm1) %lld hrdy %lld a2free %lld full(gemm2) %lld, phases gemm1 %lld gemm2 %lld | epilogue warp 2: "
-            "total %lld, wait accfull %lld a2full %lld\n", a.M, p.num_tiles, grid, trace[0], trace[1], trace[2], trace[4], trace[5],
-            trace[6], trace[7], trace[8], trace[9], trace[10], trace[11], trace[12], trace[13], trace[14]);
-  }
   return IEFVAD_OK;
 }
 

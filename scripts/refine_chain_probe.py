@@ -1,5 +1,5 @@
 """Times the refinement chain alone (fused persistent kernel vs per-step GEMMs) on the bench-size valid-row count through
-the evaluation forward's profile classes; IEFVAD_REFINE_TRACE=1 prints the fused kernel's wait-time breakdown."""
+the evaluation forward's profile classes."""
 import os
 import sys
 
