@@ -61,6 +61,7 @@ _SIGS = {
     "iefvad_graph_convolution": (_i, [_vp] * 4 + [_i, _vp, _vp, _i64, _i, _i, _i, _i, _vp, _vp]),
     "iefvad_distance_scan": (_i, [_vp, _i64, _i, _i, _vp, _vp]),
     "iefvad_transformer": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _i, _vp, _vp]),
+    "iefvad_clip_visual": (_i, [_vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _i, _vp, _vp]),
     "iefvad_process_split": (_i, [_vp, _i, _vp, _i64, _i, _i, _vp, _i64, _vp, _i, _vp]),
     "iefvad_process_feat": (_i, [_vp, _i, _vp, _i64, _i, _i, _vp, _vp, _i, _vp]),
     "iefvad_attention_train_fwd": (_i, [_vp, _i64, _i64, _i, _i, _f, C.c_uint64, _vp, _vp, _vp]),

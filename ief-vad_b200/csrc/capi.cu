@@ -7,6 +7,7 @@
 #include <vector>
 
 #include "attention.cuh"
+#include "clip.cuh"
 #include "elementwise.cuh"
 #include "event.cuh"
 #include "gemm.cuh"
@@ -609,6 +610,23 @@ int iefvad_transformer(const float* x, const float* const* params, int layers, i
     blocks[i] = ResBlockParams{p[0], p[1], p[2], p[3], p[4], p[5], p[6], p[7], p[8], p[9], p[10], p[11]};
   }
   return transformer(x, blocks.data(), layers, L, N, D, heads, attn_mask, key_padding_mask, plan, out, sms,
+                     static_cast<cudaStream_t>(stream));
+}
+
+// ------------------------------------------------------------------------------------------------ row N4 (CLIP encoder)
+
+int iefvad_clip_visual(const void* x, int dtype, int N, int resolution, int patch, int width, int layers, int heads,
+                       int output_dim, const float* const* params, int plan, float* out, void* stream) {
+  IEF_CHECK(params != nullptr, "iefvad_clip_visual: null parameter table");
+  IEF_CHECK(layers >= 0 && layers <= 64, "iefvad_clip_visual: layers %d outside [0, 64]", layers);
+  std::vector<ResBlockParams> blocks(static_cast<size_t>(layers));
+  for (int i = 0; i < layers; ++i) {
+    const float* const* p = params + 5 + 12 * i;
+    blocks[i] = ResBlockParams{p[0], p[1], p[2], p[3], p[4], p[5], p[6], p[7], p[8], p[9], p[10], p[11]};
+  }
+  const float* const* tail = params + 5 + 12 * layers;
+  const ClipVisualParams cp{params[0], params[1], params[2], params[3], params[4], blocks.data(), tail[0], tail[1], tail[2]};
+  return clip_visual(x, dtype, N, resolution, patch, width, layers, heads, output_dim, cp, plan, out,
                      static_cast<cudaStream_t>(stream));
 }
 

@@ -11,29 +11,11 @@
 #include "attention.cuh"
 #include "elementwise.cuh"
 #include "gemm.cuh"
+#include "scratch.cuh"
 
 namespace iefvad {
 
 namespace {
-
-struct Scratch {   // stream-ordered temporaries
-  cudaStream_t s;
-  std::vector<void*> ptrs;
-  explicit Scratch(cudaStream_t st) : s(st) { keep_async_pool(); }
-  ~Scratch() {
-    for (void* p : ptrs) cudaFreeAsync(p, s);
-  }
-  template <typename T>
-  int get(T** out, size_t count, bool zero = false) {
-    void* p = nullptr;
-    const size_t bytes = (count ? count : 1) * sizeof(T);
-    IEF_CUDA(cudaMallocAsync(&p, bytes, s));
-    ptrs.push_back(p);
-    if (zero) IEF_CUDA(cudaMemsetAsync(p, 0, bytes, s));
-    *out = static_cast<T*>(p);
-    return IEFVAD_OK;
-  }
-};
 
 inline int round_up(int v, int a) { return (v + a - 1) / a * a; }
 
@@ -194,16 +176,19 @@ simadj_softmax_kernel(const float* __restrict__ sim, int ld, const float* __rest
 }
 
 // ------------------------------------------------------------------------------------------------ copies
-// dst[r, c] = (r < rows && c < cols) ? src[r, c] : 0  for r < rows_p, c < cols_p (fp32 and/or bf16 hi / lo copies)
+// dst[r, c] = (r < rows && c < cols) ? src[r, c] : 0  for r < rows_p, c < cols_p (fp32 and/or bf16 hi / lo copies;
+// hi_fp16: dst_hi receives fp16 instead, no lo)
 __global__ void __launch_bounds__(256)
 pad2d_kernel(const float* __restrict__ src, int rows, int cols, long long ld_src, int rows_p, int cols_p,
-             float* __restrict__ dst_f32, bf16* __restrict__ dst_hi, bf16* __restrict__ dst_lo) {
+             float* __restrict__ dst_f32, bf16* __restrict__ dst_hi, bf16* __restrict__ dst_lo, int hi_fp16) {
   const long long total = (long long)rows_p * cols_p;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
     const int r = int(i / cols_p), c = int(i - (long long)r * cols_p);
     const float v = (r < rows && c < cols) ? src[r * ld_src + c] : 0.f;
     if (dst_f32) dst_f32[i] = v;
-    if (dst_hi) {
+    if (dst_hi && hi_fp16) {
+      reinterpret_cast<__half*>(dst_hi)[i] = __float2half_rn(v);
+    } else if (dst_hi) {
       bf16 h, l;
       split_bf16(v, h, l);
       dst_hi[i] = h;
@@ -281,7 +266,8 @@ int blocks_for(long long n, int num_sms) {
   return int(b < 1 ? 1 : (b > cap ? cap : b));
 }
 
-// one operand / result in the representation the plan needs: fp32 (plan < 0) or bf16 hi (+ lo when plan == 1)
+// one operand / result in the representation the plan needs: fp32 (plan < 0), bf16 hi (+ lo when plan == 1) or fp16
+// in `hi` (plan == 2)
 struct Mat {
   float* f = nullptr;
   bf16* hi = nullptr;
@@ -303,12 +289,12 @@ int gemm_plan(int plan, const Mat& A, const Mat& W, int M, int N, int K, EpiPara
               cudaStream_t st) {
   if (dst) {
     if (plan < 0) { ep.out_f32 = dst->f; ep.ld_f32 = dst->ld; }
-    else { ep.out_hi = dst->hi; ep.out_lo = dst->lo; ep.ld_bf = dst->ld; }
+    else { ep.out_hi = dst->hi; ep.out_lo = dst->lo; ep.ld_bf = dst->ld; ep.hi_fp16 = (plan == 2); }
   }
   if (plan < 0) return gemm_simt(A.f, A.ld, W.f, W.ld, M, N, K, ep, st);
   GemmTcArgs g;
   g.A_hi = A.hi; g.A_lo = A.lo; g.W_hi = W.hi; g.W_lo = W.lo;
-  g.M = M; g.N = N; g.K = K; g.lda = A.ld; g.ldw = W.ld; g.nsplit = (plan == 1) ? 3 : 1;
+  g.M = M; g.N = N; g.K = K; g.lda = A.ld; g.ldw = W.ld; g.nsplit = (plan == 1) ? 3 : 1; g.fp16 = (plan == 2);
   return gemm_tc(g, ep, num_sms, st);
 }
 
@@ -317,7 +303,7 @@ int to_mat(Scratch& sc, Mat* m, const float* src, int rows, int cols, long long 
            int num_sms, cudaStream_t st) {
   IEF_TRY(alloc_mat(sc, m, size_t(rows_p), cols_p, plan));
   pad2d_kernel<<<blocks_for((long long)rows_p * cols_p, num_sms), 256, 0, st>>>(src, rows, cols, ld_src, rows_p, cols_p,
-                                                                                 m->f, m->hi, m->lo);
+                                                                                 m->f, m->hi, m->lo, plan == 2);
   count_launches(1);
   IEF_CUDA(cudaGetLastError());
   return IEFVAD_OK;
@@ -438,7 +424,7 @@ int graph_convolution(const float* x, const float* adj, const float* wt, const f
       if (plan < 0) resid = xb.f;
       else {
         if (!xpad) IEF_TRY(sc.get(&xpad, size_t(Tp) * Din));
-        pad2d_kernel<<<blocks_for((long long)Tp * Din, num_sms), 256, 0, st>>>(xb32, T, Din, Din, Tp, Din, xpad, nullptr, nullptr);
+        pad2d_kernel<<<blocks_for((long long)Tp * Din, num_sms), 256, 0, st>>>(xb32, T, Din, Din, Tp, Din, xpad, nullptr, nullptr, 0);
         count_launches(1);
         resid = xpad;
       }
@@ -483,25 +469,17 @@ int graph_convolution(const float* x, const float* adj, const float* wt, const f
   return IEFVAD_OK;
 }
 
-int transformer(const float* x, const ResBlockParams* blocks, int layers, int L, int N, int D, int heads,
-                const float* attn_mask, const uint8_t* key_pad, int plan, float* out, int num_sms, cudaStream_t st) {
-  IEF_CHECK(x && out && blocks && layers >= 0 && L >= 0 && N >= 0, "transformer: bad argument");
-  IEF_CHECK(plan >= -1 && plan <= 1, "transformer: plan must be -1, 0 or 1");
-  IEF_CHECK(D > 0 && D % 128 == 0 && heads > 0 && D % heads == 0, "transformer: width %d must be a multiple of 128 and of heads=%d", D, heads);
-  const int dh = D / heads;
-  IEF_CHECK(dh == 32 || dh == 64 || dh == 96 || dh == 128, "transformer: head dim %d unsupported (32, 64, 96, 128)", dh);
-  IEF_CHECK(N <= 65535, "transformer: batch %d exceeds the grid limit", N);
-  if (L == 0 || N == 0) return IEFVAD_OK;
+int transformer_blocks(float* xa, const ResBlockParams* blocks, int layers, int L, int N, int D, int heads,
+                       const float* attn_mask, const uint8_t* key_pad, int plan, int num_sms, cudaStream_t st) {
+  if (layers == 0 || L == 0 || N == 0) return IEFVAD_OK;
   const long long M = (long long)N * L;
-  IEF_CHECK(M < (1LL << 31), "transformer: too many rows");
+  const int dh = D / heads;
   const int dhp = (dh + 63) / 64 * 64, Tpad = (L + 7) / 8 * 8;
   const float qscale = 1.0f / sqrtf(float(dh));
+  const int f16 = (plan == 2);
   Scratch sc(st);
-  float *xa, *xb;                                 // residual stream, batch-first [N, L, D]
-  IEF_TRY(sc.get(&xa, size_t(M) * D));
+  float* xb;                                      // second residual buffer: x alternates xa -> xb -> xa in each block
   IEF_TRY(sc.get(&xb, size_t(M) * D));
-  swap01_kernel<<<blocks_for(M * D / 4, num_sms), 256, 0, st>>>(x, L, N, D / 4, xa);   // [L, N, D] -> [N, L, D]
-  count_launches(1);
   Mat h, ctx, u;
   IEF_TRY(alloc_mat(sc, &h, size_t(M), D, plan));
   IEF_TRY(alloc_mat(sc, &ctx, size_t(M), D, plan == 1 ? 0 : plan));
@@ -525,7 +503,7 @@ int transformer(const float* x, const ResBlockParams* blocks, int layers, int L,
     IEF_TRY(to_mat(sc, &wf, p.fc_w, 4 * D, D, D, 4 * D, D, plan, num_sms, st));
     IEF_TRY(to_mat(sc, &wp, p.proj_w, D, 4 * D, 4 * D, D, 4 * D, plan, num_sms, st));
     // x = x + attn(ln_1(x))   (module.py:41)
-    IEF_TRY(layernorm(xa, M, D, p.ln1_w, p.ln1_b, nullptr, nullptr, 1e-5f, h.f, h.hi, h.lo, num_sms, st));
+    IEF_TRY(layernorm(xa, M, D, p.ln1_w, p.ln1_b, nullptr, nullptr, 1e-5f, h.f, h.hi, h.lo, num_sms, st, f16));
     if (plan < 0) {
       EpiParams e1;
       e1.bias = p.in_b; e1.out_f32 = qkv32; e1.ld_f32 = 3 * D;
@@ -533,20 +511,21 @@ int transformer(const float* x, const ResBlockParams* blocks, int layers, int L,
       IEF_TRY(attn_simt(qkv32, ctx.f, N, L, heads, dh, attn_mask, key_pad, st));
     } else {
       EpiParams e1;
-      e1.mode = EPI_QKV; e1.bias = p.in_b; e1.q = q; e1.k = k; e1.vt = vt;
+      e1.mode = EPI_QKV; e1.bias = p.in_b; e1.q = q; e1.k = k; e1.vt = vt; e1.hi_fp16 = f16;
       e1.T = L; e1.H = heads; e1.dh = dh; e1.dhp = dhp; e1.Tpad = Tpad; e1.D = D; e1.qscale = qscale;
       IEF_TRY(gemm_plan(plan, h, wi, int(M), 3 * D, D, e1, nullptr, num_sms, st));
       AttnTcArgs at;
       at.q = q; at.k = k; at.vt = vt; at.out = ctx.hi; at.ldo = D;
       at.B = N; at.T = L; at.H = heads; at.dh = dh; at.dhp = dhp; at.Tpad = Tpad;
       at.attn_mask = attn_mask; at.key_pad = key_pad;
+      at.fp16 = f16; at.out_fp16 = f16;
       IEF_TRY(attn_tc(at, st));
     }
     EpiParams e2;
     e2.bias = p.out_b; e2.resid = xa; e2.ld_resid = D; e2.out_f32 = xb; e2.ld_f32 = D;
     IEF_TRY(gemm_plan(plan == 1 ? 0 : plan, ctx, wo, int(M), D, D, e2, nullptr, num_sms, st));
     // x = x + mlp(ln_2(x))   (module.py:42): c_fc + QuickGELU, then c_proj with the residual
-    IEF_TRY(layernorm(xb, M, D, p.ln2_w, p.ln2_b, nullptr, nullptr, 1e-5f, h.f, h.hi, h.lo, num_sms, st));
+    IEF_TRY(layernorm(xb, M, D, p.ln2_w, p.ln2_b, nullptr, nullptr, 1e-5f, h.f, h.hi, h.lo, num_sms, st, f16));
     EpiParams e3;
     e3.bias = p.fc_b; e3.act = ACT_QUICKGELU;
     IEF_TRY(gemm_plan(plan, h, wf, int(M), 4 * D, D, e3, &u, num_sms, st));
@@ -554,6 +533,27 @@ int transformer(const float* x, const ResBlockParams* blocks, int layers, int L,
     e4.bias = p.proj_b; e4.resid = xb; e4.ld_resid = D; e4.out_f32 = xa; e4.ld_f32 = D;
     IEF_TRY(gemm_plan(plan, u, wp, int(M), D, 4 * D, e4, nullptr, num_sms, st));
   }
+  IEF_CUDA(cudaGetLastError());
+  return IEFVAD_OK;
+}
+
+int transformer(const float* x, const ResBlockParams* blocks, int layers, int L, int N, int D, int heads,
+                const float* attn_mask, const uint8_t* key_pad, int plan, float* out, int num_sms, cudaStream_t st) {
+  IEF_CHECK(x && out && blocks && layers >= 0 && L >= 0 && N >= 0, "transformer: bad argument");
+  IEF_CHECK(plan >= -1 && plan <= 2, "transformer: plan must be -1, 0, 1 or 2");
+  IEF_CHECK(D > 0 && D % 128 == 0 && heads > 0 && D % heads == 0, "transformer: width %d must be a multiple of 128 and of heads=%d", D, heads);
+  const int dh = D / heads;
+  IEF_CHECK(dh == 32 || dh == 64 || dh == 96 || dh == 128, "transformer: head dim %d unsupported (32, 64, 96, 128)", dh);
+  IEF_CHECK(N <= 65535, "transformer: batch %d exceeds the grid limit", N);
+  if (L == 0 || N == 0) return IEFVAD_OK;
+  const long long M = (long long)N * L;
+  IEF_CHECK(M < (1LL << 31), "transformer: too many rows");
+  Scratch sc(st);
+  float* xa;                                      // residual stream, batch-first [N, L, D]
+  IEF_TRY(sc.get(&xa, size_t(M) * D));
+  swap01_kernel<<<blocks_for(M * D / 4, num_sms), 256, 0, st>>>(x, L, N, D / 4, xa);   // [L, N, D] -> [N, L, D]
+  count_launches(1);
+  IEF_TRY(transformer_blocks(xa, blocks, layers, L, N, D, heads, attn_mask, key_pad, plan, num_sms, st));
   swap01_kernel<<<blocks_for(M * D / 4, num_sms), 256, 0, st>>>(xa, N, L, D / 4, out);   // [N, L, D] -> [L, N, D]
   count_launches(1);
   IEF_CUDA(cudaGetLastError());

@@ -32,9 +32,14 @@ struct ResBlockParams {   // one ResidualAttentionBlock, model/module.py:20-43 (
 
 // Transformer.forward, model/module.py:46-54, on SEQ-FIRST x [L, N, D] like the reference: `layers` pre-LN blocks
 // x += MHA(LN1 x); x += c_proj(QuickGELU(c_fc(LN2 x))).  attn_mask: optional additive [L, L]; key_pad: optional
-// [N, L] uint8 (non-zero = ignore).  out [L, N, D].
+// [N, L] uint8 (non-zero = ignore).  out [L, N, D].  plan: -1 fp32 FFMA, 0 bf16, 1 split-bf16, 2 fp16 operands.
 int transformer(const float* x, const ResBlockParams* blocks, int layers, int L, int N, int D, int heads,
                 const float* attn_mask, const uint8_t* key_pad, int plan, float* out, int num_sms,
                 cudaStream_t stream);
+
+// The block loop of `transformer` on a BATCH-FIRST fp32 residual x [N, L, D], updated in place (the residual stays
+// fp32 under every plan).  Arguments as `transformer`, already validated by the caller.
+int transformer_blocks(float* x, const ResBlockParams* blocks, int layers, int L, int N, int D, int heads,
+                       const float* attn_mask, const uint8_t* key_pad, int plan, int num_sms, cudaStream_t stream);
 
 }  // namespace iefvad

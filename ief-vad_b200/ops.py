@@ -10,7 +10,7 @@ import torch
 
 from . import _lib
 
-PLAN_CODES = {"fp32": -1, "bf16": 0, "split": 1, "fp16": 2}      # fp16: iefvad_linear only (the HH plan's GEMM)
+PLAN_CODES = {"fp32": -1, "bf16": 0, "split": 1, "fp16": 2}      # fp16: iefvad_linear, iefvad_transformer, clip
 ACTS = {None: 0, "none": 0, "relu": 1, "quickgelu": 2}
 
 

@@ -267,7 +267,8 @@ int iefvad_distance_scan(const float* s, int64_t B, int T, int D, float* y, void
 /* Transformer.forward((x, padding_mask)), model/module.py:20-54, x SEQ-FIRST [L, N, D]; params: HOST array of
  * layers * 12 device pointers per block in the order ln_1.weight, ln_1.bias, attn.in_proj_weight, attn.in_proj_bias,
  * attn.out_proj.weight, attn.out_proj.bias, ln_2.weight, ln_2.bias, mlp.c_fc.weight, mlp.c_fc.bias,
- * mlp.c_proj.weight, mlp.c_proj.bias.  attn_mask: optional additive [L, L]; key_padding_mask: optional [N, L] uint8. */
+ * mlp.c_proj.weight, mlp.c_proj.bias.  attn_mask: optional additive [L, L]; key_padding_mask: optional [N, L] uint8.
+ * plan: as above, or 2 = fp16 operands (fp32 accumulation, LayerNorm and residual stream). */
 int iefvad_transformer(const float* x, const float* const* params, int layers, int L, int N, int D, int heads,
                        const float* attn_mask, const uint8_t* key_padding_mask, int plan, float* out, void* stream);
 
@@ -296,6 +297,24 @@ int iefvad_process_feat(const void* src, int dtype, const int64_t* row_off, int6
  * plane in all three channels (an event-free batch gives 0 / 0 = NaN, as in the reference). */
 int iefvad_event_image(const uint8_t* frames, int64_t B, int C, int H, int W, float threshold, float clamp_max,
                        float* sum_out, float* event_out, void* stream);
+
+/* CLIP image encoder of the extraction step (row N4): VisionTransformer.forward(x), extracting/clip/model.py:206-241
+ * (ViT-L/14 in the reference's feature extraction).  x: DEVICE [N, 3, resolution, resolution] normalised pixels,
+ * dtype 0 fp32 / 1 fp16 / 2 bf16; out: DEVICE fp32 [N, output_dim].  Grid G = resolution / patch, T = G*G + 1 tokens.
+ * params: HOST array of 8 + 12 * layers DEVICE fp32 pointers in the order
+ *   conv1.weight [width, 3, patch, patch], class_embedding [width], positional_embedding [T, width],
+ *   ln_pre.weight, ln_pre.bias,
+ *   per block the 12 pointers of iefvad_transformer's table (transformer.resblocks.{i}.*),
+ *   ln_post.weight, ln_post.bias, proj [width, output_dim].
+ * plan: -1 fp32 FFMA, 2 fp16 operands with fp32 accumulation; LayerNorms, the residual stream and the projection are
+ * fp32 under both.  Constraints: resolution % patch == 0, width % 128 == 0 and <= 1024, width / heads in {32, 64, 96,
+ * 128}, 0 <= N <= 65535, layers <= 64; a malformed argument fails before the device is touched.
+ * Stateless like iefvad_transformer: the weights are converted on every call.  Device scratch (stream-ordered pool,
+ * released at the end of the call) under plan 2 is about 26 * width bytes per token (26 KB at ViT-L/14's width 1024,
+ * 6.7 MB per 224 px image) plus the fp16 weights (2 bytes per parameter, 0.6 GB for ViT-L/14); plan -1 needs about
+ * 44 * width bytes per token and 4 bytes per parameter. */
+int iefvad_clip_visual(const void* x, int dtype, int N, int resolution, int patch, int width, int layers, int heads,
+                       int output_dim, const float* const* params, int plan, float* out, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Instrumentation used by bench.py
