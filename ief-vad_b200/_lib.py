@@ -13,7 +13,7 @@ LIB_PATH = os.path.join(_HERE, "libiefvad.so")
 ABI_VERSION = 1
 F32, F16, BF16 = 0, 1, 2
 NOISE = {"Gaussian": 0, "StudentT": 1}
-PLANS = {"fp32": -1, "bf16": 0, "A": 2, "B": 6, "split": 7, "H": 26, "H8": 10, "HH": 56}
+PLANS = {"fp32": -1, "B": 6, "HH": 56}
 
 if not os.path.exists(LIB_PATH):
     raise ImportError(

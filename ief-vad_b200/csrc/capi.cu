@@ -108,7 +108,8 @@ int iefvad_model_set_param(iefvad_model* m, const char* key, const float* data, 
 
 int iefvad_model_set_plan(iefvad_model* m, int plan) {
   IEF_CHECK(m, "null model");
-  IEF_CHECK(plan == IEFVAD_PLAN_FP32 || (plan >= 0 && plan <= 63), "unknown precision plan %d", plan);
+  IEF_CHECK(plan == IEFVAD_PLAN_HH || plan == IEFVAD_PLAN_B || plan == IEFVAD_PLAN_FP32,
+            "unknown precision plan %d: choose IEFVAD_PLAN_HH (56), IEFVAD_PLAN_B (6) or IEFVAD_PLAN_FP32 (-1)", plan);
   m->impl.plan = plan;
   return IEFVAD_OK;
 }

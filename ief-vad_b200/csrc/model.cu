@@ -283,7 +283,9 @@ int Model::forward(const void* img, const void* ev, int in_dtype, long long B, l
             "forward: null tensor pointer");
   IEF_CHECK((w_i == nullptr) == (w_e == nullptr), "forward: w_i and w_e are written together or not at all");
   IEF_CHECK(T <= (1 << 24), "T=%lld too long", T);
-  const bool fp32_plan = plan < 0;
+  const bool fp32_plan = plan == PLAN_FP32;
+  const bool f16 = plan == PLAN_HH;        // fp16 operands, one MMA pass everywhere
+  const bool bsplit = plan == PLAN_B;      // bf16 operands, 3-term split for the heads and the refinement Linears
   if (vr) {
     IEF_CHECK(vr->len_host && vr->rowmap, "forward: valid-rows descriptor with null members");
     IEF_CHECK(!fp32_plan && L >= 1, "forward: the valid-rows mode needs a tensor-core plan and at least one attention layer");
@@ -322,8 +324,7 @@ int Model::forward(const void* img, const void* ev, int in_dtype, long long B, l
     // Out-projection + residual + LayerNorm(s) as one kernel (outproj_ln.cu) under the all-fp16 plan: y never reaches HBM.
     // Every encoder stage then works in encoder-row space (all rows, or the packed rows of the pad de-duplication); the
     // LAST layer's kernel writes its result through the inverse row map, i.e. directly as compact valid rows.
-    const bool ln_fused = !fp32_plan && (plan & PLAN_FP16_ATTENTION) && (plan & PLAN_FP16_HEADS) && D == kOutprojLnDim && L >= 1 &&
-                          outproj_ln_mode != 0 &&
+    const bool ln_fused = f16 && D == kOutprojLnDim && L >= 1 && outproj_ln_mode != 0 &&
                           (in_dtype == IEFVAD_DT_F16 || !(vr && vr->chunk_start && vr->chunk_valid));
     // Pad de-duplication (valid-rows mode, fp16 inputs, fp16 encoder, chunks of <= 256 rows): the zero-pad rows of a
     // chunk are identical, and stay identical to each other through every row-wise stage and through attention, so
@@ -331,8 +332,7 @@ int Model::forward(const void* img, const void* ev, int in_dtype, long long B, l
     // gets + log mult, which is exactly what mult equal keys contribute to the softmax).  The encoder then works on
     // Me = sum(valid + 1) packed rows instead of B * T; chunks without valid rows vanish.  Same arithmetic as the
     // dense forward up to the rounding of that one key's probability.
-    const bool dedup = direct_compact && !fp32_plan && (plan & PLAN_FP16_ATTENTION) && in_dtype == IEFVAD_DT_F16 &&
-                       T <= 256 && T % 32 == 0 && pad_dedup;
+    const bool dedup = direct_compact && f16 && in_dtype == IEFVAD_DT_F16 && T <= 256 && T % 32 == 0 && pad_dedup;
     long long Me = M;                       // rows the encoder stages before the valid-row cut run on
     if (dedup) {
       items_host.clear();
@@ -382,8 +382,8 @@ int Model::forward(const void* img, const void* ev, int in_dtype, long long B, l
     if (dedup && n_items == 0) continue;                 // no valid row in this slab
     // heads of both modalities + fusion as one kernel (heads_fuse.cu) when the caller keeps neither mu / logvar nor the fusion
     // weights (the evaluation forward) and the refinement chain takes the fp16 pair
-    const bool hf = ln_fused && vr && heads_outputs_unused && !w_i && !eval_wi_mean && (plan & PLAN_FP16_REFINE) && R > 0 &&
-                    D == kHeadsFuseDim && L >= 2 && heads_fuse_mode != 0;
+    const bool hf = ln_fused && vr && heads_outputs_unused && !w_i && !eval_wi_mean && R > 0 && D == kHeadsFuseDim && L >= 2 &&
+                    heads_fuse_mode != 0;
     if (ln_fused) {
       IEF_TRY(ln_scratch.reserve(outproj_ln_scratch_bytes(Me)));
       if (!ln_ident.p) {
@@ -403,11 +403,9 @@ int Model::forward(const void* img, const void* ev, int in_dtype, long long B, l
     for (int m = 0; m < 2; ++m) {
       const bool ragged = vr && vr->chunk_start && vr->chunk_valid;
       const uint8_t* in = static_cast<const uint8_t*>(inputs[m]) + (ragged ? 0 : size_t(row0) * D * in_esize);
-      const int e16 = (!fp32_plan && (plan & PLAN_FP16_ATTENTION)) ? 1 : 0;      // encoder operands in fp16
-      const bool esp = !fp32_plan && !e16 && (plan & PLAN_SPLIT_ENCODER);
       // fp16 inputs under an fp16-operand encoder are their own first GEMM operand AND (exactly) their own fp32
       // residual: no fp32 copy is written, a dense batch is not touched at all before the QKV GEMM
-      const bool direct16 = e16 && in_dtype == IEFVAD_DT_F16 && L >= 1 && !(vr && L == 1);
+      const bool direct16 = f16 && in_dtype == IEFVAD_DT_F16 && L >= 1 && !(vr && L == 1);
       const bf16* x16 = a_hi.as<bf16>();          // layer-0 operand (and fp16 residual when direct16)
       if (dedup) {
         // dense chunks or ragged packed rows -> the packed layout (the only pass over the inputs)
@@ -415,10 +413,9 @@ int Model::forward(const void* img, const void* ev, int in_dtype, long long B, l
         IEF_PROF(KC_INGEST, double(Mo) * D * 2 + double(Me) * D * 2,
                  pack_chunks(src, items_dev.as<ChunkItem>(), aux_dev.as<ChunkAux>(), n_items, D, a_hi.p, stream));
       } else if (ragged) {
-        IEF_CHECK(!esp, "forward: ragged inputs are not combined with the split-encoder plan");
         IEF_PROF(KC_INGEST, double(Mo) * D * in_esize + double(M) * D * (direct16 ? 2 : 4 + 2),
                  ingest_ragged(in, in_dtype, vr->chunk_start + b0, vr->start_base, vr->chunk_valid + b0, Bs, int(T), D,
-                               direct16 ? nullptr : x32.as<float>(), a_hi.as<bf16>(), (e16 && L > 0) ? 1 : 0, num_sms, stream));
+                               direct16 ? nullptr : x32.as<float>(), a_hi.as<bf16>(), (f16 && L > 0) ? 1 : 0, num_sms, stream));
       } else if (direct16) {
         IEF_CHECK((reinterpret_cast<uintptr_t>(in) & 15) == 0, "forward: fp16 inputs must be 16-byte aligned");
         x16 = reinterpret_cast<const bf16*>(in);
@@ -427,7 +424,7 @@ int Model::forward(const void* img, const void* ev, int in_dtype, long long B, l
                        num_sms, stream, 1));
       else
       IEF_PROF(KC_INGEST, double(M) * D * (in_esize + 4 + 2), ingest(in, in_dtype, M * D, x32.as<float>(), fp32_plan ? nullptr : a_hi.as<bf16>(),
-                     esp ? a_lo.as<bf16>() : nullptr, num_sms, stream, (e16 && L > 0) ? 1 : 0));
+                     nullptr, num_sms, stream, (f16 && L > 0) ? 1 : 0));
       for (int i = 0; i < L; ++i) {                                   // model/imf_vad.py:114-116 / :120-122
         const Linear& ip = in_proj[m][i];
         const Linear& op = out_proj[m][i];
@@ -443,21 +440,19 @@ int Model::forward(const void* img, const void* ev, int in_dtype, long long B, l
           IEF_PROF(KC_LAYERNORM, double(M) * D * 8, layernorm(y32.as<float>(), M, D, ln_w[m][i], ln_b[m][i], last ? whiten_w[m] : nullptr,
                             last ? whiten_b[m] : nullptr, 1e-5f, x32.as<float>(), nullptr, nullptr, num_sms, stream));
         } else {
-          const bool sp = esp;
-          const int a16 = e16;
           EpiParams e1;
-          e1.hi_fp16 = a16;
+          e1.hi_fp16 = f16;
           e1.mode = EPI_QKV; e1.bias = ip.b; e1.q = qb.as<bf16>(); e1.k = kb.as<bf16>(); e1.vt = vtb.as<bf16>();
           e1.T = dedup ? int(Me) : int(T); e1.H = H; e1.dh = dh; e1.dhp = dhq; e1.Tpad = dedup ? int(Me) : Tpad; e1.D = D; e1.qscale = qscale;
           GemmTcArgs g1;
-          g1.A_hi = (i == 0) ? x16 : a_hi.as<bf16>(); g1.A_lo = a_lo.as<bf16>(); g1.W_hi = a16 ? ip.w_h16 : ip.w_hi; g1.W_lo = ip.w_lo;
-          g1.M = int(Me); g1.N = 3 * D; g1.K = D; g1.lda = D; g1.ldw = D; g1.nsplit = sp ? 3 : 1; g1.fp16 = a16;
+          g1.A_hi = (i == 0) ? x16 : a_hi.as<bf16>(); g1.W_hi = f16 ? ip.w_h16 : ip.w_hi;
+          g1.M = int(Me); g1.N = 3 * D; g1.K = D; g1.lda = D; g1.ldw = D; g1.fp16 = f16;
           IEF_PROF(KC_GEMM_QKV, 6.0 * Me * D * D, gemm_tc(g1, e1, num_sms, stream));
           AttnTcArgs at;
           at.q = qb.as<bf16>(); at.k = kb.as<bf16>(); at.vt = vtb.as<bf16>(); at.out = h_hi.as<bf16>(); at.ldo = D;
           at.B = Bs; at.T = int(T); at.H = H; at.dh = dh; at.dhp = dhq; at.Tpad = Tpad;
           if (dedup) { at.B = 1; at.T = int(Me); at.Tpad = int(Me); at.items = items_dev.as<int>(); at.n_chunks = n_items; }
-          at.fp16 = a16; at.out_fp16 = a16;
+          at.fp16 = f16; at.out_fp16 = f16;
           if (direct_compact && last && !ln_fused) at.row_out = inv_map.as<int>();
           IEF_PROF(KC_ATTN_TC, attn_flops, attn_tc(at, stream));
           if (ln_fused) {
@@ -494,15 +489,13 @@ int Model::forward(const void* img, const void* ev, int in_dtype, long long B, l
             e2.bias = op.b; e2.resid = resid; e2.ld_resid = D; e2.out_f32 = yout; e2.ld_f32 = D;
             if (direct16 && i == 0) { e2.resid = nullptr; e2.resid_h16 = x16; }
             GemmTcArgs g2;
-            g2.A_hi = ctx; g2.W_hi = a16 ? op.w_h16 : op.w_hi; g2.M = int(Mc); g2.N = D; g2.K = D; g2.lda = D; g2.ldw = D;
-            g2.fp16 = a16;
+            g2.A_hi = ctx; g2.W_hi = f16 ? op.w_h16 : op.w_hi; g2.M = int(Mc); g2.N = D; g2.K = D; g2.lda = D; g2.ldw = D;
+            g2.fp16 = f16;
             IEF_PROF(KC_GEMM_OUT, 2.0 * Mc * D * D, gemm_tc(g2, e2, num_sms, stream));
-            // LN_i (+ whitening LN after the last layer, :117/:123); bf16 hi(/lo) feed the next GEMM
-            const bool h16 = (plan & PLAN_FP16_HEADS) != 0;                       // heads take fp16 operands, one pass
-            const bool need_lo = last ? (!h16 && (plan & PLAN_SPLIT_HEADS) != 0) : sp;
+            // LN_i (+ whitening LN after the last layer, :117/:123); hi (+ lo for the split heads) feed the next GEMM
             IEF_PROF(KC_LAYERNORM, double(Mc) * D * 8, layernorm(yout, Mc, D, ln_w[m][i], ln_b[m][i], last ? whiten_w[m] : nullptr,
                               last ? whiten_b[m] : nullptr, 1e-5f, last ? nullptr : x32.as<float>(), a_hi.as<bf16>(),
-                              need_lo ? a_lo.as<bf16>() : nullptr, num_sms, stream, ((a16 && !last) || (h16 && last)) ? 1 : 0,
+                              (last && bsplit) ? a_lo.as<bf16>() : nullptr, num_sms, stream, f16 ? 1 : 0,
                               (direct_compact && i == L - 2) ? inv_map.as<int>() : nullptr));
           }
         }
@@ -511,8 +504,7 @@ int Model::forward(const void* img, const void* ev, int in_dtype, long long B, l
         // no attention layers: only the whitening LN (model/imf_vad.py:117)
         IEF_PROF(KC_LAYERNORM, double(M) * D * 8, layernorm(x32.as<float>(), M, D, whiten_w[m], whiten_b[m], nullptr, nullptr, 1e-5f,
                           fp32_plan ? y32.as<float>() : nullptr, fp32_plan ? nullptr : a_hi.as<bf16>(),
-                          (!fp32_plan && (plan & PLAN_SPLIT_HEADS) && !(plan & PLAN_FP16_HEADS)) ? a_lo.as<bf16>() : nullptr,
-                          num_sms, stream, (!fp32_plan && (plan & PLAN_FP16_HEADS)) ? 1 : 0));
+                          bsplit ? a_lo.as<bf16>() : nullptr, num_sms, stream, f16 ? 1 : 0));
         if (fp32_plan) IEF_CUDA(cudaMemcpyAsync(x32.p, y32.p, size_t(M) * D * 4, cudaMemcpyDeviceToDevice, stream));
       }
       // heads (:125-128): one [M, D] x [2D, D]^T GEMM per modality, mu and logvar written to the user tensors
@@ -524,23 +516,20 @@ int Model::forward(const void* img, const void* ev, int in_dtype, long long B, l
         IEF_PROF(KC_GEMM_SIMT, 4.0 * Mo * D * D, gemm_simt(x32.as<float>(), D, heads[m].w, D, int(Mo), 2 * D, D, eh, stream));
       } else {
         GemmTcArgs gh;
-        const bool h16 = (plan & PLAN_FP16_HEADS) != 0;
         gh.A_hi = (ln_fused && vr) ? h_lo.as<bf16>() : a_hi.as<bf16>(); gh.A_lo = a_lo.as<bf16>();
-        gh.W_hi = h16 ? heads[m].w_h16 : heads[m].w_hi; gh.W_lo = heads[m].w_lo;
+        gh.W_hi = f16 ? heads[m].w_h16 : heads[m].w_hi; gh.W_lo = heads[m].w_lo;
         gh.M = int(Mo); gh.N = 2 * D; gh.K = D; gh.lda = D; gh.ldw = D;
-        gh.nsplit = (!h16 && (plan & PLAN_SPLIT_HEADS)) ? 3 : 1;
-        gh.fp16 = h16 ? 1 : 0;
+        gh.nsplit = bsplit ? 3 : 1;
+        gh.fp16 = f16 ? 1 : 0;
         IEF_PROF(KC_GEMM_HEADS, 4.0 * Mo * D * D, gemm_tc(gh, eh, num_sms, stream));
       }
     }
     if (Mo == 0) continue;
     // uncertainty-weighted fusion (:130-144)
-    const bool r16 = !fp32_plan && (plan & PLAN_FP16_REFINE);             // fp16 single-pass refinement operands
-    const bool rsp = !fp32_plan && !r16 && (plan & PLAN_SPLIT_REFINE);
     float* fused_out = fused + out0 * D;
     // fp16 refinement: the residual stream lives as an fp16 pair x = hi + lo (hi is the GEMM operand anyway), so a
     // refinement step moves 7.5 KB per row through HBM instead of 12 KB (no separate fp32 copy of x)
-    const bool pair16 = r16 && R > 0;
+    const bool pair16 = f16 && R > 0;
     float* xcur = (R == 0) ? fused_out : (pair16 ? nullptr : x32.as<float>());
     if (hf) {
       HeadsFuseArgs ha;
@@ -549,14 +538,14 @@ int Model::forward(const void* img, const void* ev, int in_dtype, long long B, l
       IEF_PROF(KC_HEADS_FUSE, 8.0 * Mo * D * D, heads_fuse(ha, num_sms, stream));
     } else {
       bf16* f_hi = (fp32_plan || R == 0) ? nullptr : a_hi.as<bf16>();
-      bf16* f_lo = ((rsp || pair16) && R > 0) ? a_lo.as<bf16>() : nullptr;
+      bf16* f_lo = f_hi ? a_lo.as<bf16>() : nullptr;     // both tensor-core plans start the refinement from a hi + lo pair
       const double fuse_bytes = double(Mo) * D * (16 + (w_i ? 8 : 0) + (xcur ? 4 : 0) + (f_hi ? 2 : 0) + (f_lo ? 2 : 0));
       if (eval_wi_mean && eval_we_mean && !w_i)      // the evaluation loop's w_i.mean(-1) / w_e.mean(-1), train/ucf_test.py:124-131
         IEF_PROF(KC_FUSE, fuse_bytes, fuse_rows(image_mu + out0 * D, event_mu + out0 * D, image_logvar + out0 * D, event_logvar + out0 * D,
-                 Mo, D, factor, eps, eval_wi_mean + out0, eval_we_mean + out0, xcur, f_hi, f_lo, num_sms, stream, r16 ? 1 : 0));
+                 Mo, D, factor, eps, eval_wi_mean + out0, eval_we_mean + out0, xcur, f_hi, f_lo, num_sms, stream, f16 ? 1 : 0));
       else
         IEF_PROF(KC_FUSE, fuse_bytes, fuse(image_mu + out0 * D, event_mu + out0 * D, image_logvar + out0 * D, event_logvar + out0 * D, Mo * D,
-                 factor, eps, w_i ? w_i + out0 * D : nullptr, w_e ? w_e + out0 * D : nullptr, xcur, f_hi, f_lo, num_sms, stream, r16 ? 1 : 0));
+                 factor, eps, w_i ? w_i + out0 * D : nullptr, w_e ? w_e + out0 * D : nullptr, xcur, f_hi, f_lo, num_sms, stream, f16 ? 1 : 0));
     }
     // iterative refinement (:146-149): x <- x - lambda * (W2 relu(W1 x + b1) + b2)
     // fp16-pair stream with enough rows: ONE persistent kernel keeps each 256-row tile on chip for all R steps
@@ -583,23 +572,23 @@ int Model::forward(const void* img, const void* ev, int in_dtype, long long B, l
         IEF_PROF(KC_GEMM_SIMT, 2.0 * Mo * D * D, gemm_simt(h32.as<float>(), D, ref2[i].w, D, int(Mo), D, D, e2, stream));
       } else {
         EpiParams e1;
-        e1.bias = ref1[i].b; e1.act = ACT_RELU; e1.out_hi = h_hi.as<bf16>(); e1.out_lo = rsp ? h_lo.as<bf16>() : nullptr;
-        e1.ld_bf = D; e1.hi_fp16 = r16 ? 1 : 0;
+        e1.bias = ref1[i].b; e1.act = ACT_RELU; e1.out_hi = h_hi.as<bf16>(); e1.out_lo = bsplit ? h_lo.as<bf16>() : nullptr;
+        e1.ld_bf = D; e1.hi_fp16 = f16 ? 1 : 0;
         GemmTcArgs g1;
-        g1.A_hi = a_hi.as<bf16>(); g1.A_lo = a_lo.as<bf16>(); g1.W_hi = r16 ? ref1[i].w_h16 : ref1[i].w_hi; g1.W_lo = ref1[i].w_lo;
-        g1.M = int(Mo); g1.N = D; g1.K = D; g1.lda = D; g1.ldw = D; g1.nsplit = rsp ? 3 : 1; g1.fp16 = r16 ? 1 : 0;
+        g1.A_hi = a_hi.as<bf16>(); g1.A_lo = a_lo.as<bf16>(); g1.W_hi = f16 ? ref1[i].w_h16 : ref1[i].w_hi; g1.W_lo = ref1[i].w_lo;
+        g1.M = int(Mo); g1.N = D; g1.K = D; g1.lda = D; g1.ldw = D; g1.nsplit = bsplit ? 3 : 1; g1.fp16 = f16 ? 1 : 0;
         IEF_PROF(KC_GEMM_REF1, 2.0 * Mo * D * D, gemm_tc(g1, e1, num_sms, stream));
         EpiParams e2;
         e2.bias = ref2[i].b; e2.resid = x32.as<float>(); e2.ld_resid = D; e2.alpha = -lambda_ref;
         e2.out_f32 = xnext; e2.ld_f32 = D;
-        if (!last) { e2.out_hi = a_hi.as<bf16>(); e2.out_lo = (rsp || pair16) ? a_lo.as<bf16>() : nullptr; e2.ld_bf = D; e2.hi_fp16 = r16 ? 1 : 0; }
-        if (pair16) {
+        if (!last) { e2.out_hi = a_hi.as<bf16>(); e2.out_lo = a_lo.as<bf16>(); e2.ld_bf = D; e2.hi_fp16 = f16 ? 1 : 0; }
+        if (f16) {
           e2.resid = nullptr; e2.resid_h16 = a_hi.as<bf16>(); e2.resid_l16 = a_lo.as<bf16>();
           if (!last) e2.out_f32 = nullptr;          // x stays an fp16 pair until the last step writes `fused`
         }
         GemmTcArgs g2;
-        g2.A_hi = h_hi.as<bf16>(); g2.A_lo = h_lo.as<bf16>(); g2.W_hi = r16 ? ref2[i].w_h16 : ref2[i].w_hi; g2.W_lo = ref2[i].w_lo;
-        g2.M = int(Mo); g2.N = D; g2.K = D; g2.lda = D; g2.ldw = D; g2.nsplit = rsp ? 3 : 1; g2.fp16 = r16 ? 1 : 0;
+        g2.A_hi = h_hi.as<bf16>(); g2.A_lo = h_lo.as<bf16>(); g2.W_hi = f16 ? ref2[i].w_h16 : ref2[i].w_hi; g2.W_lo = ref2[i].w_lo;
+        g2.M = int(Mo); g2.N = D; g2.K = D; g2.lda = D; g2.ldw = D; g2.nsplit = bsplit ? 3 : 1; g2.fp16 = f16 ? 1 : 0;
         IEF_PROF(KC_GEMM_REF2, 2.0 * Mo * D * D, gemm_tc(g2, e2, num_sms, stream));
       }
     }

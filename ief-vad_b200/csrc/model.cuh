@@ -15,15 +15,13 @@
 
 namespace iefvad {
 
-// precision plan: -1 = every contraction in fp32 FFMA; otherwise a bit mask of which bf16 GEMM groups use the
-// 3-term split (A_hi.W_hi + A_hi.W_lo + A_lo.W_hi)
-// PLAN_FP16_REFINE: the refinement Linears take fp16 (E5M10) operands in a single MMA pass instead of the 3-term bf16
-// split - the same 8.5e-5 score error at a third of the MMA work (DESIGN.md section 4)
-// PLAN_FP16_ATTENTION: the encoder (in-projection, q / k / v / P of the attention core, out-projection) uses fp16
-// operands - fp16 inputs are then exact, and the attention core is where bf16's mantissa dominates the error once the
-// heads / refinement are taken care of (zero-padded clips: 1.4e-3 with bf16, 1.7e-4 with fp16)
-enum : int { PLAN_FP32 = -1, PLAN_SPLIT_ENCODER = 1, PLAN_SPLIT_HEADS = 2, PLAN_SPLIT_REFINE = 4, PLAN_FP16_REFINE = 8,
-             PLAN_FP16_ATTENTION = 16, PLAN_FP16_HEADS = 32 };
+// precision plans (the values of IEFVAD_PLAN_* in include/iefvad.h):
+// PLAN_HH: fp16 (E5M10) operands in one MMA pass for every GEMM and the attention core.  fp16 inputs are then exact, and
+// one fp16 pass matches the 3-term bf16 split at a third of the MMA work (DESIGN.md section 4)
+// PLAN_B: bf16 operands; the heads and the refinement Linears use the 3-term split (A_hi.W_hi + A_hi.W_lo + A_lo.W_hi).
+// fp32's exponent range: the fall-back when an fp16 operand overflows
+// PLAN_FP32: every contraction in fp32 FFMA
+enum : int { PLAN_FP32 = -1, PLAN_B = 6, PLAN_HH = 56 };
 
 struct DevBuf {
   void* p = nullptr;
@@ -74,7 +72,7 @@ struct ValidRows {
 struct Model {
   int D = 0, H = 0, L = 0, R = 0, dh = 0, dhp = 0;
   float lambda_ref = 0.5f, factor = 1.f, eps = 1e-8f;
-  int plan = PLAN_FP16_HEADS | PLAN_FP16_REFINE | PLAN_FP16_ATTENTION;
+  int plan = PLAN_HH;
   bool pad_dedup = true;         // valid-rows mode: one representative per chunk for its identical zero-pad rows
   int refine_fused = -1;         // refinement chain as ONE persistent kernel (refine_fused.cu): -1 = when it pays (enough
                                  // rows to fill the CTA pairs), 0 = never (per-step GEMMs), 1 = always

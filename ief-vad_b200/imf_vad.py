@@ -10,7 +10,7 @@ in hand-written CUDA kernels reached through the C ABI - there is no PyTorch or 
 from __future__ import annotations
 
 import os
-from typing import Dict, Optional
+from typing import Dict, Optional, Tuple
 
 import torch
 import torch.nn as nn
@@ -18,6 +18,7 @@ import torch.nn as nn
 from . import _lib
 
 _MODALITIES = ("image", "event")
+_DTYPE_CODES = {torch.float32: _lib.F32, torch.float16: _lib.F16, torch.bfloat16: _lib.BF16}
 
 
 def _norm_device(device) -> torch.device:
@@ -188,6 +189,20 @@ class MultiModal_Fusion_Attn_Iter(nn.Module):
                                                        src.numel(), stream))
             self._uploaded[name] = tag
 
+    def _prepare(self, device: torch.device) -> Tuple[int, int]:
+        """The native model on `device` with current parameters, options, precision plan and pad de-duplication:
+        (handle, stream).  An unknown plan name raises ValueError before anything touches the device."""
+        plan = _lib.PLANS.get(str(self.precision))
+        if plan is None:
+            raise ValueError(f"unknown precision plan {self.precision!r}; choose from {sorted(_lib.PLANS)}")
+        with torch.cuda.device(device):
+            stream = torch.cuda.current_stream(device).cuda_stream
+            h = self._native(device)
+            self._sync_params(h, device, stream)
+            _lib.check(_lib.lib.iefvad_model_set_plan(h, plan))
+            _lib.check(_lib.lib.iefvad_model_set_pad_dedup(h, 1 if self.pad_dedup else 0))
+        return h, stream
+
     # ------------------------------------------------------------------ forward
     def forward(self, image_features: torch.Tensor, event_features: torch.Tensor,
                 with_scores: bool = False) -> Dict[str, torch.Tensor]:
@@ -208,31 +223,22 @@ class MultiModal_Fusion_Attn_Iter(nn.Module):
         if D != self.embed_dim:
             raise RuntimeError(f"last dimension {D} != embed_dim {self.embed_dim}")
         device = image_features.device
-        codes = {torch.float32: _lib.F32, torch.float16: _lib.F16, torch.bfloat16: _lib.BF16}
-        if image_features.dtype not in codes or event_features.dtype != image_features.dtype:
+        if image_features.dtype not in _DTYPE_CODES or event_features.dtype != image_features.dtype:
             image_features, event_features = image_features.float(), event_features.float()
         img = image_features.contiguous()
         ev = event_features.contiguous()
-        plan = _lib.PLANS.get(str(self.precision))
-        if plan is None:
-            raise ValueError(f"unknown precision plan {self.precision!r}; choose from {sorted(_lib.PLANS)}")
+        h, _ = self._prepare(device)
         with torch.cuda.device(device):
-            stream = torch.cuda.current_stream(device).cuda_stream
-            h = self._native(device)
-            self._sync_params(h, device, stream)
-            _lib.check(_lib.lib.iefvad_model_set_plan(h, plan))
-            _lib.check(_lib.lib.iefvad_model_set_pad_dedup(h, 1 if self.pad_dedup else 0))
-
             def launch(img_t, ev_t, wide_t, logits_t, scores_t):
                 _lib.check(_lib.lib.iefvad_model_forward(
-                    h, img_t.data_ptr(), ev_t.data_ptr(), codes[img_t.dtype], B, T,
+                    h, img_t.data_ptr(), ev_t.data_ptr(), _DTYPE_CODES[img_t.dtype], B, T,
                     wide_t[0].data_ptr(), logits_t.data_ptr(), wide_t[1].data_ptr(), wide_t[2].data_ptr(),
                     wide_t[3].data_ptr(), wide_t[4].data_ptr(), wide_t[5].data_ptr(), wide_t[6].data_ptr(),
                     _lib.ptr(scores_t), torch.cuda.current_stream(device).cuda_stream))
 
             # Small problems are bound by launching ~60 kernels from the host (0.5 ms for one 256-row clip): replay
             # them as one CUDA graph over static buffers (two copies in, one clone out).  IEFVAD_GRAPH_ROWS=0 disables.
-            replay = self._graph_replay(device, B, T, D, img, ev, plan, with_scores, launch) if B * T else None
+            replay = self._graph_replay(device, B, T, D, img, ev, with_scores, launch) if B * T else None
             if replay is not None:
                 wide, logits, scores = replay
             else:
@@ -268,7 +274,7 @@ class MultiModal_Fusion_Attn_Iter(nn.Module):
         keys = ("fused", "logits", "image_mu", "event_mu", "image_logvar", "event_logvar", "w_i", "w_e")
         return dict(zip(keys, outs))
 
-    def _graph_replay(self, device, B, T, D, img, ev, plan, with_scores, launch):
+    def _graph_replay(self, device, B, T, D, img, ev, with_scores, launch):
         """One CUDA-graph replay of the forward for a small [B, T] problem, or None (too large, disabled, already
         capturing, or capture failed once for this shape).  The graph is captured over static input / output buffers
         after an eager warm-up call that sizes every library workspace; parameters live in the library's own arena, so
@@ -276,7 +282,8 @@ class MultiModal_Fusion_Attn_Iter(nn.Module):
         limit = int(os.environ.get("IEFVAD_GRAPH_ROWS", "2048") or 0)
         if B * T > limit or torch.cuda.is_current_stream_capturing():
             return None
-        key = (str(device), B, T, img.dtype, plan, bool(with_scores), self.refine_fused, self.outproj_ln, self.heads_fuse)
+        key = (str(device), B, T, img.dtype, str(self.precision), bool(with_scores), self.refine_fused, self.outproj_ln,
+               self.heads_fuse)
         cache = self.__dict__.setdefault("_graphs", {})
         entry = cache.get(key)
         if entry is False:
@@ -332,8 +339,7 @@ class MultiModal_Fusion_Attn_Iter(nn.Module):
         then taken to be the zero pads of `process_split` and are not read)."""
         if img.dim() != 3 or img.shape != ev.shape or img.shape[-1] != self.embed_dim:
             raise RuntimeError(f"expected two [B, T, {self.embed_dim}] tensors")
-        codes = {torch.float32: _lib.F32, torch.float16: _lib.F16, torch.bfloat16: _lib.BF16}
-        if img.dtype not in codes or ev.dtype != img.dtype:
+        if img.dtype not in _DTYPE_CODES or ev.dtype != img.dtype:
             raise RuntimeError("inputs must share one of the dtypes float32 / float16 / bfloat16")
         on_host = not img.is_cuda
         if on_host != (not ev.is_cuda):
@@ -342,9 +348,6 @@ class MultiModal_Fusion_Attn_Iter(nn.Module):
         if on_host and device.type != "cuda":
             raise RuntimeError("host inputs need the target CUDA device")
         img, ev = img.contiguous(), ev.contiguous()
-        plan = _lib.PLANS.get(str(self.precision))
-        if plan is None:
-            raise ValueError(f"unknown precision plan {self.precision!r}; choose from {sorted(_lib.PLANS)}")
         B, T, _ = img.shape
         if (valid_lengths is None) != (rowmap is None):
             raise RuntimeError("valid_lengths and rowmap go together")
@@ -356,18 +359,14 @@ class MultiModal_Fusion_Attn_Iter(nn.Module):
                 raise RuntimeError("valid_lengths must have B entries and rowmap must be a device int32 tensor of sum(len)")
             arr = (C.c_int64 * B)(*lens)
             lens_ptr, n_out, keep = C.cast(arr, C.c_void_p), sum(lens), (img, ev, arr, rowmap)
+        h, stream = self._prepare(device)
         with torch.cuda.device(device):
-            stream = torch.cuda.current_stream(device).cuda_stream
-            h = self._native(device)
-            self._sync_params(h, device, stream)
-            _lib.check(_lib.lib.iefvad_model_set_plan(h, plan))
-            _lib.check(_lib.lib.iefvad_model_set_pad_dedup(h, 1 if self.pad_dedup else 0))
             logits = torch.empty(max(n_out, 1), dtype=torch.float32, device=device)[:n_out]
             scores = torch.empty(max(n_out, 1), dtype=torch.float32, device=device)[:n_out]
             self._set_eval_outputs(h, extra, n_out, device)
             try:
                 _lib.check(_lib.lib.iefvad_model_forward_scores(
-                    h, img.data_ptr(), ev.data_ptr(), codes[img.dtype], int(on_host), B, T, lens_ptr, _lib.ptr(rowmap),
+                    h, img.data_ptr(), ev.data_ptr(), _DTYPE_CODES[img.dtype], int(on_host), B, T, lens_ptr, _lib.ptr(rowmap),
                     logits.data_ptr(), scores.data_ptr(), stream))
             finally:
                 if extra:
@@ -383,12 +382,11 @@ class MultiModal_Fusion_Attn_Iter(nn.Module):
         chunk; the chunk / pad rule of data/tools.py:100-114 is applied on the device while ingesting.  valid_lengths:
         host ints [B]; rowmap (int32), chunk_start (int64), chunk_valid (int32): device tensors.  Compact results."""
         import ctypes as C
-        codes = {torch.float32: _lib.F32, torch.float16: _lib.F16, torch.bfloat16: _lib.BF16}
         lens = [int(v) for v in valid_lengths]
         B, n = len(lens), sum(int(v) for v in valid_lengths)
         if img_packed.is_cuda or ev_packed.is_cuda or img_packed.shape != ev_packed.shape or img_packed.dtype != ev_packed.dtype:
             raise RuntimeError("scores_ragged takes two host tensors of the same shape and dtype")
-        if tuple(img_packed.shape) != (n, self.embed_dim) or img_packed.dtype not in codes:
+        if tuple(img_packed.shape) != (n, self.embed_dim) or img_packed.dtype not in _DTYPE_CODES:
             raise RuntimeError(f"packed features must be [{n}, {self.embed_dim}] float32 / float16 / bfloat16")
         if any(v < 0 or v > T for v in lens):
             raise RuntimeError("valid lengths must lie in [0, T]")
@@ -396,23 +394,16 @@ class MultiModal_Fusion_Attn_Iter(nn.Module):
         for t, dt, cnt in ((rowmap, torch.int32, n), (chunk_start, torch.int64, B), (chunk_valid, torch.int32, B)):
             if not t.is_cuda or t.dtype != dt or t.numel() != cnt:
                 raise RuntimeError("rowmap / chunk_start / chunk_valid must be device tensors (int32 [sum len], int64 [B], int32 [B])")
-        plan = _lib.PLANS.get(str(self.precision))
-        if plan is None:
-            raise ValueError(f"unknown precision plan {self.precision!r}; choose from {sorted(_lib.PLANS)}")
         img, ev = img_packed.contiguous(), ev_packed.contiguous()
         arr = (C.c_int64 * B)(*lens)
+        h, stream = self._prepare(device)
         with torch.cuda.device(device):
-            stream = torch.cuda.current_stream(device).cuda_stream
-            h = self._native(device)
-            self._sync_params(h, device, stream)
-            _lib.check(_lib.lib.iefvad_model_set_plan(h, plan))
-            _lib.check(_lib.lib.iefvad_model_set_pad_dedup(h, 1 if self.pad_dedup else 0))
             logits = torch.empty(max(n, 1), dtype=torch.float32, device=device)[:n]
             scores = torch.empty(max(n, 1), dtype=torch.float32, device=device)[:n]
             self._set_eval_outputs(h, extra, n, device)
             try:
                 _lib.check(_lib.lib.iefvad_model_forward_scores_ragged(
-                    h, img.data_ptr(), ev.data_ptr(), codes[img.dtype], B, T, C.cast(arr, C.c_void_p), rowmap.data_ptr(),
+                    h, img.data_ptr(), ev.data_ptr(), _DTYPE_CODES[img.dtype], B, T, C.cast(arr, C.c_void_p), rowmap.data_ptr(),
                     chunk_start.data_ptr(), chunk_valid.data_ptr(), logits.data_ptr(), scores.data_ptr(), stream))
             finally:
                 if extra:

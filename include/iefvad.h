@@ -33,21 +33,16 @@ extern "C" {
 #define IEFVAD_NOISE_GAUSSIAN 0
 #define IEFVAD_NOISE_STUDENT_T 1
 
-/* precision plans (`plan`): -1 = every contraction in fp32 FFMA (1e-5 class);
- * >= 0 = tcgen05 bf16 GEMMs, OR-mask of the GEMM groups that use the 3-term bf16 split */
+/* precision plans of the model (iefvad_model_set_plan), fp32 accumulation throughout; LayerNorm, softmax statistics,
+ * fusion and the classifier are fp32 under every plan.  Any other value is rejected (IEFVAD_ERR_INVALID).
+ *   IEFVAD_PLAN_HH (default): every GEMM and the attention core take fp16 (E5M10) operands in one tcgen05 pass - the
+ *     11-bit mantissa at bf16's MMA rate; the fp16 range (65 504) is guarded, see iefvad_model_check_finite.
+ *   IEFVAD_PLAN_B: bf16 operands (fp32's exponent range); the mu / logvar heads and the refinement Linears use the
+ *     3-term bf16 split A_hi.W_hi + A_hi.W_lo + A_lo.W_hi.  The fall-back when plan HH overflows.
+ *   IEFVAD_PLAN_FP32: every contraction in fp32 FFMA (1e-5 class), the accuracy yardstick. */
 #define IEFVAD_PLAN_FP32 (-1)
-#define IEFVAD_PLAN_BF16 0
-#define IEFVAD_PLAN_SPLIT_ENCODER 1
-#define IEFVAD_PLAN_SPLIT_HEADS 2
-#define IEFVAD_PLAN_SPLIT_REFINE 4
-#define IEFVAD_PLAN_FP16_REFINE 8 /* refinement Linears: fp16 (E5M10) operands, one MMA pass, fp32 accumulate */
-#define IEFVAD_PLAN_A (IEFVAD_PLAN_SPLIT_HEADS)
-#define IEFVAD_PLAN_B (IEFVAD_PLAN_SPLIT_HEADS | IEFVAD_PLAN_SPLIT_REFINE) /* bf16 operands everywhere */
-#define IEFVAD_PLAN_FP16_ATTENTION 16 /* encoder (QKV in-projection, attention core, out-projection): fp16 operands */
-#define IEFVAD_PLAN_H (IEFVAD_PLAN_SPLIT_HEADS | IEFVAD_PLAN_FP16_REFINE | IEFVAD_PLAN_FP16_ATTENTION)
-#define IEFVAD_PLAN_FP16_HEADS 32 /* mu / logvar heads: fp16 operands, one MMA pass (overrides SPLIT_HEADS) */
-#define IEFVAD_PLAN_HH (IEFVAD_PLAN_FP16_HEADS | IEFVAD_PLAN_FP16_REFINE | IEFVAD_PLAN_FP16_ATTENTION) /* fp16 operands everywhere */
-/* ^ default: fp16 (11-bit mantissa, same tcgen05 kind::f16 rate) where bf16's 8-bit mantissa limits accuracy */
+#define IEFVAD_PLAN_B 6
+#define IEFVAD_PLAN_HH 56
 
 int iefvad_abi_version(void);
 const char* iefvad_last_error(void);
@@ -125,7 +120,7 @@ int iefvad_model_set_pad_dedup(iefvad_model* m, int on);
  * ascending.  The encoder then runs on all rows up to and including the last attention core; out-projection,
  * LayerNorms, heads, fusion, refinement and classifier (65 %% of the FLOPs) run on the valid rows only, and
  * logits / scores are COMPACT ([sum len]).
- * Pad de-duplication (default on, iefvad_model_set_pad_dedup; fp16 inputs, fp16-operand plans, T <= 256, >= 2
+ * Pad de-duplication (default on, iefvad_model_set_pad_dedup; fp16 inputs, plan HH, T <= 256, >= 2
  * layers): the rows past len are taken to be the all-zero pads process_split writes (data/tools.py:100-114) and are
  * not read - identical rows stay identical through the encoder, so ONE representative per chunk is computed and
  * enters every softmax with multiplicity T - len (+ log(T - len) on its score).  Same arithmetic as the dense

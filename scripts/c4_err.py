@@ -13,7 +13,7 @@ from conftest import load_golden  # noqa: E402
 from iefvad_b200 import synth  # noqa: E402
 from iefvad_b200.imf_vad import MMFMIL  # noqa: E402
 
-plans = sys.argv[1:] or ["fp32", "H", "HH", "H8", "B", "A", "split", "bf16"]
+plans = sys.argv[1:] or ["fp32", "HH", "B"]
 img, ev, lengths, labels = synth.make_c4_batch()
 valid = (np.arange(256)[None, :] < lengths.numpy()[:, None])
 sig = lambda a: 1 / (1 + np.exp(-a.astype(np.float64)))  # noqa: E731

@@ -13,8 +13,8 @@ from oracle import iefvad_oracle as O
 pytestmark = pytest.mark.gpu
 
 OUT_KEYS = ["fused", "logits", "image_mu", "event_mu", "image_logvar", "event_logvar", "w_i", "w_e"]
-SCORE_TOL = {"fp32": 1e-5, "B": 1e-3, "A": 1e-3, "split": 1e-3, "H": 1e-3, "HH": 1e-3}
-TENSOR_TOL = {"fp32": 2e-5, "B": 1e-3, "A": 2e-3, "split": 1e-3, "H": 1e-3, "HH": 1e-3}
+SCORE_TOL = {"fp32": 1e-5, "B": 1e-3, "HH": 1e-3}
+TENSOR_TOL = {"fp32": 2e-5, "B": 1e-3, "HH": 1e-3}
 
 
 @pytest.fixture(scope="module")
@@ -39,7 +39,7 @@ def _small_model(pkg, z):
 
 
 @pytest.mark.parametrize("name", ["small_studentt", "small_gaussian", "small_r0"])
-@pytest.mark.parametrize("plan", ["fp32", "B", "A", "H", "HH"])
+@pytest.mark.parametrize("plan", ["fp32", "B", "HH"])
 def test_small_models_all_eight_tensors(pkg, name, plan):
     z = load_golden(name + ".npz")
     m = _small_model(pkg, z)
@@ -72,7 +72,7 @@ def full(pkg):
 
 
 @pytest.mark.parametrize("tag", ["full_default", "full_perturbed"])
-@pytest.mark.parametrize("plan", ["fp32", "B", "A", "H", "HH"])
+@pytest.mark.parametrize("plan", ["fp32", "B", "HH"])
 def test_full_size_c1_against_reference_golden(pkg, full, tag, plan):
     _, synth = pkg
     m, z = full[tag]
@@ -90,7 +90,7 @@ def test_full_size_c1_against_reference_golden(pkg, full, tag, plan):
         assert e < TENSOR_TOL[plan], (k, e)
 
 
-@pytest.mark.parametrize("plan", ["fp32", "B", "H", "HH"])
+@pytest.mark.parametrize("plan", ["fp32", "B", "HH"])
 def test_full_size_ragged_chunked_and_long(pkg, full, plan):
     _, synth = pkg
     m, z = full["full_perturbed"]
@@ -212,7 +212,7 @@ def test_host_input_pipeline_equals_device_forward(pkg, full):
         _lib.check(_lib.lib.iefvad_model_set_host_part_rows(m.temporal._handle, 32768))
 
 
-@pytest.mark.parametrize("plan", ["fp32", "H", "HH", "B"])
+@pytest.mark.parametrize("plan", ["fp32", "HH", "B"])
 def test_c4_train_shape_forward_and_clas2(pkg, full, plan):
     """Config 4: B=64 x T=256 eval-mode forward + CLAS2 (train/ucf_train.py:60-73, train/loss.py:18-30) against the
     reference's golden logits and loss."""
@@ -234,7 +234,7 @@ def test_c4_train_shape_forward_and_clas2(pkg, full, plan):
     assert abs(float(loss) - float(z["c4:loss"])) < (1e-5 if plan == "fp32" else 2e-4)
 
 
-@pytest.mark.parametrize("plan", ["H", "HH", "B"])
+@pytest.mark.parametrize("plan", ["HH", "B"])
 def test_c5_long_sequence_t16384(pkg, full, plan):
     """Config 5: one video of T = 16384 fed directly (no chunking): streaming-softmax attention over 128 key blocks,
     against the reference's golden logits (CPU fp32, 25 s / 12 GB there)."""
@@ -249,7 +249,7 @@ def test_c5_long_sequence_t16384(pkg, full, plan):
     assert O.max_norm_err(out["fused"].cpu().numpy()[0, rows], z["c5:fused:rows"]) < TENSOR_TOL[plan]
 
 
-@pytest.mark.parametrize("plan", ["H", "HH", "B"])
+@pytest.mark.parametrize("plan", ["HH", "B"])
 def test_valid_rows_mode_is_bit_identical_to_the_full_forward(pkg, full, plan):
     """iefvad_model_forward_scores with a row map: stages after the last attention core run on the valid rows only;
     without pad de-duplication the compact logits / scores equal the valid rows of the full forward bit for bit

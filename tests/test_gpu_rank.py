@@ -172,7 +172,7 @@ def test_evaluator_matches_reference_eval_loop(ops):
         fi.append(a)
         fe.append(b)
     ev.set_device_features(ev.chunk_features(fi), ev.chunk_features(fe))
-    for plan, tol in (("fp32", 1e-5), ("B", 1e-3), ("H", 1e-3), ("HH", 1e-3)):
+    for plan, tol in (("fp32", 1e-5), ("B", 1e-3), ("HH", 1e-3)):
         model.temporal.precision = plan
         with torch.no_grad():
             res = ev.step()
