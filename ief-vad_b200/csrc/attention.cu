@@ -53,7 +53,7 @@ __global__ void __launch_bounds__(192, 2)
 attn_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                const __grid_constant__ CUtensorMap tmVt, bf16* __restrict__ out, int ldo, int T, int H,
                const float* __restrict__ attn_mask /* [T,T] additive or null */,
-               const uint8_t* __restrict__ key_pad /* [B,T] 1 = ignore, or null */, int fp16, int out_fp16,
+               const uint8_t* __restrict__ key_pad /* [B,T] 1 = ignore, or null */, int fp16,
                const int* __restrict__ row_out) {
   using Cfg = AttnCfg<DH, DHP>;
   extern __shared__ uint8_t smem_raw[];
@@ -258,13 +258,8 @@ attn_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ 
         uint8_t* ptile = smem + Cfg::kOffP + (c >> 1) * (QB * 128) + r * 128;
 #pragma unroll
         for (int g = 0; g < 4; ++g) {
-          uint4 u;
-          u.x = pack_16x2(v[g * 8 + 0], v[g * 8 + 1], fp16);
-          u.y = pack_16x2(v[g * 8 + 2], v[g * 8 + 3], fp16);
-          u.z = pack_16x2(v[g * 8 + 4], v[g * 8 + 5], fp16);
-          u.w = pack_16x2(v[g * 8 + 6], v[g * 8 + 7], fp16);
           const int chunk = ((c & 1) * 4 + g) ^ (r & 7);
-          *reinterpret_cast<uint4*>(ptile + chunk * 16) = u;
+          *reinterpret_cast<uint4*>(ptile + chunk * 16) = pack_16x8(v + g * 8, fp16);
         }
       }
       l += lsum;
@@ -290,14 +285,7 @@ attn_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ 
       const float inv = 1.f / l;
       bf16* dst = out + ro * ldo + h * DH;
 #pragma unroll
-      for (int d = 0; d < DH; d += 8) {
-        uint4 u;
-        u.x = pack_16x2(o_acc[d + 0] * inv, o_acc[d + 1] * inv, out_fp16);
-        u.y = pack_16x2(o_acc[d + 2] * inv, o_acc[d + 3] * inv, out_fp16);
-        u.z = pack_16x2(o_acc[d + 4] * inv, o_acc[d + 5] * inv, out_fp16);
-        u.w = pack_16x2(o_acc[d + 6] * inv, o_acc[d + 7] * inv, out_fp16);
-        *reinterpret_cast<uint4*>(dst + d) = u;
-      }
+      for (int d = 0; d < DH; d += 8) *reinterpret_cast<uint4*>(dst + d) = pack_16x8(o_acc + d, fp16, inv);
     }
   }
 
@@ -325,7 +313,7 @@ int launch_attn_tc(const AttnTcArgs& a, cudaStream_t stream) {
   IEF_TRY(make_tmap_3d(&tv, a.vt, a.T, DH, BH, uint64_t(a.Tpad) * 2, uint64_t(DH) * a.Tpad * 2, 64, DH, 1));
   dim3 grid((a.T + QB - 1) / QB, a.H, a.B);
   attn_tc_kernel<DH, DHP><<<grid, 192, Cfg::kSmemBytes, stream>>>(tq, tk, tv, a.out, a.ldo, a.T, a.H, a.attn_mask,
-                                                              a.key_pad, a.fp16, a.out_fp16, a.row_out);
+                                                              a.key_pad, a.fp16, a.row_out);
   count_launches(1);
   IEF_CUDA(cudaGetLastError());
   return IEFVAD_OK;

@@ -12,8 +12,7 @@ struct AttnTcArgs {
   int B = 0, T = 0, H = 0, dh = 0, dhp = 0, Tpad = 0;
   const float* attn_mask = nullptr;    // optional additive [T, T]
   const uint8_t* key_pad = nullptr;    // optional [B, T], non-zero = ignore key
-  int fp16 = 0;                        // q / k / vt hold fp16 and P is rounded to fp16 (11-bit mantissa), else bf16
-  int out_fp16 = 0;                    // `out` receives fp16 instead of bf16
+  int fp16 = 0;                        // q / k / vt / out hold fp16 and P is rounded to fp16 (11-bit mantissa), else bf16
   const int* row_out = nullptr;        // optional [B*T]: output row of query row b*T+t (compact layouts), < 0 = drop
   // ragged items (short kernel only): q / k are [H, T, dhp], vt [H, dh, Tpad] over ALL packed rows and items[c] =
   // {first row, rows (<= 256), valid rows, multiplicity of the last row as a key (0 = none)} for n_chunks row ranges

@@ -53,7 +53,7 @@ template <int DH, int DHP>
 __global__ void __launch_bounds__(kThreads, 1)
 attn_long_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                  const __grid_constant__ CUtensorMap tmVt, bf16* __restrict__ out, int ldo, int T, int H, int n_items,
-                 int fp16, int out_fp16, const int* __restrict__ row_out) {
+                 int fp16, const int* __restrict__ row_out) {
   using Cfg = LongCfg<DH, DHP>;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -300,14 +300,7 @@ attn_long_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
       if (tq < T && ro >= 0) {
         bf16* dst = out + ro * ldo + h * DH + hf * (DH / 2);
 #pragma unroll
-        for (int d = 0; d < DH / 2; d += 8) {
-          uint4 u;
-          u.x = pack_16x2(o[d + 0] * inv, o[d + 1] * inv, out_fp16);
-          u.y = pack_16x2(o[d + 2] * inv, o[d + 3] * inv, out_fp16);
-          u.z = pack_16x2(o[d + 4] * inv, o[d + 5] * inv, out_fp16);
-          u.w = pack_16x2(o[d + 6] * inv, o[d + 7] * inv, out_fp16);
-          *reinterpret_cast<uint4*>(dst + d) = u;
-        }
+        for (int d = 0; d < DH / 2; d += 8) *reinterpret_cast<uint4*>(dst + d) = pack_16x8(o + d, fp16, inv);
       }
       named_bar_sync(1 + t, 256);        // the slots are written again by the next item's first block
     }
@@ -339,7 +332,7 @@ int launch_attn_long(const AttnTcArgs& a, int num_sms, cudaStream_t stream) {
   IEF_CHECK(items < (1LL << 31), "attn_long: too many work items");
   const int grid = items < num_sms ? int(items) : num_sms;
   attn_long_kernel<DH, DHP><<<grid, kThreads, Cfg::kSmemBytes, stream>>>(tq, tk, tv, a.out, a.ldo, a.T, a.H, int(items),
-                                                                        a.fp16, a.out_fp16, a.row_out);
+                                                                        a.fp16, a.row_out);
   count_launches(1);
   IEF_CUDA(cudaGetLastError());
   return IEFVAD_OK;

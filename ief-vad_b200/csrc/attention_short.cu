@@ -54,7 +54,7 @@ template <int DH, int DHP>
 __global__ void __launch_bounds__(kThreads, 1)
 attn_short_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                   const __grid_constant__ CUtensorMap tmVt, bf16* __restrict__ out, int ldo, int T, int H, int n_items,
-                  int fp16, int out_fp16, const int* __restrict__ row_out, const int4* __restrict__ items) {
+                  int fp16, const int* __restrict__ row_out, const int4* __restrict__ items) {
   using Cfg = ShortCfg<DH, DHP>;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -349,14 +349,7 @@ attn_short_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
       if (tq < Tk && ro >= 0) {
         bf16* dst = out + ro * ldo + h * DH + hf * (DH / 2);
 #pragma unroll
-        for (int d = 0; d < DH / 2; d += 8) {
-          uint4 u;
-          u.x = pack_16x2(o[d + 0] * inv, o[d + 1] * inv, out_fp16);
-          u.y = pack_16x2(o[d + 2] * inv, o[d + 3] * inv, out_fp16);
-          u.z = pack_16x2(o[d + 4] * inv, o[d + 5] * inv, out_fp16);
-          u.w = pack_16x2(o[d + 6] * inv, o[d + 7] * inv, out_fp16);
-          *reinterpret_cast<uint4*>(dst + d) = u;
-        }
+        for (int d = 0; d < DH / 2; d += 8) *reinterpret_cast<uint4*>(dst + d) = pack_16x8(o + d, fp16, inv);
       }
     }
   }
@@ -388,7 +381,7 @@ int launch_attn_short(const AttnTcArgs& a, int num_sms, cudaStream_t stream) {
   const int n_items = a.items ? a.n_chunks * a.H : int(BH);
   const int grid = n_items < num_sms ? n_items : num_sms;
   attn_short_kernel<DH, DHP><<<grid, kThreads, Cfg::kSmemBytes, stream>>>(tq, tk, tv, a.out, a.ldo, a.T, a.H, n_items,
-                                                                         a.fp16, a.out_fp16, a.row_out, reinterpret_cast<const int4*>(a.items));
+                                                                         a.fp16, a.row_out, reinterpret_cast<const int4*>(a.items));
   count_launches(1);
   IEF_CUDA(cudaGetLastError());
   return IEFVAD_OK;

@@ -1,4 +1,4 @@
-// Shared device helpers for the IEF-VAD sm_100a kernels: error plumbing, bf16 hi/lo splitting,
+// Shared device helpers for the IEF-VAD sm_100a kernels: error plumbing, 16-bit (fp16 / bf16) hi/lo splitting,
 // and thin inline-PTX wrappers for mbarrier, TMA (cp.async.bulk.tensor) and tcgen05 / TMEM.
 #pragma once
 
@@ -64,6 +64,47 @@ __device__ __forceinline__ uint32_t pack_16x2(float a, float b, int f16) {
 __device__ __forceinline__ void split_bf16(float x, bf16& hi, bf16& lo) {
   hi = __float2bfloat16_rn(x);
   lo = __float2bfloat16_rn(x - __bfloat162float(hi));
+}
+
+// The 16-bit operand pair of two floats, packed like pack_16x2: hi = round16(x), lo = round16(x - float(hi)).
+// hi + lo carries x to ~16 mantissa bits in bf16 and ~22 in fp16 (E5M10) - the fp16 plans' residual stream.
+__device__ __forceinline__ void split_16x2(float a, float b, int f16, uint32_t& hi, uint32_t& lo) {
+  if (f16) {
+    const __half2 h = __floats2half2_rn(a, b);
+    const float2 hf = __half22float2(h);
+    const __half2 l = __floats2half2_rn(a - hf.x, b - hf.y);
+    hi = *reinterpret_cast<const uint32_t*>(&h);
+    lo = *reinterpret_cast<const uint32_t*>(&l);
+  } else {
+    const __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
+    const float2 hf = __bfloat1622float2(h);
+    hi = *reinterpret_cast<const uint32_t*>(&h);
+    lo = pack_bf16x2(a - hf.x, b - hf.y);
+  }
+}
+
+// eight floats, each times `s`, -> one 16-byte vector of 16-bit values in element order
+__device__ __forceinline__ uint4 pack_16x8(const float* v, int f16, float s = 1.f) {
+  return make_uint4(pack_16x2(v[0] * s, v[1] * s, f16), pack_16x2(v[2] * s, v[3] * s, f16),
+                    pack_16x2(v[4] * s, v[5] * s, f16), pack_16x2(v[6] * s, v[7] * s, f16));
+}
+
+// eight fp16 values -> floats; with `lo`, eight split_16x2 fp16 pairs -> float(hi) + float(lo)
+__device__ __forceinline__ void unpack_f16x8(const uint4& hi, const uint4* lo, float* r) {
+  const __half2* h = reinterpret_cast<const __half2*>(&hi);
+#pragma unroll
+  for (int q = 0; q < 4; ++q) {
+    const float2 f = __half22float2(h[q]);
+    r[2 * q] = f.x; r[2 * q + 1] = f.y;
+  }
+  if (lo) {
+    const __half2* l = reinterpret_cast<const __half2*>(lo);
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      const float2 f = __half22float2(l[q]);
+      r[2 * q] += f.x; r[2 * q + 1] += f.y;
+    }
+  }
 }
 
 __device__ __forceinline__ float warp_sum(float v) {

@@ -60,21 +60,9 @@ ingest_kernel(const Tin* __restrict__ in, long long n8, float* __restrict__ out_
       o[0] = make_float4(v[0], v[1], v[2], v[3]);
       o[1] = make_float4(v[4], v[5], v[6], v[7]);
     }
-    uint32_t hi[4], lo[4];
+    uint32_t hi[4], lo[4];                    // fp16: exact for fp16 inputs, the remainder is zero then
 #pragma unroll
-    for (int q = 0; q < 4; ++q) {
-      if (hi_fp16) {                          // fp16 operand copy (exact for fp16 inputs) + fp16 remainder (zero then)
-        const __half2 h2 = __floats2half2_rn(v[2 * q], v[2 * q + 1]);
-        hi[q] = *reinterpret_cast<const uint32_t*>(&h2);
-        const float2 hf = __half22float2(h2);
-        const __half2 l2 = __floats2half2_rn(v[2 * q] - hf.x, v[2 * q + 1] - hf.y);
-        lo[q] = *reinterpret_cast<const uint32_t*>(&l2);
-        continue;
-      }
-      const bf16 ah = __float2bfloat16_rn(v[2 * q]), bh = __float2bfloat16_rn(v[2 * q + 1]);
-      hi[q] = pack_bf16x2(__bfloat162float(ah), __bfloat162float(bh));
-      lo[q] = pack_bf16x2(v[2 * q] - __bfloat162float(ah), v[2 * q + 1] - __bfloat162float(bh));
-    }
+    for (int q = 0; q < 4; ++q) split_16x2(v[2 * q], v[2 * q + 1], hi_fp16, hi[q], lo[q]);
     if (out_hi) *reinterpret_cast<uint4*>(out_hi + i * 8) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
     if (out_lo) *reinterpret_cast<uint4*>(out_lo + i * 8) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
   }
@@ -105,13 +93,17 @@ ingest_ragged_kernel(const Tin* __restrict__ packed, const long long* __restrict
       o[0] = make_float4(v[0], v[1], v[2], v[3]);
       o[1] = make_float4(v[4], v[5], v[6], v[7]);
     }
-    if (out_hi) {
-      uint4 u;
-      u.x = pack_16x2(v[0], v[1], hi_fp16); u.y = pack_16x2(v[2], v[3], hi_fp16);
-      u.z = pack_16x2(v[4], v[5], hi_fp16); u.w = pack_16x2(v[6], v[7], hi_fp16);
-      *reinterpret_cast<uint4*>(out_hi + i * 8) = u;
-    }
+    if (out_hi) *reinterpret_cast<uint4*>(out_hi + i * 8) = pack_16x8(v, hi_fp16);
   }
+}
+
+// four consecutive values -> their 16-bit pairs at hi[off, off + 4) and (when lo != null) lo[off, off + 4)
+__device__ __forceinline__ void store_split4(const float* v, int f16, bf16* hi, bf16* lo, long long off) {
+  uint2 h, l;
+  split_16x2(v[0], v[1], f16, h.x, l.x);
+  split_16x2(v[2], v[3], f16, h.y, l.y);
+  *reinterpret_cast<uint2*>(hi + off) = h;
+  if (lo) *reinterpret_cast<uint2*>(lo + off) = l;
 }
 
 // ---------------------------------------------------------------- LayerNorm: one warp per row, row in registers
@@ -168,18 +160,7 @@ layernorm_kernel(const float* __restrict__ x, long long M, const float* __restri
           *reinterpret_cast<float4*>(out_f32 + ro * D + (lane + 32 * i) * 4) =
               make_float4(v[4 * i], v[4 * i + 1], v[4 * i + 2], v[4 * i + 3]);
       }
-      if (out_hi && hi_fp16) {
-        uint2 u;
-        u.x = pack_16x2(v[4 * i], v[4 * i + 1], 1);
-        u.y = pack_16x2(v[4 * i + 2], v[4 * i + 3], 1);
-        *reinterpret_cast<uint2*>(out_hi + off) = u;
-      } else if (out_hi) {
-        bf16 h[4], l[4];
-#pragma unroll
-        for (int e = 0; e < 4; ++e) split_bf16(v[4 * i + e], h[e], l[e]);
-        *reinterpret_cast<uint2*>(out_hi + off) = *reinterpret_cast<uint2*>(h);
-        if (out_lo) *reinterpret_cast<uint2*>(out_lo + off) = *reinterpret_cast<uint2*>(l);
-      }
+      if (out_hi) store_split4(v + 4 * i, hi_fp16, out_hi, out_lo, off);
     }
   }
 }
@@ -196,41 +177,13 @@ fuse_kernel(const float4* __restrict__ mu_i, const float4* __restrict__ mu_e, co
     const float li[4] = {c.x, c.y, c.z, c.w}, le[4] = {d.x, d.y, d.z, d.w};
     float wi[4], we[4], f[4];
 #pragma unroll
-    for (int e = 0; e < 4; ++e) {
-      // exact op order of model/imf_vad.py:134-144, every product / sum rounded separately like ATen
-      const float ri = __fmul_rn(factor, expf(-li[e]));
-      const float re = __fmul_rn(factor, expf(-le[e]));
-      const float den = __fadd_rn(__fadd_rn(ri, re), eps);
-      wi[e] = __fdiv_rn(ri, den);
-      we[e] = __fdiv_rn(re, den);
-      f[e] = __fadd_rn(__fmul_rn(wi[e], mi[e]), __fmul_rn(we[e], me[e]));
-    }
+    for (int e = 0; e < 4; ++e) f[e] = fuse_one(mi[e], me[e], li[e], le[e], factor, eps, wi[e], we[e]);
     if (w_i) {                                  // the evaluation forward does not return the fusion weights
       __stcs(w_i + i, make_float4(wi[0], wi[1], wi[2], wi[3]));
       __stcs(w_e + i, make_float4(we[0], we[1], we[2], we[3]));
     }
     if (fused) fused[i] = make_float4(f[0], f[1], f[2], f[3]);
-    if (fused_hi && hi_fp16) {                 // fp16 operand copy (refinement chain of plan H)
-      const __half2 h01 = __floats2half2_rn(f[0], f[1]), h23 = __floats2half2_rn(f[2], f[3]);
-      uint2 u;
-      u.x = *reinterpret_cast<const uint32_t*>(&h01);
-      u.y = *reinterpret_cast<const uint32_t*>(&h23);
-      *reinterpret_cast<uint2*>(fused_hi + i * 4) = u;
-      if (fused_lo) {                           // fp16 remainder: hi + lo carries the residual stream (~22 bits)
-        const float2 f01 = __half22float2(h01), f23 = __half22float2(h23);
-        const __half2 l01 = __floats2half2_rn(f[0] - f01.x, f[1] - f01.y), l23 = __floats2half2_rn(f[2] - f23.x, f[3] - f23.y);
-        uint2 ul;
-        ul.x = *reinterpret_cast<const uint32_t*>(&l01);
-        ul.y = *reinterpret_cast<const uint32_t*>(&l23);
-        *reinterpret_cast<uint2*>(fused_lo + i * 4) = ul;
-      }
-    } else if (fused_hi) {
-      bf16 h[4], l[4];
-#pragma unroll
-      for (int e = 0; e < 4; ++e) split_bf16(f[e], h[e], l[e]);
-      *reinterpret_cast<uint2*>(fused_hi + i * 4) = *reinterpret_cast<uint2*>(h);
-      if (fused_lo) *reinterpret_cast<uint2*>(fused_lo + i * 4) = *reinterpret_cast<uint2*>(l);
-    }
+    if (fused_hi) store_split4(f, hi_fp16, fused_hi, fused_lo, i * 4);   // operand pair of the refinement chain
   }
 }
 
@@ -253,36 +206,13 @@ fuse_rows_kernel(const float4* __restrict__ mu_i, const float4* __restrict__ mu_
       float f[4];
 #pragma unroll
       for (int e = 0; e < 4; ++e) {
-        const float ri = __fmul_rn(factor, expf(-li[e]));
-        const float re = __fmul_rn(factor, expf(-le[e]));
-        const float den = __fadd_rn(__fadd_rn(ri, re), eps);
-        const float wi = __fdiv_rn(ri, den), we = __fdiv_rn(re, den);
+        float wi, we;
+        f[e] = fuse_one(mi[e], me[e], li[e], le[e], factor, eps, wi, we);
         si += wi;
         se += we;
-        f[e] = __fadd_rn(__fmul_rn(wi, mi[e]), __fmul_rn(we, me[e]));
       }
       if (fused) fused[i] = make_float4(f[0], f[1], f[2], f[3]);
-      if (fused_hi && hi_fp16) {
-        const __half2 h01 = __floats2half2_rn(f[0], f[1]), h23 = __floats2half2_rn(f[2], f[3]);
-        uint2 u;
-        u.x = *reinterpret_cast<const uint32_t*>(&h01);
-        u.y = *reinterpret_cast<const uint32_t*>(&h23);
-        *reinterpret_cast<uint2*>(fused_hi + i * 4) = u;
-        if (fused_lo) {
-          const float2 f01 = __half22float2(h01), f23 = __half22float2(h23);
-          const __half2 l01 = __floats2half2_rn(f[0] - f01.x, f[1] - f01.y), l23 = __floats2half2_rn(f[2] - f23.x, f[3] - f23.y);
-          uint2 ul;
-          ul.x = *reinterpret_cast<const uint32_t*>(&l01);
-          ul.y = *reinterpret_cast<const uint32_t*>(&l23);
-          *reinterpret_cast<uint2*>(fused_lo + i * 4) = ul;
-        }
-      } else if (fused_hi) {
-        bf16 h[4], l[4];
-#pragma unroll
-        for (int e = 0; e < 4; ++e) split_bf16(f[e], h[e], l[e]);
-        *reinterpret_cast<uint2*>(fused_hi + i * 4) = *reinterpret_cast<uint2*>(h);
-        if (fused_lo) *reinterpret_cast<uint2*>(fused_lo + i * 4) = *reinterpret_cast<uint2*>(l);
-      }
+      if (fused_hi) store_split4(f, hi_fp16, fused_hi, fused_lo, i * 4);
     }
     si = warp_sum(si);
     se = warp_sum(se);

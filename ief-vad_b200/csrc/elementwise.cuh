@@ -5,9 +5,9 @@ namespace iefvad {
 
 enum : int { IEFVAD_DT_F32 = 0, IEFVAD_DT_F16 = 1, IEFVAD_DT_BF16 = 2 };
 
-// in (f32 / f16 / bf16, n elements, n % 8 == 0) -> optional fp32 copy, optional bf16 hi, optional bf16 lo
+// in (f32 / f16 / bf16, n elements, n % 8 == 0) -> optional fp32 copy, optional 16-bit hi, optional 16-bit lo
 int ingest(const void* in, int dtype, long long n, float* out_f32, bf16* out_hi, bf16* out_lo, int num_sms,
-           cudaStream_t stream, int hi_fp16 = 0 /* out_hi receives fp16 instead of bf16 (no lo) */);
+           cudaStream_t stream, int hi_fp16 = 0 /* out_hi / out_lo receive fp16 instead of bf16 */);
 
 // The same for a ragged batch: `packed` holds only the valid rows of the n_chunks zero-padded [T, D] chunks, chunk c's
 // rows starting at packed row chunk_start[c] - start_base (device arrays); pad rows are written as zeros.
@@ -18,7 +18,7 @@ int ingest_ragged(const void* packed, int dtype, const long long* chunk_start, l
 // out = LN(x; w1, b1) or LN(LN(x; w1, b1); w2, b2) when w2 != null.  x [M, D] fp32.
 int layernorm(const float* x, long long M, int D, const float* w1, const float* b1, const float* w2, const float* b2,
               float eps, float* out_f32, bf16* out_hi, bf16* out_lo, int num_sms, cudaStream_t stream,
-              int hi_fp16 = 0 /* out_hi receives fp16 instead of bf16 (no lo) */,
+              int hi_fp16 = 0 /* out_hi / out_lo receive fp16 instead of bf16 */,
               const int* f32_row_out = nullptr /* [M]: row of out_f32 that receives source row r, < 0 = none */);
 
 // Packed ("dedup-pad") row layout of a batch of zero-padded chunks: chunk c owns rows [start, start + span) of which the
@@ -39,10 +39,23 @@ int inverse_rowmap_items(const ChunkItem* items, const ChunkAux* aux, int n_item
 int inverse_rowmap(const int* rowmap, long long row_base, long long n_rows, long long M, int* inv, int num_sms,
                    cudaStream_t stream);
 
+// The fusion of one element, model/imf_vad.py:134-144 in its exact op order, every product / sum rounded separately
+// like ATen: w_i, w_e and the returned fused value.  fuse, fuse_rows and heads_fuse all compute it here, which keeps
+// them bit-identical with one another.
+__device__ __forceinline__ float fuse_one(float mu_i, float mu_e, float lv_i, float lv_e, float factor, float eps,
+                                          float& w_i, float& w_e) {
+  const float ri = __fmul_rn(factor, expf(-lv_i));
+  const float re = __fmul_rn(factor, expf(-lv_e));
+  const float den = __fadd_rn(__fadd_rn(ri, re), eps);
+  w_i = __fdiv_rn(ri, den);
+  w_e = __fdiv_rn(re, den);
+  return __fadd_rn(__fmul_rn(w_i, mu_i), __fmul_rn(w_e, mu_e));
+}
+
 // model/imf_vad.py:130-144.  n elements; fused / fused_hi / fused_lo optional.
 int fuse(const float* mu_i, const float* mu_e, const float* lv_i, const float* lv_e, long long n, float factor,
          float eps, float* w_i, float* w_e, float* fused, bf16* fused_hi, bf16* fused_lo, int num_sms,
-         cudaStream_t stream, int hi_fp16 = 0 /* fused_hi receives fp16 instead of bf16 */);
+         cudaStream_t stream, int hi_fp16 = 0 /* fused_hi / fused_lo receive fp16 instead of bf16 */);
 
 // The same with one warp per row, which also writes the row means of w_i / w_e (what the reference's evaluation loop keeps
 // of them, train/ucf_test.py:124-131) instead of the [rows, D] weight tensors.

@@ -2,7 +2,6 @@
 // contraction in IEEE fp32 like the reference, model/imf_vad.py:109-150) and the on-device yardstick
 // for the tcgen05 path.  Classic 64x64x16 smem tiling, 128 threads, 4x8 register micro-tiles.
 #include "common.cuh"
-#include "epilogue.cuh"
 #include "gemm.cuh"
 
 namespace iefvad {
@@ -10,6 +9,39 @@ namespace iefvad {
 namespace {
 
 constexpr int SBM = 64, SBN = 64, SBK = 16;
+
+// Store NC (multiple of 4, <= 32) consecutive fp32 columns [col0, col0+NC) of one output row.  `v` holds the raw
+// accumulators.  Every pointer dereferenced here is 16-byte aligned because col0 % 4 == 0 and all leading dimensions
+// are multiples of 8.
+template <int NC>
+__device__ __forceinline__ void epi_store_row(const EpiParams& p, long long row, int col0, float* v) {
+#pragma unroll
+  for (int j = 0; j < NC; ++j) {
+    float x = v[j];
+    if (p.bias) x += __ldg(p.bias + col0 + j);
+    v[j] = apply_act(x, p.act);
+  }
+  if (p.resid) {
+    const float* r = p.resid + row * p.ld_resid + col0;
+#pragma unroll
+    for (int j = 0; j < NC; j += 4) {
+      const float4 rv = *reinterpret_cast<const float4*>(r + j);
+      v[j + 0] = rv.x + p.alpha * v[j + 0];
+      v[j + 1] = rv.y + p.alpha * v[j + 1];
+      v[j + 2] = rv.z + p.alpha * v[j + 2];
+      v[j + 3] = rv.w + p.alpha * v[j + 3];
+    }
+  } else if (p.alpha != 1.f) {
+#pragma unroll
+    for (int j = 0; j < NC; ++j) v[j] *= p.alpha;
+  }
+  if (p.out_f32) {
+    float* o = (col0 < p.split_col) ? p.out_f32 + row * p.ld_f32 + col0
+                                    : p.out_f32_b + row * p.ld_f32 + (col0 - p.split_col);
+#pragma unroll
+    for (int j = 0; j < NC; j += 4) *reinterpret_cast<float4*>(o + j) = make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]);
+  }
+}
 
 __global__ void __launch_bounds__(128)
 gemm_simt_kernel(const float* __restrict__ A, int lda, const float* __restrict__ W, int ldw, int M, int N, int K,
@@ -70,6 +102,7 @@ int gemm_simt(const float* A, int lda, const float* W, int ldw, int M, int N, in
   IEF_CHECK(M > 0 && N > 0 && K > 0, "gemm_simt: empty problem");
   IEF_CHECK(K % SBK == 0 && N % 8 == 0 && lda % 4 == 0 && ldw % 4 == 0,
             "gemm_simt: need K %% 16 == 0, N %% 8 == 0, lda/ldw %% 4 == 0 (K=%d N=%d)", K, N);
+  IEF_CHECK(ep.mode == EPI_ROWMAJOR && !ep.out_hi && !ep.resid_h16, "gemm_simt: the epilogue writes fp32 rows only");
   dim3 grid((M + SBM - 1) / SBM, (N + SBN - 1) / SBN);
   gemm_simt_kernel<<<grid, 128, 0, stream>>>(A, lda, W, ldw, M, N, K, ep);
   count_launches(1);

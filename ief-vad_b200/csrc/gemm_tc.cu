@@ -26,7 +26,6 @@
 #include <cstring>
 
 #include "common.cuh"
-#include "epilogue.cuh"
 #include "gemm.cuh"
 #include "tensormap.cuh"
 
@@ -348,12 +347,7 @@ gemm_tc_kernel(const __grid_constant__ TcMaps tm, int M, int N, int K, int nspli
         const float s = (which == 0) ? ep.qscale : 1.f;
         uint4 u[4];
 #pragma unroll
-        for (int g = 0; g < 4; ++g) {
-          u[g].x = pack_16x2(v[g * 8 + 0] * s, v[g * 8 + 1] * s, ep.hi_fp16);
-          u[g].y = pack_16x2(v[g * 8 + 2] * s, v[g * 8 + 3] * s, ep.hi_fp16);
-          u[g].z = pack_16x2(v[g * 8 + 4] * s, v[g * 8 + 5] * s, ep.hi_fp16);
-          u[g].w = pack_16x2(v[g * 8 + 6] * s, v[g * 8 + 7] * s, ep.hi_fp16);
-        }
+        for (int g = 0; g < 4; ++g) u[g] = pack_16x8(v + g * 8, ep.hi_fp16, s);
         if (!ep.qk_tma) {
           if (row < M) {
             bf16* dst = (which == 0 ? ep.q : ep.k) + ((b * ep.H + h) * ep.T + t) * (long long)ep.dhp + d0;
@@ -386,23 +380,9 @@ gemm_tc_kernel(const __grid_constant__ TcMaps tm, int M, int N, int K, int nspli
         if (R16) {
 #pragma unroll
           for (int g = 0; g < 4; ++g) {
-            const uint4 h4 = *reinterpret_cast<const uint4*>(rb + sw64(lane, g));
-            const uint32_t hw[4] = {h4.x, h4.y, h4.z, h4.w};
             float r[8];
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-              const float2 f = __half22float2(*reinterpret_cast<const __half2*>(&hw[q]));
-              r[2 * q] = f.x; r[2 * q + 1] = f.y;
-            }
-            if (ep.resid_lo) {
-              const uint4 l4 = *reinterpret_cast<const uint4*>(rb + kBfBox + sw64(lane, g));
-              const uint32_t lw[4] = {l4.x, l4.y, l4.z, l4.w};
-#pragma unroll
-              for (int q = 0; q < 4; ++q) {
-                const float2 f = __half22float2(*reinterpret_cast<const __half2*>(&lw[q]));
-                r[2 * q] += f.x; r[2 * q + 1] += f.y;
-              }
-            }
+            unpack_f16x8(*reinterpret_cast<const uint4*>(rb + sw64(lane, g)),
+                         ep.resid_lo ? reinterpret_cast<const uint4*>(rb + kBfBox + sw64(lane, g)) : nullptr, r);
 #pragma unroll
             for (int j = 0; j < 8; ++j) v[g * 8 + j] = fmaf(ep.alpha, v[g * 8 + j], r[j]);
           }
@@ -441,20 +421,7 @@ gemm_tc_kernel(const __grid_constant__ TcMaps tm, int M, int N, int K, int nspli
         for (int g = 0; g < 4; ++g) {
           uint32_t hi[4], lo[4];
 #pragma unroll
-          for (int q = 0; q < 4; ++q) {
-            const float a = v[g * 8 + 2 * q], b = v[g * 8 + 2 * q + 1];
-            if (ep.hi_fp16) {
-              const __half2 h2 = __floats2half2_rn(a, b);
-              hi[q] = *reinterpret_cast<const uint32_t*>(&h2);
-              const float2 hf = __half22float2(h2);
-              const __half2 l2 = __floats2half2_rn(a - hf.x, b - hf.y);     // fp16 remainder: hi + lo ~ 22 mantissa bits
-              lo[q] = *reinterpret_cast<const uint32_t*>(&l2);
-            } else {
-              const float ah = __bfloat162float(__float2bfloat16_rn(a)), bh = __bfloat162float(__float2bfloat16_rn(b));
-              hi[q] = pack_bf16x2(ah, bh);
-              lo[q] = pack_bf16x2(a - ah, b - bh);
-            }
-          }
+          for (int q = 0; q < 4; ++q) split_16x2(v[g * 8 + 2 * q], v[g * 8 + 2 * q + 1], ep.hi_fp16, hi[q], lo[q]);
           *reinterpret_cast<uint4*>(hb + sw64(lane, g)) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
           if (ep.has_lo) *reinterpret_cast<uint4*>(lb + sw64(lane, g)) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
         }

@@ -518,7 +518,7 @@ int transformer_blocks(float* xa, const ResBlockParams* blocks, int layers, int 
       at.q = q; at.k = k; at.vt = vt; at.out = ctx.hi; at.ldo = D;
       at.B = N; at.T = L; at.H = heads; at.dh = dh; at.dhp = dhp; at.Tpad = Tpad;
       at.attn_mask = attn_mask; at.key_pad = key_pad;
-      at.fp16 = f16; at.out_fp16 = f16;
+      at.fp16 = f16;
       IEF_TRY(attn_tc(at, st));
     }
     EpiParams e2;

@@ -6,13 +6,14 @@
 // half of tensor memory (N = 256 accumulator) and the event modality's into the other half, and the epilogue fuses them from
 // TMEM: 3 KB of x in, the 16-bit (hi, lo) pair of `fused` out - 4.5 KB per row.
 // Same arithmetic, instruction for instruction, as gemm_tc (fp16 operands, fp32 accumulation in k order, + bias) followed
-// by fuse_kernel (expf, IEEE division, separately rounded products): the pair is bit-identical to the three-launch form.
+// by fuse_kernel (the same fuse_one): the pair is bit-identical to the three-launch form.
 // TMEM is full (2 x 256 columns), so the epilogue of a tile does not overlap the MMAs of the next one - but the operand ring
 // (6 stages) refills meanwhile, and the kernel still moves a sixth of the bytes.  Sixteen epilogue warps (four per scheduler,
 // one 32-feature chunk each, 8 features at a time to stay inside 96 registers) keep that exposed epilogue short: it is bound
 // by the CUDA cores (expf and IEEE division per element).
 #include <cstring>
 
+#include "elementwise.cuh"
 #include "heads_fuse.cuh"
 #include "tensormap.cuh"
 
@@ -191,26 +192,14 @@ heads_fuse_kernel(const __grid_constant__ CUtensorMap txi, const __grid_constant
 #pragma unroll
           for (int e = 0; e < 4; ++e) {
             const int i = g * 4 + e;
-            // exact op order of model/imf_vad.py:134-144 (== fuse_kernel), every product / sum rounded separately
-            const float mui = __fadd_rn(mi[i], b0[e]), lvi = __fadd_rn(li[i], b1[e]);
-            const float mue = __fadd_rn(me[i], b2[e]), lve = __fadd_rn(le[i], b3[e]);
-            const float ri = __fmul_rn(p.factor, expf(-lvi));
-            const float re = __fmul_rn(p.factor, expf(-lve));
-            const float den = __fadd_rn(__fadd_rn(ri, re), p.eps);
-            const float wi = __fdiv_rn(ri, den), we = __fdiv_rn(re, den);
-            f[i] = __fadd_rn(__fmul_rn(wi, mui), __fmul_rn(we, mue));
+            float wi, we;
+            f[i] = fuse_one(__fadd_rn(mi[i], b0[e]), __fadd_rn(me[i], b2[e]), __fadd_rn(li[i], b1[e]),
+                            __fadd_rn(le[i], b3[e]), p.factor, p.eps, wi, we);
           }
         }
         uint32_t hi[4];
 #pragma unroll
-        for (int q = 0; q < 4; ++q) {
-          const float a = f[2 * q], b = f[2 * q + 1];
-          const __half2 h2 = __floats2half2_rn(a, b);
-          hi[q] = *reinterpret_cast<const uint32_t*>(&h2);
-          const float2 hf = __half22float2(h2);
-          const __half2 l2 = __floats2half2_rn(a - hf.x, b - hf.y);
-          lo_keep[step * 4 + q] = *reinterpret_cast<const uint32_t*>(&l2);
-        }
+        for (int q = 0; q < 4; ++q) split_16x2(f[2 * q], f[2 * q + 1], 1, hi[q], lo_keep[step * 4 + q]);
         *reinterpret_cast<uint4*>(Bx + sw64(lane, step)) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
       }
       fence_proxy_async_smem();

@@ -110,7 +110,8 @@ int Model::init(int embed_dim, int num_heads, int layers, int refine_steps, floa
   IEF_CUDA(cudaGetDevice(&device));
   IEF_CUDA(cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, device));
 
-  // ---- carve one fp32 arena (+ bf16 hi / lo arenas mirroring the weight matrices)
+  // ---- carve one fp32 arena (+ bf16 hi / lo and fp16 arenas mirroring the weight matrices).  The encoder's in- and
+  // out-projections run one 16-bit operand pass in every plan, so only the heads and refinement weights keep a bf16 lo.
   struct Want { std::string key; long long numel; bool is_weight; float** dst; bf16** hi; bf16** lo; bf16** h16 = nullptr; };
   std::vector<Want> wants;
   const char* mods[2] = {"image", "event"};
@@ -129,11 +130,11 @@ int Model::init(int embed_dim, int num_heads, int layers, int refine_steps, floa
       Linear& op = out_proj[m][i];
       ip.out = 3 * D; ip.in = D; op.out = D; op.in = D;
       snprintf(buf, sizeof(buf), "temporal.%s_attn_layers.%d.in_proj_weight", mods[m], i);
-      wants.push_back({buf, 3LL * D * D, true, &ip.w, &ip.w_hi, &ip.w_lo, &ip.w_h16});
+      wants.push_back({buf, 3LL * D * D, true, &ip.w, &ip.w_hi, nullptr, &ip.w_h16});
       snprintf(buf, sizeof(buf), "temporal.%s_attn_layers.%d.in_proj_bias", mods[m], i);
       wants.push_back({buf, 3LL * D, false, &ip.b, nullptr, nullptr});
       snprintf(buf, sizeof(buf), "temporal.%s_attn_layers.%d.out_proj.weight", mods[m], i);
-      wants.push_back({buf, 1LL * D * D, true, &op.w, &op.w_hi, &op.w_lo, &op.w_h16});
+      wants.push_back({buf, 1LL * D * D, true, &op.w, &op.w_hi, nullptr, &op.w_h16});
       snprintf(buf, sizeof(buf), "temporal.%s_attn_layers.%d.out_proj.bias", mods[m], i);
       wants.push_back({buf, D, false, &op.b, nullptr, nullptr});
       snprintf(buf, sizeof(buf), "temporal.%s_norms.%d.weight", mods[m], i);
@@ -164,20 +165,21 @@ int Model::init(int embed_dim, int num_heads, int layers, int refine_steps, floa
   wants.push_back({"temporal.classifier.weight", D, false, &cls_w, nullptr, nullptr});
   wants.push_back({"temporal.classifier.bias", 1, false, &cls_b, nullptr, nullptr});
 
-  size_t f32_elems = 0, bf_elems = 0, h16_elems = 0;
+  size_t f32_elems = 0, bf_elems = 0, lo_elems = 0, h16_elems = 0;
   for (auto& w : wants) {
     f32_elems += align_up(size_t(w.numel), 64);
     if (w.is_weight) bf_elems += align_up(size_t(w.numel), 64);
+    if (w.lo) lo_elems += align_up(size_t(w.numel), 64);
     if (w.h16) h16_elems += align_up(size_t(w.numel), 64);
   }
   IEF_TRY(params_h16.reserve((h16_elems ? h16_elems : 64) * sizeof(bf16)));
   IEF_TRY(params_f32.reserve(f32_elems * sizeof(float)));
   IEF_TRY(params_hi.reserve(bf_elems * sizeof(bf16)));
-  IEF_TRY(params_lo.reserve(bf_elems * sizeof(bf16)));
+  IEF_TRY(params_lo.reserve(lo_elems * sizeof(bf16)));
   IEF_CUDA(cudaMemset(params_f32.p, 0, params_f32.bytes));
   IEF_TRY(status.reserve(4 * sizeof(int)));
   IEF_CUDA(cudaMemset(status.p, 0, status.bytes));
-  size_t fo = 0, bo = 0, ho = 0;
+  size_t fo = 0, bo = 0, lo_o = 0, ho = 0;
   for (auto& w : wants) {
     *w.dst = params_f32.as<float>() + fo;
     fo += align_up(size_t(w.numel), 64);
@@ -186,10 +188,13 @@ int Model::init(int embed_dim, int num_heads, int layers, int refine_steps, floa
     s.numel = w.numel;
     if (w.is_weight) {
       *w.hi = params_hi.as<bf16>() + bo;
-      *w.lo = params_lo.as<bf16>() + bo;
       s.hi = *w.hi;
-      s.lo = *w.lo;
       bo += align_up(size_t(w.numel), 64);
+    }
+    if (w.lo) {
+      *w.lo = params_lo.as<bf16>() + lo_o;
+      s.lo = *w.lo;
+      lo_o += align_up(size_t(w.numel), 64);
     }
     if (w.h16) {
       *w.h16 = params_h16.as<bf16>() + ho;
@@ -452,7 +457,7 @@ int Model::forward(const void* img, const void* ev, int in_dtype, long long B, l
           at.q = qb.as<bf16>(); at.k = kb.as<bf16>(); at.vt = vtb.as<bf16>(); at.out = h_hi.as<bf16>(); at.ldo = D;
           at.B = Bs; at.T = int(T); at.H = H; at.dh = dh; at.dhp = dhq; at.Tpad = Tpad;
           if (dedup) { at.B = 1; at.T = int(Me); at.Tpad = int(Me); at.items = items_dev.as<int>(); at.n_chunks = n_items; }
-          at.fp16 = f16; at.out_fp16 = f16;
+          at.fp16 = f16;
           if (direct_compact && last && !ln_fused) at.row_out = inv_map.as<int>();
           IEF_PROF(KC_ATTN_TC, attn_flops, attn_tc(at, stream));
           if (ln_fused) {

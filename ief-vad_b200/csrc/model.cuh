@@ -1,5 +1,5 @@
 // Device-resident IEF-VAD model: fp32 master parameters (state_dict layout of model/imf_vad.py:69-107),
-// packed bf16 hi/lo copies for the tensor-core plans, and a grow-only activation workspace.
+// packed 16-bit copies for the tensor-core plans, and a grow-only activation workspace.
 #pragma once
 #include <string>
 #include <unordered_map>
@@ -35,8 +35,8 @@ struct Linear {          // y = x W^T + b, W [out, in]
   float* w = nullptr;    // fp32 master
   float* b = nullptr;
   bf16* w_hi = nullptr;
-  bf16* w_lo = nullptr;
-  bf16* w_h16 = nullptr;  // fp16 copy (16-bit storage), refinement Linears only
+  bf16* w_lo = nullptr;   // bf16(w - hi) for plan B's 3-term split: heads and refinement Linears only
+  bf16* w_h16 = nullptr;  // fp16 copy (16-bit storage)
   int out = 0, in = 0;
 };
 
@@ -44,8 +44,8 @@ struct ParamSlot {
   float* dst = nullptr;
   long long numel = 0;
   bf16* hi = nullptr;    // packed copies refreshed on upload (weights only)
-  bf16* lo = nullptr;
-  bf16* h16 = nullptr;   // fp16 copy (refinement weights)
+  bf16* lo = nullptr;    // heads and refinement weights only
+  bf16* h16 = nullptr;   // fp16 copy
   bool loaded = false;
 };
 
@@ -105,8 +105,6 @@ struct Model {
   DevBuf status;                         // int[4]: [0] bit 0 = a non-finite logit was produced since the last check
   std::vector<ChunkItem> items_host;     // packed-row layout of the current slab (valid-rows mode, see forward)
   std::vector<ChunkAux> aux_host;
-  long long ws_rows = 0;
-  int ws_T = 0;
 
   int init(int embed_dim, int heads, int layers, int refine_steps, float lambda, int noise_model, float nu, float epsilon);
   int set_param(const char* key, const float* dptr, long long numel, cudaStream_t stream);

@@ -443,16 +443,7 @@ outproj_ln_kernel(const __grid_constant__ CUtensorMap ta, const __grid_constant_
         for (int g = 0; g < 4; ++g) {
           uint32_t hi[4], lo[4];
 #pragma unroll
-          for (int q = 0; q < 4; ++q) {
-            const float a = v[g * 8 + 2 * q], b = v[g * 8 + 2 * q + 1];
-            const __half2 h2 = __floats2half2_rn(a, b);
-            hi[q] = *reinterpret_cast<const uint32_t*>(&h2);
-            if (OUT_LO) {
-              const float2 hf = __half22float2(h2);
-              const __half2 l2 = __floats2half2_rn(a - hf.x, b - hf.y);
-              lo[q] = *reinterpret_cast<const uint32_t*>(&l2);
-            }
-          }
+          for (int q = 0; q < 4; ++q) split_16x2(v[g * 8 + 2 * q], v[g * 8 + 2 * q + 1], 1, hi[q], lo[q]);
           *reinterpret_cast<uint4*>(Hb + sw64(lane, g)) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
           if (OUT_LO) *reinterpret_cast<uint4*>(Lb + sw64(lane, g)) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
         }

@@ -397,29 +397,18 @@ refine_chain_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_consta
         const float4* bp = reinterpret_cast<const float4*>(b2 + col0);
 #pragma unroll
         for (int g = 0; g < 8; ++g) {
-          const uint32_t hw[4] = {h4[g].x, h4[g].y, h4[g].z, h4[g].w}, lw[4] = {l4[g].x, l4[g].y, l4[g].z, l4[g].w};
           const float4 ba = __ldg(bp + 2 * g), bb = __ldg(bp + 2 * g + 1);
           const float bias[8] = {ba.x, ba.y, ba.z, ba.w, bb.x, bb.y, bb.z, bb.w};
+          float x[8];
+          unpack_f16x8(h4[g], &l4[g], x);
+          // the same operation order as the two-launch epilogue: (acc + bias), then fma(-lambda, ., hi + lo)
 #pragma unroll
-          for (int e = 0; e < 4; ++e) {
-            const float2 fh = __half22float2(*reinterpret_cast<const __half2*>(&hw[e]));
-            const float2 fl = __half22float2(*reinterpret_cast<const __half2*>(&lw[e]));
-            // the same operation order as the two-launch epilogue: (acc + bias), then fma(-lambda, ., hi + lo)
-            v[8 * g + 2 * e] = fmaf(nlam, v[8 * g + 2 * e] + bias[2 * e], fh.x + fl.x);
-            v[8 * g + 2 * e + 1] = fmaf(nlam, v[8 * g + 2 * e + 1] + bias[2 * e + 1], fh.y + fl.y);
-          }
+          for (int e = 0; e < 8; ++e) v[8 * g + e] = fmaf(nlam, v[8 * g + e] + bias[e], x[e]);
           if (!last) {                            // the new pair, kept in the registers the old one came in
-            uint32_t nh[4], nl[4];
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-              const __half2 h2 = __floats2half2_rn(v[8 * g + 2 * e], v[8 * g + 2 * e + 1]);
-              const float2 hfl = __half22float2(h2);
-              const __half2 l2 = __floats2half2_rn(v[8 * g + 2 * e] - hfl.x, v[8 * g + 2 * e + 1] - hfl.y);
-              nh[e] = *reinterpret_cast<const uint32_t*>(&h2);
-              nl[e] = *reinterpret_cast<const uint32_t*>(&l2);
-            }
-            h4[g] = make_uint4(nh[0], nh[1], nh[2], nh[3]);
-            l4[g] = make_uint4(nl[0], nl[1], nl[2], nl[3]);
+            split_16x2(v[8 * g], v[8 * g + 1], 1, h4[g].x, l4[g].x);
+            split_16x2(v[8 * g + 2], v[8 * g + 3], 1, h4[g].y, l4[g].y);
+            split_16x2(v[8 * g + 4], v[8 * g + 5], 1, h4[g].z, l4[g].z);
+            split_16x2(v[8 * g + 6], v[8 * g + 7], 1, h4[g].w, l4[g].w);
           }
         }
         // out through the tiles the chunk came in (every lane rewrites exactly the slots it read): two bulk tensor stores;

@@ -60,7 +60,7 @@ void iefvad_model_destroy(iefvad_model* m);
 
 /* Upload one parameter by its reference state_dict key (e.g. "temporal.image_attn_layers.0.in_proj_weight",
  * "temporal.refinement_blocks.3.2.bias"; the 78 tensors of model/imf_vad.py:69-107).  `data`: device fp32,
- * contiguous, `numel` elements.  bf16 hi/lo copies are refreshed on the given stream. */
+ * contiguous, `numel` elements.  The 16-bit operand copies of a weight are refreshed on the given stream. */
 int iefvad_model_set_param(iefvad_model* m, const char* key, const float* data, int64_t numel, void* stream);
 
 int iefvad_model_set_plan(iefvad_model* m, int plan);
