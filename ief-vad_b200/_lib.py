@@ -49,6 +49,7 @@ _SIGS = {
     "iefvad_linear": (_i, [_vp] * 4 + [_f, _i, _i64, _i, _i, _i, _i, _vp, _vp]),
     "iefvad_outproj_ln": (_i, [_vp] * 8 + [_f, _i64, _vp, _vp, _vp, _vp]),
     "iefvad_mha": (_i, [_vp] * 5 + [_i64, _i64, _i, _i, _vp, _vp, _i, _vp, _vp]),
+    "iefvad_attention_core": (_i, [_vp] * 3 + [_i64, _i64, _i, _i, _i, _i64] + [_vp] * 4 + [_i, _i, _vp, _i64, _vp]),
     "iefvad_classifier": (_i, [_vp, _i64, _i, _vp, _vp, _vp, _vp, _vp]),
     "iefvad_mil_topk_mean": (_i, [_vp, _vp, _i64, _i64, _i, _vp, _vp, _i, _vp]),
     "iefvad_clas2": (_i, [_vp, _vp, _i64, _vp, _i64, _i64, _vp, _vp, _vp]),

@@ -28,7 +28,6 @@ namespace {
 constexpr float kLog2e = 1.4426950408889634f;
 constexpr int kSoftmaxWarps = 16;
 constexpr int kThreads = (kSoftmaxWarps + 2) * 32;
-constexpr float kNone = -30000.f;        // "no key yet" in the integer log2 domain: 2^(kNone - anything sane) == 0
 
 template <int DH, int DHP>
 struct LongCfg {
@@ -198,7 +197,10 @@ attn_long_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
       const int bh = item / q_pairs, qp = item - bh * q_pairs;
       const int b = bh / H, h = bh - b * H;
       const int tq = qp * 256 + t * 128 + r;
-      float run = kNone;          // running row maximum (integer, log2 domain), the same in both halves of the row
+      // running row maximum (integer, log2 domain), the same in both halves of the row.  It starts at -inf, not at a
+      // finite "no key yet" value: scores may lie anywhere in fp32 (below -20 000 with fp16 operands), and half 0 of
+      // every block holds a key, so the first block makes it finite
+      float run = -INFINITY;
       float l = 0.f;              // this half's share of the row sum, in units of 2^run
 
       for (int j = 0; j < nb; ++j, ++n) {
@@ -221,7 +223,7 @@ attn_long_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
           for (int i = 0; i < 64; ++i)
             if (k_lo + i < T) mx = fmaxf(mx, v[i]);
         }
-        const float mloc = (mx == -INFINITY) ? kNone : ceilf(mx * kLog2e);
+        const float mloc = ceilf(mx * kLog2e);                        // -inf for an empty half
         *slot(par, hf) = mloc;
         // ---- P = 2^(S log2e - mloc) in (0, 1], packed; nothing here depends on the other half or on earlier blocks
         uint32_t pk[32];

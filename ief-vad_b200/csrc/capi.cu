@@ -475,7 +475,7 @@ int iefvad_mha(const float* x, const float* in_w, const float* in_b, const float
                int plan, float* out, void* stream) {
   IEF_CHECK(x && in_w && in_b && out_w && out_b && out, "iefvad_mha: null argument");
   IEF_CHECK(num_heads > 0 && D % num_heads == 0, "iefvad_mha: heads must divide D");
-  IEF_CHECK(plan >= -1 && plan <= 1, "iefvad_mha: plan must be -1, 0 or 1");
+  IEF_CHECK(plan >= -1 && plan <= 2, "iefvad_mha: plan must be -1 (fp32), 0 (bf16), 1 (split-bf16) or 2 (fp16)");
   IEF_CHECK(B >= 0 && T >= 0 && B * T < (1LL << 31), "iefvad_mha: bad sizes");
   if (B == 0 || T == 0) return IEFVAD_OK;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -508,27 +508,64 @@ int iefvad_mha(const float* x, const float* in_w, const float* in_b, const float
   IEF_TRY(sc.get(&k, size_t(M) * num_heads * dhp * 2));
   IEF_TRY(sc.get(&vt, size_t(B) * num_heads * dh * Tpad * 2));
   IEF_TRY(sc.get(&ctx, size_t(M) * D * 2));
-  IEF_TRY(ingest(x, IEFVAD_DT_F32, M * D, nullptr, (bf16*)xh, (bf16*)xl, sms, st));
-  IEF_TRY(ingest(in_w, IEFVAD_DT_F32, 3LL * D * D, nullptr, (bf16*)iwh, (bf16*)iwl, sms, st));
-  IEF_TRY(ingest(out_w, IEFVAD_DT_F32, 1LL * D * D, nullptr, (bf16*)owh, (bf16*)owl, sms, st));
+  // plan 2 is the default model plan HH's arithmetic: fp16 operands everywhere, and on the unmasked short-sequence kernel
+  // q / k rows of d_h rather than d_h padded to 64 (model.cu, Model::forward)
+  const int f16 = plan == 2 ? 1 : 0;
+  const int dhq = (f16 && T <= 256 && dh % 32 == 0 && !attn_mask && !key_padding_mask) ? dh : dhp;
+  if (f16) {
+    IEF_TRY(to_half(x, M * D, xh, sms, st));
+    IEF_TRY(to_half(in_w, 3LL * D * D, iwh, sms, st));
+    IEF_TRY(to_half(out_w, 1LL * D * D, owh, sms, st));
+  } else {
+    IEF_TRY(ingest(x, IEFVAD_DT_F32, M * D, nullptr, (bf16*)xh, (bf16*)xl, sms, st));
+    IEF_TRY(ingest(in_w, IEFVAD_DT_F32, 3LL * D * D, nullptr, (bf16*)iwh, (bf16*)iwl, sms, st));
+    IEF_TRY(ingest(out_w, IEFVAD_DT_F32, 1LL * D * D, nullptr, (bf16*)owh, (bf16*)owl, sms, st));
+  }
   EpiParams e1;
-  e1.mode = EPI_QKV; e1.bias = in_b; e1.q = (bf16*)q; e1.k = (bf16*)k; e1.vt = (bf16*)vt;
-  e1.T = int(T); e1.H = num_heads; e1.dh = dh; e1.dhp = dhp; e1.Tpad = Tpad; e1.D = D;
+  e1.mode = EPI_QKV; e1.bias = in_b; e1.q = (bf16*)q; e1.k = (bf16*)k; e1.vt = (bf16*)vt; e1.hi_fp16 = f16;
+  e1.T = int(T); e1.H = num_heads; e1.dh = dh; e1.dhp = dhq; e1.Tpad = Tpad; e1.D = D;
   e1.qscale = 1.0f / sqrtf(float(dh));
   GemmTcArgs g1;
   g1.A_hi = (bf16*)xh; g1.A_lo = (bf16*)xl; g1.W_hi = (bf16*)iwh; g1.W_lo = (bf16*)iwl;
-  g1.M = int(M); g1.N = 3 * D; g1.K = D; g1.lda = D; g1.ldw = D; g1.nsplit = plan == 1 ? 3 : 1;
+  g1.M = int(M); g1.N = 3 * D; g1.K = D; g1.lda = D; g1.ldw = D; g1.nsplit = plan == 1 ? 3 : 1; g1.fp16 = f16;
   IEF_TRY(gemm_tc(g1, e1, sms, st));
   AttnTcArgs at;
   at.q = (bf16*)q; at.k = (bf16*)k; at.vt = (bf16*)vt; at.out = (bf16*)ctx; at.ldo = D;
-  at.B = int(B); at.T = int(T); at.H = num_heads; at.dh = dh; at.dhp = dhp; at.Tpad = Tpad;
-  at.attn_mask = attn_mask; at.key_pad = key_padding_mask;
+  at.B = int(B); at.T = int(T); at.H = num_heads; at.dh = dh; at.dhp = dhq; at.Tpad = Tpad;
+  at.attn_mask = attn_mask; at.key_pad = key_padding_mask; at.fp16 = f16;
   IEF_TRY(attn_tc(at, st));
   EpiParams e2;
   e2.bias = out_b; e2.out_f32 = out; e2.ld_f32 = D;
   GemmTcArgs g2;
-  g2.A_hi = (bf16*)ctx; g2.W_hi = (bf16*)owh; g2.M = int(M); g2.N = D; g2.K = D; g2.lda = D; g2.ldw = D;
+  g2.A_hi = (bf16*)ctx; g2.W_hi = (bf16*)owh; g2.M = int(M); g2.N = D; g2.K = D; g2.lda = D; g2.ldw = D; g2.fp16 = f16;
   return gemm_tc(g2, e2, sms, st);
+}
+
+int iefvad_attention_core(const void* q, const void* k, const void* vt, int64_t B, int64_t T, int H, int dh, int dhp,
+                          int64_t Tpad, const float* attn_mask, const uint8_t* key_pad, const int32_t* row_out,
+                          const int32_t* items, int n_chunks, int fp16, void* out, int64_t ldo, void* stream) {
+  IEF_CHECK(q && k && vt && out, "iefvad_attention_core: null argument");
+  IEF_CHECK(((reinterpret_cast<uintptr_t>(q) | reinterpret_cast<uintptr_t>(k) | reinterpret_cast<uintptr_t>(vt) |
+              reinterpret_cast<uintptr_t>(out)) & 15) == 0, "iefvad_attention_core: q, k, vt and out must be 16-byte aligned");
+  IEF_CHECK(B > 0 && T > 0 && H > 0 && B * H * T < (1LL << 31), "iefvad_attention_core: bad sizes B=%lld T=%lld H=%d",
+            (long long)B, (long long)T, H);
+  IEF_CHECK(dh > 0 && dhp >= dh && dhp % 8 == 0, "iefvad_attention_core: need 0 < dh <= dhp, dhp %% 8 == 0 (dh=%d dhp=%d)",
+            dh, dhp);
+  IEF_CHECK(Tpad >= T && Tpad % 8 == 0 && Tpad < (1LL << 31), "iefvad_attention_core: Tpad=%lld must be a multiple of 8 "
+            "and >= T=%lld", (long long)Tpad, (long long)T);
+  IEF_CHECK(ldo >= int64_t(H) * dh && ldo % 8 == 0 && ldo < (1LL << 31), "iefvad_attention_core: ldo=%lld must be a "
+            "multiple of 8 and >= H * dh", (long long)ldo);
+  IEF_CHECK(fp16 == 0 || fp16 == 1, "iefvad_attention_core: fp16 must be 0 (bf16) or 1 (fp16)");
+  IEF_CHECK(n_chunks >= 0 && (items != nullptr) == (n_chunks > 0), "iefvad_attention_core: items and n_chunks > 0 go "
+            "together");
+  IEF_CHECK(!items || (B == 1 && !attn_mask && !key_pad), "iefvad_attention_core: ragged items need B = 1 and no masks");
+  AttnTcArgs at;
+  at.q = static_cast<const bf16*>(q); at.k = static_cast<const bf16*>(k); at.vt = static_cast<const bf16*>(vt);
+  at.out = static_cast<bf16*>(out); at.ldo = int(ldo);
+  at.B = int(B); at.T = int(T); at.H = H; at.dh = dh; at.dhp = dhp; at.Tpad = int(Tpad);
+  at.attn_mask = attn_mask; at.key_pad = key_pad; at.fp16 = fp16; at.row_out = row_out;
+  at.items = items; at.n_chunks = n_chunks;
+  return attn_tc(at, static_cast<cudaStream_t>(stream));
 }
 
 int iefvad_classifier(const float* x, int64_t rows, int dim, const float* w, const float* bias, float* logits,

@@ -10,7 +10,7 @@ import torch
 
 from . import _lib
 
-PLAN_CODES = {"fp32": -1, "bf16": 0, "split": 1, "fp16": 2}      # fp16: iefvad_linear, iefvad_transformer, clip
+PLAN_CODES = {"fp32": -1, "bf16": 0, "split": 1, "fp16": 2}      # fp16: linear, mha, iefvad_transformer, clip
 ACTS = {None: 0, "none": 0, "relu": 1, "quickgelu": 2}
 
 
@@ -107,6 +107,37 @@ def mha(x, in_w, in_b, out_w, out_b, num_heads: int, attn_mask=None, key_padding
         _lib.check(_lib.lib.iefvad_mha(x.data_ptr(), in_w.data_ptr(), in_b.data_ptr(), out_w.data_ptr(),
                                        out_b.data_ptr(), B, T, D, num_heads, _lib.ptr(am), _lib.ptr(kp),
                                        PLAN_CODES[plan], out.data_ptr(), _stream(x)))
+    return out
+
+
+def attention_core(q, k, vt, attn_mask=None, key_padding_mask=None, row_out=None, items=None, out=None):
+    """softmax(q k^T) v on the tensor-core attention kernels (iefvad_attention_core), in their own layouts.
+    q, k [B, H, T, dhp] and vt [B, H, dh, Tpad], all fp16 or all bf16 (the kernels run in that format); q is already
+    scaled by dh^-1/2.  attn_mask [T, T] additive, key_padding_mask [B, T] (True = ignore), row_out int32 [B*T] (output
+    row per query row, < 0 = dropped), items int32 [n_chunks, 4] ragged rows (B = 1).  out: [rows, ldo] tensor of the
+    operands' dtype that receives head h in columns [h dh, (h+1) dh), untouched elsewhere; default [B*T, H*dh] zeros."""
+    if q.dtype not in (torch.float16, torch.bfloat16) or k.dtype != q.dtype or vt.dtype != q.dtype:
+        raise RuntimeError(f"attention_core: q, k and vt must all be fp16 or all bf16, got {q.dtype}, {k.dtype}, {vt.dtype}")
+    for name, t in (("q", q), ("k", k), ("vt", vt)):
+        if not t.is_cuda or not t.is_contiguous() or t.dim() != 4:
+            raise RuntimeError(f"attention_core: {name} must be a contiguous 4-d CUDA tensor")
+    B, H, T, dhp = q.shape
+    dh, Tpad = vt.shape[2], vt.shape[3]
+    if tuple(k.shape) != (B, H, T, dhp) or tuple(vt.shape[:2]) != (B, H):
+        raise RuntimeError(f"attention_core: shapes q {list(q.shape)}, k {list(k.shape)}, vt {list(vt.shape)} disagree")
+    if out is None:
+        out = torch.zeros((B * T, H * dh), dtype=q.dtype, device=q.device)
+    if out.dtype != q.dtype or out.dim() != 2 or out.stride(1) != 1:
+        raise RuntimeError("attention_core: out must be a [rows, ldo] tensor of the operands' dtype with unit column stride")
+    am = _f32c(attn_mask, "attention_core") if attn_mask is not None else None
+    kp = key_padding_mask.to(torch.uint8).contiguous() if key_padding_mask is not None else None
+    ro = row_out.to(torch.int32).contiguous() if row_out is not None else None
+    it = items.to(torch.int32).contiguous() if items is not None else None
+    with torch.cuda.device(q.device):
+        _lib.check(_lib.lib.iefvad_attention_core(q.data_ptr(), k.data_ptr(), vt.data_ptr(), B, T, H, dh, dhp, Tpad,
+                                                  _lib.ptr(am), _lib.ptr(kp), _lib.ptr(ro), _lib.ptr(it),
+                                                  0 if it is None else it.shape[0], int(q.dtype == torch.float16),
+                                                  out.data_ptr(), out.stride(0), _stream(q)))
     return out
 
 

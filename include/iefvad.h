@@ -182,10 +182,27 @@ int iefvad_outproj_ln(const float* ctx, const float* w, const float* bias, const
 
 /* nn.MultiheadAttention(batch_first=True)(x, x, x)[0] in eval mode (model/imf_vad.py:115; torch/nn/functional.py:6244).
  * x [B, T, D] fp32; in_w [3D, D], in_b [3D], out_w [D, D], out_b [D].  attn_mask: optional additive [T, T] fp32;
- * key_padding_mask: optional [B, T] uint8 (non-zero = ignore).  plan as for iefvad_linear. */
+ * key_padding_mask: optional [B, T] uint8 (non-zero = ignore).  plan as for iefvad_linear; plan 2 runs the default model
+ * plan HH's arithmetic (fp16 projections and fp16 attention, unpadded q / k rows where the model uses them). */
 int iefvad_mha(const float* x, const float* in_w, const float* in_b, const float* out_w, const float* out_b,
                int64_t B, int64_t T, int D, int num_heads, const float* attn_mask, const uint8_t* key_padding_mask,
                int plan, float* out, void* stream);
+
+/* The tensor-core attention core softmax(q k^T) v on its own, in the kernels' layouts (what iefvad_mha and the forward
+ * run after the QKV projection).  fp16 = 1: q, k, vt and out hold fp16 and P is rounded to fp16; 0: bf16.
+ *   q, k [B, H, T, dhp] (q already scaled by dh^-1/2; columns dh..dhp are never read), vt [B, H, dh, Tpad] (columns
+ *   T..Tpad are never read).  out [B*T, ldo]: head h writes columns [h dh, (h+1) dh) of row b*T + t.
+ *   attn_mask: optional additive [T, T] fp32; key_pad: optional [B, T] uint8 (non-zero = ignore the key).
+ *   row_out: optional int32 [B*T]: query row b*T + t is stored in row row_out[b*T + t] of out, or dropped when < 0.
+ *   items / n_chunks: optional ragged rows (B = 1, no masks): int32 [n_chunks, 4] = {first row, rows (<= 256), valid
+ *   rows, mult}; chunk c attends its rows over its rows only, and when mult > 0 its last row (row `valid`) counts as
+ *   `mult` identical keys.  Row indices, also those of row_out, are then rows of the packed [H, T, dhp] tensors.
+ * T <= 256 or items without masks run the short-sequence kernel, T > 256 without masks the long-sequence kernel, and
+ * any mask the flash kernel.  Head dims (dh, dhp): (96, 128), (64, 64), (128, 128), (32, 64) on every kernel, and
+ * (96, 96), (32, 32) on the short-sequence kernel; other pairs fail with IEFVAD_ERR_INVALID before any launch. */
+int iefvad_attention_core(const void* q, const void* k, const void* vt, int64_t B, int64_t T, int H, int dh, int dhp,
+                          int64_t Tpad, const float* attn_mask, const uint8_t* key_pad, const int32_t* row_out,
+                          const int32_t* items, int n_chunks, int fp16, void* out, int64_t ldo, void* stream);
 
 /* Linear(embed_dim -> 1), model/imf_vad.py:150 (+ optional sigmoid). */
 int iefvad_classifier(const float* x, int64_t rows, int dim, const float* w, const float* bias, float* logits,

@@ -46,3 +46,21 @@ def test_invalid_arguments_fail_loudly_without_a_gpu():
     assert rc != 0 and "embed_dim" in _lib.last_error()
     rc = _lib.lib.iefvad_model_create(h, 768, 7, 2, 10, 0.5, 1, 8.0, 1e-8)   # heads do not divide
     assert rc != 0 and "num_heads" in _lib.last_error()
+
+
+def test_attention_core_rejects_malformed_arguments_without_a_gpu():
+    """iefvad_attention_core checks its arguments before it touches the device (the addresses here are never read)."""
+    from iefvad_b200 import _lib
+    p = 1 << 20
+    ok = dict(q=p, k=p, vt=p, B=1, T=64, H=2, dh=64, dhp=64, Tpad=64, attn_mask=None, key_pad=None, row_out=None,
+              items=None, n_chunks=0, fp16=1, out=p, ldo=128, stream=None)
+    bad = [
+        (dict(q=None), "null"), (dict(out=p + 8), "aligned"), (dict(T=0), "sizes"), (dict(dhp=32), "dhp"),
+        (dict(dhp=68), "dhp"), (dict(Tpad=60), "Tpad"), (dict(Tpad=68), "Tpad"), (dict(ldo=120), "ldo"),
+        (dict(ldo=132), "ldo"), (dict(fp16=2), "fp16"), (dict(items=p), "n_chunks"), (dict(n_chunks=3), "n_chunks"),
+        (dict(items=p, n_chunks=3, B=2), "items"), (dict(items=p, n_chunks=3, attn_mask=p), "items"),
+        (dict(items=p, n_chunks=3, key_pad=p), "items"),
+    ]
+    for change, word in bad:
+        rc = _lib.lib.iefvad_attention_core(*{**ok, **change}.values())
+        assert rc != 0 and word in _lib.last_error(), (change, rc, _lib.last_error())
