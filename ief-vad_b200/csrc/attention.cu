@@ -398,6 +398,10 @@ attn_simt_kernel(const float* __restrict__ qkv, float* __restrict__ out, int T, 
 
 }  // namespace
 
+int attn_qk_cols(const AttnTcArgs& a) {
+  return (attn_short_supported(a) && a.dh % 32 == 0) ? a.dh : (a.dh + 63) / 64 * 64;
+}
+
 int attn_tc(const AttnTcArgs& a, cudaStream_t stream) {
   IEF_CHECK(a.B > 0 && a.T > 0 && a.H > 0, "attn_tc: empty problem");
   IEF_CHECK(a.Tpad % 8 == 0 && a.Tpad >= a.T, "attn_tc: Tpad=%d must be a multiple of 8 and >= T=%d", a.Tpad, a.T);

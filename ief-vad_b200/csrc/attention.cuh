@@ -32,6 +32,11 @@ int attn_long(const AttnTcArgs& a, cudaStream_t stream);
 bool attn_short_supported(const AttnTcArgs& a);
 int attn_short(const AttnTcArgs& a, cudaStream_t stream);
 
+// Row width (dhp) of q / k that attn_tc reads for these arguments (dhp itself is not consulted): d_h where the
+// short-sequence kernel runs, which takes 32-column chunks under the 64-byte swizzle, else d_h padded to a multiple of
+// 64 for the 128-byte-swizzled kernels.
+int attn_qk_cols(const AttnTcArgs& a);
+
 // fp32 plan: qkv fp32 [B*T, 3*H*dh] (bias added, q unscaled) -> out fp32 [B*T, H*dh]
 int attn_simt(const float* qkv, float* out, int B, int T, int H, int dh, const float* attn_mask,
               const uint8_t* key_pad, cudaStream_t stream);

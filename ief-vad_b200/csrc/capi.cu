@@ -39,31 +39,6 @@ struct iefvad_model {
   uint64_t host_seq = 0;          // parts issued so far: the ping-pong of the input buffers continues across calls
 };
 
-namespace {
-
-int current_sms(int* out) {
-  int dev = 0;
-  IEF_CUDA(cudaGetDevice(&dev));
-  IEF_CUDA(cudaDeviceGetAttribute(out, cudaDevAttrMultiProcessorCount, dev));
-  return IEFVAD_OK;
-}
-
-struct Scratch {   // stream-ordered temporaries of the stand-alone operators (test surface, not the hot path)
-  cudaStream_t s;
-  std::vector<void*> ptrs;
-  explicit Scratch(cudaStream_t st) : s(st) { keep_async_pool(); }
-  ~Scratch() {
-    for (void* p : ptrs) cudaFreeAsync(p, s);
-  }
-  int get(void** out, size_t bytes) {
-    IEF_CUDA(cudaMallocAsync(out, bytes ? bytes : 16, s));
-    ptrs.push_back(*out);
-    return IEFVAD_OK;
-  }
-};
-
-}  // namespace
-
 extern "C" {
 
 int iefvad_abi_version(void) { return IEFVAD_ABI_VERSION; }
@@ -375,7 +350,7 @@ int iefvad_fuse(const float* mu_i, const float* mu_e, const float* logvar_i, con
                 float factor, float epsilon, float* w_i, float* w_e, float* fused, void* stream) {
   IEF_CHECK(mu_i && mu_e && logvar_i && logvar_e && w_i && w_e, "iefvad_fuse: null argument");
   int sms = 0;
-  IEF_TRY(current_sms(&sms));
+  IEF_TRY(device_sms(&sms));
   return fuse(mu_i, mu_e, logvar_i, logvar_e, n, factor, epsilon, w_i, w_e, fused, nullptr, nullptr, sms,
               static_cast<cudaStream_t>(stream));
 }
@@ -384,7 +359,7 @@ int iefvad_layernorm(const float* x, int64_t rows, int dim, const float* w1, con
                      const float* b2, float eps, float* out, void* stream) {
   IEF_CHECK(x && out, "iefvad_layernorm: null argument");
   int sms = 0;
-  IEF_TRY(current_sms(&sms));
+  IEF_TRY(device_sms(&sms));
   return layernorm(x, rows, dim, w1, b1, w2, b2, eps, out, nullptr, nullptr, sms, static_cast<cudaStream_t>(stream));
 }
 
@@ -392,53 +367,25 @@ int iefvad_linear(const float* x, const float* w, const float* bias, const float
                   int64_t rows, int in_f, int out_f, int plan, int tile_n, float* out, void* stream) {
   IEF_CHECK(x && w && out, "iefvad_linear: null argument");
   IEF_CHECK(rows >= 0 && rows < (1LL << 31), "iefvad_linear: bad row count");
-  IEF_CHECK(plan >= -1 && plan <= 2, "iefvad_linear: plan must be -1 (fp32), 0 (bf16), 1 (split-bf16) or 2 (fp16)");
+  IEF_TRY(check_plan("iefvad_linear", plan));
   if (rows == 0) return IEFVAD_OK;
+  IEF_CHECK(plan < 0 || ((rows * in_f) % 8 == 0 && (int64_t(out_f) * in_f) % 8 == 0),
+            "iefvad_linear: sizes must be multiples of 8");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   int sms = 0;
-  IEF_TRY(current_sms(&sms));
+  IEF_TRY(device_sms(&sms));
   EpiParams ep;
   ep.bias = bias; ep.act = act; ep.resid = resid; ep.ld_resid = out_f; ep.alpha = alpha;
   ep.out_f32 = out; ep.ld_f32 = out_f;
-  if (plan < 0) return gemm_simt(x, in_f, w, in_f, int(rows), out_f, in_f, ep, st);
-  IEF_CHECK((rows * in_f) % 8 == 0 && (int64_t(out_f) * in_f) % 8 == 0, "iefvad_linear: sizes must be multiples of 8");
   Scratch sc(st);
-  void *xh, *xl, *wh, *wl;
-  IEF_TRY(sc.get(&xh, size_t(rows) * in_f * 2));
-  IEF_TRY(sc.get(&xl, size_t(rows) * in_f * 2));
-  IEF_TRY(sc.get(&wh, size_t(out_f) * in_f * 2));
-  IEF_TRY(sc.get(&wl, size_t(out_f) * in_f * 2));
-  if (plan == 2) {                  // fp16 (E5M10) operands, one MMA pass: what the default plan HH runs everywhere
-    IEF_TRY(to_half(x, rows * in_f, xh, sms, st));
-    IEF_TRY(to_half(w, int64_t(out_f) * in_f, wh, sms, st));
-  } else {
-    IEF_TRY(ingest(x, IEFVAD_DT_F32, rows * in_f, nullptr, (bf16*)xh, (bf16*)xl, sms, st));
-    IEF_TRY(ingest(w, IEFVAD_DT_F32, int64_t(out_f) * in_f, nullptr, (bf16*)wh, (bf16*)wl, sms, st));
-  }
-  GemmTcArgs g;
-  g.A_hi = (bf16*)xh; g.A_lo = (bf16*)xl; g.W_hi = (bf16*)wh; g.W_lo = (bf16*)wl;
-  g.M = int(rows); g.N = out_f; g.K = in_f; g.lda = in_f; g.ldw = in_f; g.nsplit = plan == 1 ? 3 : 1;
-  g.fp16 = plan == 2 ? 1 : 0;
+  Mat xm, wm;
+  IEF_TRY(to_mat(sc, &xm, x, int(rows), in_f, in_f, int(rows), in_f, plan, sms, st));
+  IEF_TRY(to_mat(sc, &wm, w, out_f, in_f, in_f, out_f, in_f, plan, sms, st));
+  if (plan < 0) return gemm_plan(plan, xm, wm, int(rows), out_f, in_f, ep, nullptr, sms, st);
+  GemmTcArgs g = tc_args(plan, xm, wm, int(rows), out_f, in_f);
   g.force_bn = tile_n == 512 ? 256 : tile_n;          // 512 = 256-column tiles on CTA pairs
   g.force_cg = tile_n == 512 ? 2 : (tile_n ? 1 : 0);
-  // Small output, long contraction (the wgrad GEMMs of the training step: [768, 768] = dY^T [768, 16 384] . X^T): without
-  // split-K 72 CTAs walk 768 k-blocks each.  K slices become extra row tiles of a [S x rows, out_f] partial buffer (256-column
-  // tiles on CTA pairs), summed in slice order afterwards - deterministic, unlike atomics.
-  if (tile_n == 0 && !bias && !resid && act == ACT_NONE && rows % 256 == 0 && out_f % 256 == 0 && in_f >= 4096 &&
-      (rows / 256) * (out_f / 256) * 2 <= sms / 2) {
-    int S = (sms / 2) / int((rows / 256) * (out_f / 256));
-    while (S > 1 && (in_f / 64) % S != 0) --S;
-    if (S > 1) {
-      void* part;
-      IEF_TRY(sc.get(&part, size_t(S) * rows * out_f * 4));
-      ep.alpha = 1.f;
-      ep.out_f32 = static_cast<float*>(part);
-      g.ksplit = S; g.force_bn = 256; g.force_cg = 2;
-      IEF_TRY(gemm_tc(g, ep, sms, st));
-      return sum_slices(static_cast<const float*>(part), S, rows * out_f, alpha, out, sms, st);
-    }
-  }
-  return gemm_tc(g, ep, sms, st);
+  return gemm_tc_split_k(g, ep, sc, sms, st);
 }
 
 int iefvad_outproj_ln(const float* ctx, const float* w, const float* bias, const float* resid, const float* ln_w,
@@ -449,20 +396,21 @@ int iefvad_outproj_ln(const float* ctx, const float* w, const float* bias, const
   if (rows == 0) return IEFVAD_OK;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   int sms = 0;
-  IEF_TRY(current_sms(&sms));
+  IEF_TRY(device_sms(&sms));
   constexpr int D = kOutprojLnDim;
   Scratch sc(st);
-  void *ch, *wh, *rh, *rl, *scr, *idt;
+  uint8_t *scr = nullptr, *idt = nullptr;
+  bf16 *ch = nullptr, *wh = nullptr, *rh = nullptr, *rl = nullptr;
   IEF_TRY(sc.get(&idt, outproj_ln_identity_bytes()));
   IEF_TRY(outproj_ln_identity(idt, st));
-  IEF_TRY(sc.get(&ch, size_t(rows) * D * 2));
-  IEF_TRY(sc.get(&wh, size_t(D) * D * 2));
-  IEF_TRY(sc.get(&rh, size_t(rows) * D * 2));
-  IEF_TRY(sc.get(&rl, size_t(rows) * D * 2));
+  IEF_TRY(sc.get(&ch, size_t(rows) * D));
+  IEF_TRY(sc.get(&wh, size_t(D) * D));
+  IEF_TRY(sc.get(&rh, size_t(rows) * D));
+  IEF_TRY(sc.get(&rl, size_t(rows) * D));
   IEF_TRY(sc.get(&scr, outproj_ln_scratch_bytes(rows)));
   IEF_TRY(to_half(ctx, rows * D, ch, sms, st));
   IEF_TRY(to_half(w, int64_t(D) * D, wh, sms, st));
-  IEF_TRY(ingest(resid, IEFVAD_DT_F32, rows * D, nullptr, (bf16*)rh, (bf16*)rl, sms, st, 1));
+  IEF_TRY(ingest(resid, IEFVAD_DT_F32, rows * D, nullptr, rh, rl, sms, st, 1));
   OutprojLnArgs a;
   a.ctx = ch; a.w16 = wh; a.bias = bias; a.res_hi = rh; a.res_lo = rl; a.ln_w = ln_w; a.ln_b = ln_b; a.ln2_w = ln2_w;
   a.ln2_b = ln2_b; a.eps = eps; a.out_hi = out_hi_f16; a.out_lo = out_lo_f16; a.row_map = row_map; a.M = rows; a.scratch = scr;
@@ -475,70 +423,23 @@ int iefvad_mha(const float* x, const float* in_w, const float* in_b, const float
                int plan, float* out, void* stream) {
   IEF_CHECK(x && in_w && in_b && out_w && out_b && out, "iefvad_mha: null argument");
   IEF_CHECK(num_heads > 0 && D % num_heads == 0, "iefvad_mha: heads must divide D");
-  IEF_CHECK(plan >= -1 && plan <= 2, "iefvad_mha: plan must be -1 (fp32), 0 (bf16), 1 (split-bf16) or 2 (fp16)");
+  IEF_TRY(check_plan("iefvad_mha", plan));
   IEF_CHECK(B >= 0 && T >= 0 && B * T < (1LL << 31), "iefvad_mha: bad sizes");
   if (B == 0 || T == 0) return IEFVAD_OK;
+  IEF_CHECK(plan < 0 || D % 64 == 0, "iefvad_mha: tensor-core plans need D %% 64 == 0");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   int sms = 0;
-  IEF_TRY(current_sms(&sms));
-  const int64_t M = B * T;
-  const int dh = D / num_heads, dhp = (dh + 63) / 64 * 64, Tpad = int((T + 7) / 8 * 8);
+  IEF_TRY(device_sms(&sms));
+  const int M = int(B * T);
   Scratch sc(st);
-  if (plan < 0) {
-    void *qkv, *ctx;
-    IEF_TRY(sc.get(&qkv, size_t(M) * 3 * D * 4));
-    IEF_TRY(sc.get(&ctx, size_t(M) * D * 4));
-    EpiParams e1;
-    e1.bias = in_b; e1.out_f32 = (float*)qkv; e1.ld_f32 = 3 * D;
-    IEF_TRY(gemm_simt(x, D, in_w, D, int(M), 3 * D, D, e1, st));
-    IEF_TRY(attn_simt((float*)qkv, (float*)ctx, int(B), int(T), num_heads, dh, attn_mask, key_padding_mask, st));
-    EpiParams e2;
-    e2.bias = out_b; e2.out_f32 = out; e2.ld_f32 = D;
-    return gemm_simt((float*)ctx, D, out_w, D, int(M), D, D, e2, st);
-  }
-  IEF_CHECK(D % 64 == 0, "iefvad_mha: tensor-core plans need D %% 64 == 0");
-  void *xh, *xl, *iwh, *iwl, *owh, *owl, *q, *k, *vt, *ctx;
-  IEF_TRY(sc.get(&xh, size_t(M) * D * 2));
-  IEF_TRY(sc.get(&xl, size_t(M) * D * 2));
-  IEF_TRY(sc.get(&iwh, size_t(3) * D * D * 2));
-  IEF_TRY(sc.get(&iwl, size_t(3) * D * D * 2));
-  IEF_TRY(sc.get(&owh, size_t(D) * D * 2));
-  IEF_TRY(sc.get(&owl, size_t(D) * D * 2));
-  IEF_TRY(sc.get(&q, size_t(M) * num_heads * dhp * 2));
-  IEF_TRY(sc.get(&k, size_t(M) * num_heads * dhp * 2));
-  IEF_TRY(sc.get(&vt, size_t(B) * num_heads * dh * Tpad * 2));
-  IEF_TRY(sc.get(&ctx, size_t(M) * D * 2));
-  // plan 2 is the default model plan HH's arithmetic: fp16 operands everywhere, and on the unmasked short-sequence kernel
-  // q / k rows of d_h rather than d_h padded to 64 (model.cu, Model::forward)
-  const int f16 = plan == 2 ? 1 : 0;
-  const int dhq = (f16 && T <= 256 && dh % 32 == 0 && !attn_mask && !key_padding_mask) ? dh : dhp;
-  if (f16) {
-    IEF_TRY(to_half(x, M * D, xh, sms, st));
-    IEF_TRY(to_half(in_w, 3LL * D * D, iwh, sms, st));
-    IEF_TRY(to_half(out_w, 1LL * D * D, owh, sms, st));
-  } else {
-    IEF_TRY(ingest(x, IEFVAD_DT_F32, M * D, nullptr, (bf16*)xh, (bf16*)xl, sms, st));
-    IEF_TRY(ingest(in_w, IEFVAD_DT_F32, 3LL * D * D, nullptr, (bf16*)iwh, (bf16*)iwl, sms, st));
-    IEF_TRY(ingest(out_w, IEFVAD_DT_F32, 1LL * D * D, nullptr, (bf16*)owh, (bf16*)owl, sms, st));
-  }
-  EpiParams e1;
-  e1.mode = EPI_QKV; e1.bias = in_b; e1.q = (bf16*)q; e1.k = (bf16*)k; e1.vt = (bf16*)vt; e1.hi_fp16 = f16;
-  e1.T = int(T); e1.H = num_heads; e1.dh = dh; e1.dhp = dhq; e1.Tpad = Tpad; e1.D = D;
-  e1.qscale = 1.0f / sqrtf(float(dh));
-  GemmTcArgs g1;
-  g1.A_hi = (bf16*)xh; g1.A_lo = (bf16*)xl; g1.W_hi = (bf16*)iwh; g1.W_lo = (bf16*)iwl;
-  g1.M = int(M); g1.N = 3 * D; g1.K = D; g1.lda = D; g1.ldw = D; g1.nsplit = plan == 1 ? 3 : 1; g1.fp16 = f16;
-  IEF_TRY(gemm_tc(g1, e1, sms, st));
-  AttnTcArgs at;
-  at.q = (bf16*)q; at.k = (bf16*)k; at.vt = (bf16*)vt; at.out = (bf16*)ctx; at.ldo = D;
-  at.B = int(B); at.T = int(T); at.H = num_heads; at.dh = dh; at.dhp = dhq; at.Tpad = Tpad;
-  at.attn_mask = attn_mask; at.key_pad = key_padding_mask; at.fp16 = f16;
-  IEF_TRY(attn_tc(at, st));
-  EpiParams e2;
-  e2.bias = out_b; e2.out_f32 = out; e2.ld_f32 = D;
-  GemmTcArgs g2;
-  g2.A_hi = (bf16*)ctx; g2.W_hi = (bf16*)owh; g2.M = int(M); g2.N = D; g2.K = D; g2.lda = D; g2.ldw = D; g2.fp16 = f16;
-  return gemm_tc(g2, e2, sms, st);
+  Mat xm, iw, ow;
+  AttnWork aw;
+  IEF_TRY(to_mat(sc, &xm, x, M, D, D, M, D, plan, sms, st));
+  IEF_TRY(to_mat(sc, &iw, in_w, 3 * D, D, D, 3 * D, D, plan, sms, st));
+  IEF_TRY(to_mat(sc, &ow, out_w, D, D, D, D, D, plan, sms, st));
+  IEF_TRY(alloc_attn_work(sc, &aw, plan, int(B), int(T), D, num_heads));
+  return attention_sublayer(plan, xm, iw, in_b, ow, out_b, int(B), int(T), D, num_heads, attn_mask, key_padding_mask,
+                            nullptr, out, aw, sms, st);
 }
 
 int iefvad_attention_core(const void* q, const void* k, const void* vt, int64_t B, int64_t T, int H, int dh, int dhp,
@@ -572,7 +473,7 @@ int iefvad_classifier(const float* x, int64_t rows, int dim, const float* w, con
                       float* scores, void* stream) {
   IEF_CHECK(x && w && bias && logits, "iefvad_classifier: null argument");
   int sms = 0;
-  IEF_TRY(current_sms(&sms));
+  IEF_TRY(device_sms(&sms));
   return classifier(x, rows, dim, w, bias, logits, scores, sms, static_cast<cudaStream_t>(stream));
 }
 
@@ -618,7 +519,7 @@ int iefvad_distance_adj(int64_t batch_size, int max_seqlen, float* out, void* st
 int iefvad_similarity_adj(const float* x, const float* weight0_t, const int64_t* seq_len_host, int64_t B, int T, int in_f,
                           int out_f, int plan, float* out, void* stream) {
   int sms = 0;
-  IEF_TRY(current_sms(&sms));
+  IEF_TRY(device_sms(&sms));
   return similarity_adj(x, weight0_t, reinterpret_cast<const long long*>(seq_len_host), B, T, in_f, out_f, plan, out, sms,
                         static_cast<cudaStream_t>(stream));
 }
@@ -627,7 +528,7 @@ int iefvad_graph_convolution(const float* x, const float* adj, const float* weig
                              const float* conv_w, const float* conv_b, int64_t B, int T, int in_f, int out_f, int plan,
                              float* out, void* stream) {
   int sms = 0;
-  IEF_TRY(current_sms(&sms));
+  IEF_TRY(device_sms(&sms));
   return graph_convolution(x, adj, weight_t, bias, residual, conv_w, conv_b, B, T, in_f, out_f, plan, out, sms,
                            static_cast<cudaStream_t>(stream));
 }
@@ -641,7 +542,7 @@ int iefvad_transformer(const float* x, const float* const* params, int layers, i
   IEF_CHECK(params != nullptr || layers == 0, "iefvad_transformer: null parameter table");
   IEF_CHECK(layers >= 0 && layers <= 64, "iefvad_transformer: 0..64 layers");
   int sms = 0;
-  IEF_TRY(current_sms(&sms));
+  IEF_TRY(device_sms(&sms));
   std::vector<ResBlockParams> blocks(static_cast<size_t>(layers));
   for (int i = 0; i < layers; ++i) {
     const float* const* p = params + 12 * i;
@@ -692,13 +593,13 @@ int iefvad_event_image(const uint8_t* frames, int64_t B, int C, int H, int W, fl
   IEF_CHECK(frames, "iefvad_event_image: null frames");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   int sms = 0;
-  IEF_TRY(current_sms(&sms));
+  IEF_TRY(device_sms(&sms));
   Scratch sc(st);
-  void *cnt, *mx;
-  IEF_TRY(sc.get(&cnt, size_t(B) * H * W * 4));
-  IEF_TRY(sc.get(&mx, 16));
-  return event_image(frames, B, C, H, W, threshold, clamp_max, sum_out, event_out, static_cast<float*>(cnt),
-                     static_cast<unsigned*>(mx), sms, st);
+  float* cnt = nullptr;
+  unsigned* mx = nullptr;
+  IEF_TRY(sc.get(&cnt, size_t(B) * H * W));
+  IEF_TRY(sc.get(&mx, 4));
+  return event_image(frames, B, C, H, W, threshold, clamp_max, sum_out, event_out, cnt, mx, sms, st);
 }
 
 int iefvad_bench_gemm(int64_t M, int N, int K, int nsplit, int tile_n, int stages, int epi_kind, int iters,
@@ -706,21 +607,23 @@ int iefvad_bench_gemm(int64_t M, int N, int K, int nsplit, int tile_n, int stage
   IEF_CHECK(M > 0 && M < (1LL << 31) && N > 0 && K > 0 && iters > 0 && ms_per_iter, "iefvad_bench_gemm: bad argument");
   IEF_CHECK(epi_kind >= 0 && epi_kind <= 7, "iefvad_bench_gemm: epi_kind in [0, 7]");
   int sms = 0;
-  IEF_TRY(current_sms(&sms));
+  IEF_TRY(device_sms(&sms));
   cudaStream_t st = nullptr;
   Scratch sc(st);
-  void *ah, *al, *wh, *wl, *bias, *resid, *of, *oh, *ol, *q, *k, *vt;
+  bf16 *ah = nullptr, *al = nullptr, *wh = nullptr, *wl = nullptr, *oh = nullptr, *ol = nullptr, *q = nullptr, *k = nullptr,
+       *vt = nullptr;
+  float *bias = nullptr, *resid = nullptr, *of = nullptr;
   const int H = 8, dh = N / 3 / H > 0 ? N / 3 / H : 1, dhp = (dh + 63) / 64 * 64;
   const int T = 256, Tpad = 256;
-  IEF_TRY(sc.get(&ah, size_t(M) * K * 2));
-  IEF_TRY(sc.get(&al, size_t(M) * K * 2));
-  IEF_TRY(sc.get(&wh, size_t(N) * K * 2));
-  IEF_TRY(sc.get(&wl, size_t(N) * K * 2));
-  IEF_TRY(sc.get(&bias, size_t(N) * 4));
-  IEF_TRY(sc.get(&resid, size_t(M) * N * 4));
-  IEF_TRY(sc.get(&of, size_t(M) * N * 4));
-  IEF_TRY(sc.get(&oh, size_t(M) * N * 2));
-  IEF_TRY(sc.get(&ol, size_t(M) * N * 2));
+  IEF_TRY(sc.get(&ah, size_t(M) * K));
+  IEF_TRY(sc.get(&al, size_t(M) * K));
+  IEF_TRY(sc.get(&wh, size_t(N) * K));
+  IEF_TRY(sc.get(&wl, size_t(N) * K));
+  IEF_TRY(sc.get(&bias, size_t(N)));
+  IEF_TRY(sc.get(&resid, size_t(M) * N));
+  IEF_TRY(sc.get(&of, size_t(M) * N));
+  IEF_TRY(sc.get(&oh, size_t(M) * N));
+  IEF_TRY(sc.get(&ol, size_t(M) * N));
   IEF_CUDA(cudaMemsetAsync(ah, 0x3c, size_t(M) * K * 2, st));     // bf16 0x3c3c ~ 0.0115: finite, non-zero operands
   IEF_CUDA(cudaMemsetAsync(al, 0x3a, size_t(M) * K * 2, st));
   IEF_CUDA(cudaMemsetAsync(wh, 0x3c, size_t(N) * K * 2, st));
@@ -728,33 +631,33 @@ int iefvad_bench_gemm(int64_t M, int N, int K, int nsplit, int tile_n, int stage
   IEF_CUDA(cudaMemsetAsync(bias, 0, size_t(N) * 4, st));
   IEF_CUDA(cudaMemsetAsync(resid, 0, size_t(M) * N * 4, st));
   EpiParams ep;
-  ep.bias = static_cast<float*>(bias);
+  ep.bias = bias;
   if (epi_kind == 0) ep.mode = EPI_DISCARD;
-  if (epi_kind == 1) { ep.out_f32 = (float*)of; ep.ld_f32 = N; }
+  if (epi_kind == 1) { ep.out_f32 = of; ep.ld_f32 = N; }
   if (epi_kind == 2) {
-    ep.resid = (float*)resid; ep.ld_resid = N; ep.alpha = -0.5f; ep.out_f32 = (float*)of; ep.ld_f32 = N;
-    ep.out_hi = (bf16*)oh; ep.out_lo = (bf16*)ol; ep.ld_bf = N;
+    ep.resid = resid; ep.ld_resid = N; ep.alpha = -0.5f; ep.out_f32 = of; ep.ld_f32 = N;
+    ep.out_hi = oh; ep.out_lo = ol; ep.ld_bf = N;
   }
-  if (epi_kind == 3) { ep.act = ACT_RELU; ep.out_hi = (bf16*)oh; ep.out_lo = (bf16*)ol; ep.ld_bf = N; }
-  if (epi_kind == 5) { ep.act = ACT_RELU; ep.out_hi = (bf16*)oh; ep.ld_bf = N; ep.hi_fp16 = 1; }
+  if (epi_kind == 3) { ep.act = ACT_RELU; ep.out_hi = oh; ep.out_lo = ol; ep.ld_bf = N; }
+  if (epi_kind == 5) { ep.act = ACT_RELU; ep.out_hi = oh; ep.ld_bf = N; ep.hi_fp16 = 1; }
   if (epi_kind == 6) {
-    ep.resid = (float*)resid; ep.ld_resid = N; ep.alpha = -0.5f; ep.out_f32 = (float*)of; ep.ld_f32 = N;
-    ep.out_hi = (bf16*)oh; ep.ld_bf = N; ep.hi_fp16 = 1;
+    ep.resid = resid; ep.ld_resid = N; ep.alpha = -0.5f; ep.out_f32 = of; ep.ld_f32 = N;
+    ep.out_hi = oh; ep.ld_bf = N; ep.hi_fp16 = 1;
   }
   if (epi_kind == 7) {        // refinement Linear2 of the fp16 plans: fp16 pair in, fp16 pair out (in place)
     ep.resid_h16 = oh; ep.resid_l16 = ol; ep.ld_resid = N; ep.alpha = -0.5f;
-    ep.out_hi = (bf16*)oh; ep.out_lo = (bf16*)ol; ep.ld_bf = N; ep.hi_fp16 = 1;
+    ep.out_hi = oh; ep.out_lo = ol; ep.ld_bf = N; ep.hi_fp16 = 1;
   }
   if (epi_kind == 4) {
     IEF_CHECK(N % (3 * H * 32) == 0 && M % T == 0, "iefvad_bench_gemm: qkv epilogue needs N = 3*8*dh, M %% 256 == 0");
-    IEF_TRY(sc.get(&q, size_t(M) * H * dhp * 2));
-    IEF_TRY(sc.get(&k, size_t(M) * H * dhp * 2));
-    IEF_TRY(sc.get(&vt, size_t(M) * H * dh * 2));
-    ep.mode = EPI_QKV; ep.q = (bf16*)q; ep.k = (bf16*)k; ep.vt = (bf16*)vt; ep.T = T; ep.H = H; ep.dh = dh; ep.dhp = dhp;
+    IEF_TRY(sc.get(&q, size_t(M) * H * dhp));
+    IEF_TRY(sc.get(&k, size_t(M) * H * dhp));
+    IEF_TRY(sc.get(&vt, size_t(M) * H * dh));
+    ep.mode = EPI_QKV; ep.q = q; ep.k = k; ep.vt = vt; ep.T = T; ep.H = H; ep.dh = dh; ep.dhp = dhp;
     ep.Tpad = Tpad; ep.D = N / 3; ep.qscale = 0.1f;
   }
   GemmTcArgs g;
-  g.A_hi = (bf16*)ah; g.A_lo = (bf16*)al; g.W_hi = (bf16*)wh; g.W_lo = (bf16*)wl;
+  g.A_hi = ah; g.A_lo = al; g.W_hi = wh; g.W_lo = wl;
   g.M = int(M); g.N = N; g.K = K; g.lda = K; g.ldw = K; g.nsplit = nsplit; g.force_stages = stages;
   g.force_bn = tile_n == 512 ? 256 : tile_n;
   g.force_cg = tile_n == 512 ? 2 : (tile_n ? 1 : 0);
@@ -799,11 +702,11 @@ int iefvad_attention_train_bwd(const float* qkv, const float* out, const float* 
   IEF_CHECK(B >= 0 && B < 65536 && T >= 0 && T < (1 << 24), "iefvad_attention_train_bwd: bad B / T");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   int sms = 0;
-  IEF_TRY(current_sms(&sms));
+  IEF_TRY(device_sms(&sms));
   Scratch sc(st);
-  void* delta = nullptr;
-  IEF_TRY(sc.get(&delta, size_t(B) * heads * T * 4));
-  return attn_train_bwd(qkv, out, dout, lse, int(B), int(T), heads, head_dim, p_drop, seed, static_cast<float*>(delta), dqkv, sms, st);
+  float* delta = nullptr;
+  IEF_TRY(sc.get(&delta, size_t(B) * heads * T));
+  return attn_train_bwd(qkv, out, dout, lse, int(B), int(T), heads, head_dim, p_drop, seed, delta, dqkv, sms, st);
 }
 
 int iefvad_layernorm_bwd(const float* x, const float* weight, const float* dy, int64_t rows, int dim, float eps, float* dx,
@@ -811,22 +714,22 @@ int iefvad_layernorm_bwd(const float* x, const float* weight, const float* dy, i
   IEF_CHECK(x && weight && dy && dx && dweight && dbias, "iefvad_layernorm_bwd: null argument");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   int sms = 0;
-  IEF_TRY(current_sms(&sms));
+  IEF_TRY(device_sms(&sms));
   Scratch sc(st);
-  void* scratch = nullptr;
-  IEF_TRY(sc.get(&scratch, (size_t(2) * rows + size_t(2) * train_colsum_blocks(rows, sms) * dim) * 4));
-  return layernorm_bwd(x, weight, dy, rows, dim, eps, dx, dweight, dbias, static_cast<float*>(scratch), sms, st);
+  float* scratch = nullptr;
+  IEF_TRY(sc.get(&scratch, size_t(2) * rows + size_t(2) * train_colsum_blocks(rows, sms) * dim));
+  return layernorm_bwd(x, weight, dy, rows, dim, eps, dx, dweight, dbias, scratch, sms, st);
 }
 
 int iefvad_colsum(const float* a, const float* row_weight, int64_t rows, int dim, float* out, void* stream) {
   IEF_CHECK(a && out, "iefvad_colsum: null argument");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   int sms = 0;
-  IEF_TRY(current_sms(&sms));
+  IEF_TRY(device_sms(&sms));
   Scratch sc(st);
-  void* scratch = nullptr;
-  IEF_TRY(sc.get(&scratch, size_t(2) * train_colsum_blocks(rows, sms) * dim * 4));
-  return colsum(a, row_weight, rows, dim, out, static_cast<float*>(scratch), sms, st);
+  float* scratch = nullptr;
+  IEF_TRY(sc.get(&scratch, size_t(2) * train_colsum_blocks(rows, sms) * dim));
+  return colsum(a, row_weight, rows, dim, out, scratch, sms, st);
 }
 
 int iefvad_fuse_bwd(const float* mu_i, const float* mu_e, const float* logvar_i, const float* logvar_e, const float* g_fused,
@@ -835,7 +738,7 @@ int iefvad_fuse_bwd(const float* mu_i, const float* mu_e, const float* logvar_i,
                     float* d_logvar_i, float* d_logvar_e, void* stream) {
   IEF_CHECK(mu_i && mu_e && logvar_i && logvar_e && d_mu_i && d_mu_e && d_logvar_i && d_logvar_e, "iefvad_fuse_bwd: null argument");
   int sms = 0;
-  IEF_TRY(current_sms(&sms));
+  IEF_TRY(device_sms(&sms));
   return fuse_bwd(mu_i, mu_e, logvar_i, logvar_e, g_fused, g_wi, g_we, g_mu_i, g_mu_e, g_logvar_i, g_logvar_e, n, factor, epsilon,
                   d_mu_i, d_mu_e, d_logvar_i, d_logvar_e, sms, static_cast<cudaStream_t>(stream));
 }
@@ -843,28 +746,28 @@ int iefvad_fuse_bwd(const float* mu_i, const float* mu_e, const float* logvar_i,
 int iefvad_relu_bwd(const float* dh, const float* h, int64_t n, float* out, void* stream) {
   IEF_CHECK(dh && h && out, "iefvad_relu_bwd: null argument");
   int sms = 0;
-  IEF_TRY(current_sms(&sms));
+  IEF_TRY(device_sms(&sms));
   return relu_bwd(dh, h, n, out, sms, static_cast<cudaStream_t>(stream));
 }
 
 int iefvad_quickgelu(const float* x, int64_t n, float* out, void* stream) {
   IEF_CHECK(x && out, "iefvad_quickgelu: null argument");
   int sms = 0;
-  IEF_TRY(current_sms(&sms));
+  IEF_TRY(device_sms(&sms));
   return quickgelu(x, n, out, sms, static_cast<cudaStream_t>(stream));
 }
 
 int iefvad_axpy(float* y, const float* x, float alpha, int64_t n, void* stream) {
   IEF_CHECK(y && x, "iefvad_axpy: null argument");
   int sms = 0;
-  IEF_TRY(current_sms(&sms));
+  IEF_TRY(device_sms(&sms));
   return axpy(y, x, alpha, n, sms, static_cast<cudaStream_t>(stream));
 }
 
 int iefvad_outer(const float* a, const float* w, int64_t rows, int dim, float* out, void* stream) {
   IEF_CHECK(a && w && out, "iefvad_outer: null argument");
   int sms = 0;
-  IEF_TRY(current_sms(&sms));
+  IEF_TRY(device_sms(&sms));
   return outer(a, w, rows, dim, out, sms, static_cast<cudaStream_t>(stream));
 }
 
@@ -878,37 +781,24 @@ int iefvad_wgrad(const float* dy, const float* x, int64_t rows, int out_f, int i
   IEF_CHECK(rows > 0 && rows < (1LL << 31) && out_f % 32 == 0 && in_f % 32 == 0, "iefvad_wgrad: bad sizes");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   int sms = 0;
-  IEF_TRY(current_sms(&sms));
+  IEF_TRY(device_sms(&sms));
   const int64_t Mp = (rows + 63) / 64 * 64;
   Scratch sc(st);
-  void *yh, *yl, *xh, *xl;
-  IEF_TRY(sc.get(&yh, size_t(out_f) * Mp * 2));
-  IEF_TRY(sc.get(&yl, size_t(out_f) * Mp * 2));
-  IEF_TRY(sc.get(&xh, size_t(in_f) * Mp * 2));
-  IEF_TRY(sc.get(&xl, size_t(in_f) * Mp * 2));
+  bf16 *yh = nullptr, *yl = nullptr, *xh = nullptr, *xl = nullptr;
+  IEF_TRY(sc.get(&yh, size_t(out_f) * Mp));
+  IEF_TRY(sc.get(&yl, size_t(out_f) * Mp));
+  IEF_TRY(sc.get(&xh, size_t(in_f) * Mp));
+  IEF_TRY(sc.get(&xl, size_t(in_f) * Mp));
   // both operands go from row-major fp32 straight to the K-major bf16 hi / lo form the GEMM reads: one pass each instead
   // of a transposition to fp32 followed by the conversion
-  IEF_TRY(transpose_split(dy, rows, out_f, (bf16*)yh, (bf16*)yl, Mp, st));
-  IEF_TRY(transpose_split(x, rows, in_f, (bf16*)xh, (bf16*)xl, Mp, st));
+  IEF_TRY(transpose_split(dy, rows, out_f, yh, yl, Mp, st));
+  IEF_TRY(transpose_split(x, rows, in_f, xh, xl, Mp, st));
   GemmTcArgs g;
-  g.A_hi = (bf16*)yh; g.A_lo = (bf16*)yl; g.W_hi = (bf16*)xh; g.W_lo = (bf16*)xl;
+  g.A_hi = yh; g.A_lo = yl; g.W_hi = xh; g.W_lo = xl;
   g.M = out_f; g.N = in_f; g.K = int(Mp); g.lda = int(Mp); g.ldw = int(Mp); g.nsplit = 3;
   EpiParams ep;
   ep.alpha = alpha; ep.out_f32 = dw; ep.ld_f32 = in_f;
-  if (out_f % 256 == 0 && in_f % 256 == 0 && Mp >= 4096 && (out_f / 256) * (in_f / 256) * 2 <= sms / 2) {
-    int S = (sms / 2) / ((out_f / 256) * (in_f / 256));
-    while (S > 1 && (Mp / 64) % S != 0) --S;
-    if (S > 1) {
-      void* part;
-      IEF_TRY(sc.get(&part, size_t(S) * out_f * in_f * 4));
-      ep.alpha = 1.f;
-      ep.out_f32 = static_cast<float*>(part);
-      g.ksplit = S; g.force_bn = 256; g.force_cg = 2;
-      IEF_TRY(gemm_tc(g, ep, sms, st));
-      return sum_slices(static_cast<const float*>(part), S, int64_t(out_f) * in_f, alpha, dw, sms, st);
-    }
-  }
-  return gemm_tc(g, ep, sms, st);
+  return gemm_tc_split_k(g, ep, sc, sms, st);
 }
 
 int iefvad_clas2_bwd(const float* logits, const float* means, const float* labels, int64_t label_stride, const int32_t* idx,
@@ -940,10 +830,10 @@ int iefvad_train_loss_fwd(const float* logits, const float* labels, int64_t labe
   IEF_CHECK(reinterpret_cast<uintptr_t>(record) % 32 == 0, "iefvad_train_loss_fwd: record must be 32-byte aligned");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   Scratch sc(st);
-  void* slabs = nullptr;
-  IEF_TRY(sc.get(&slabs, size_t(2) * train_loss_slabs(B * T) * sizeof(double)));
+  double* slabs = nullptr;
+  IEF_TRY(sc.get(&slabs, size_t(2) * train_loss_slabs(B * T)));
   return train_loss_fwd(logits, labels, label_stride, reinterpret_cast<const long long*>(lengths), int(B), int(T), mu_i, mu_e,
-                        logvar_i, logvar_e, D, nu, reg_weight, kl_weight, means, idx, kmax, record, static_cast<double*>(slabs),
+                        logvar_i, logvar_e, D, nu, reg_weight, kl_weight, means, idx, kmax, record, slabs,
                         total, loss_cls, loss_reg, loss_kl, st);
 }
 
@@ -961,10 +851,10 @@ int iefvad_train_loss_bwd(const float* logits, const float* means, const float* 
   IEF_CHECK(reinterpret_cast<uintptr_t>(record) % 32 == 0, "iefvad_train_loss_bwd: record must be 32-byte aligned");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   Scratch sc(st);
-  void* g_cls_total = nullptr;
-  IEF_TRY(sc.get(&g_cls_total, sizeof(float)));
+  float* g_cls_total = nullptr;
+  IEF_TRY(sc.get(&g_cls_total, 1));
   return train_loss_bwd(logits, means, labels, label_stride, idx, int(B), int(T), kmax, mu_i, mu_e, logvar_i, logvar_e, D, record,
-                        nu, reg_weight, kl_weight, g_total, g_cls, g_reg, g_kl, static_cast<float*>(g_cls_total), d_logits,
+                        nu, reg_weight, kl_weight, g_total, g_cls, g_reg, g_kl, g_cls_total, d_logits,
                         d_mu_i, d_mu_e, d_logvar_i, d_logvar_e, st);
 }
 
@@ -986,12 +876,13 @@ int iefvad_locmap_match(const int32_t* prop_count, const int32_t* prop_se, const
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int cap = int(num_videos) * 8 > 8192 ? int(num_videos) * 8 : 8192;
   Scratch sc(st);
-  void *ws, *wi, *wa;
-  IEF_TRY(sc.get(&ws, size_t(num_classes) * cap * 4 * 2));      // rounded up to a power of two inside the kernel
-  IEF_TRY(sc.get(&wi, size_t(num_classes) * cap * 4 * 2));
-  IEF_TRY(sc.get(&wa, size_t(num_gt ? num_gt : 1) * 4));
+  float* ws = nullptr;
+  int *wi = nullptr, *wa = nullptr;
+  IEF_TRY(sc.get(&ws, size_t(num_classes) * cap * 2));      // rounded up to a power of two inside the kernel
+  IEF_TRY(sc.get(&wi, size_t(num_classes) * cap * 2));
+  IEF_TRY(sc.get(&wa, size_t(num_gt ? num_gt : 1)));
   return locmap_match(prop_count, prop_se, prop_score, int(num_videos), num_classes, gt, gt_off, iou_threshold, cap * 2,
-                      static_cast<float*>(ws), static_cast<int*>(wi), static_cast<int*>(wa), ap, n_pred, st);
+                      ws, wi, wa, ap, n_pred, st);
 }
 
 int iefvad_profile_read(double* ms, double* work, int64_t* launches) {

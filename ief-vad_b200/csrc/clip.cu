@@ -10,17 +10,11 @@
 #include <vector>
 
 #include "elementwise.cuh"
-#include "gemm.cuh"
-#include "scratch.cuh"
+#include "operand.cuh"
 
 namespace iefvad {
 
 namespace {
-
-int grid_of(long long n, int num_sms) {
-  const long long b = (n + 255) / 256, cap = (long long)num_sms * 8;
-  return int(b < 1 ? 1 : (b > cap ? cap : b));
-}
 
 __device__ __forceinline__ float load_f(const float* p, long long i) { return p[i]; }
 __device__ __forceinline__ float load_f(const __half* p, long long i) { return __half2float(p[i]); }
@@ -46,18 +40,6 @@ clip_im2col_kernel(const Tin* __restrict__ x, long long rows, int R, int P, int 
       v = load_f(x, ((n * 3 + ch) * R + gy * P + ky) * (long long)R + gx * P + kx);
     }
     store_f(dst, i, v);
-  }
-}
-
-// conv1.weight [W, K] -> [W, Kp] in the operand type, zero columns [K, Kp)
-template <typename Tout>
-__global__ void __launch_bounds__(256)
-clip_pad_weight_kernel(const float* __restrict__ w, int rows, int K, int Kp, Tout* __restrict__ dst) {
-  const long long total = (long long)rows * Kp;
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
-    const long long r = i / Kp;
-    const int c = int(i - r * Kp);
-    store_f(dst, i, c < K ? w[r * K + c] : 0.f);
   }
 }
 
@@ -147,7 +129,7 @@ clip_head_kernel(const float* __restrict__ x, int N, int T, int W, const float* 
 template <typename Tout>
 int launch_im2col(const void* x, int dtype, long long rows, int R, int P, int G, int Kp, Tout* dst, int sms,
                   cudaStream_t st) {
-  const int grid = grid_of(rows * Kp, sms);
+  const int grid = blocks_for(rows * Kp, sms);
   if (dtype == IEFVAD_DT_F32)
     clip_im2col_kernel<<<grid, 256, 0, st>>>(static_cast<const float*>(x), rows, R, P, G, Kp, dst);
   else if (dtype == IEFVAD_DT_F16)
@@ -186,9 +168,8 @@ int clip_visual(const void* x, int dtype, int N, int R, int P, int W, int layers
   IEF_CHECK(M < (1LL << 31), "clip_visual: %lld token rows exceed the GEMM row limit", M);
   IEF_CHECK(N == 0 || (x && out), "clip_visual: null input or output");
   if (N == 0) return IEFVAD_OK;
-  int dev = 0, sms = 0;
-  IEF_CUDA(cudaGetDevice(&dev));
-  IEF_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  int sms = 0;
+  IEF_TRY(device_sms(&sms));
 
   const int K = 3 * P * P, Kp = (K + 63) / 64 * 64;
   Scratch sc(st);
@@ -196,31 +177,17 @@ int clip_visual(const void* x, int dtype, int N, int R, int P, int W, int layers
   IEF_TRY(sc.get(&patches, size_t(Mp) * W));
   IEF_TRY(sc.get(&xr, size_t(M) * W));
   // patch embedding (model.py:226)
+  Mat col, wc;
+  IEF_TRY(alloc_mat(sc, &col, size_t(Mp), Kp, plan));
+  if (plan < 0) IEF_TRY(launch_im2col(x, dtype, Mp, R, P, G, Kp, col.f, sms, st));
+  else IEF_TRY(launch_im2col(x, dtype, Mp, R, P, G, Kp, reinterpret_cast<__half*>(col.hi), sms, st));
+  IEF_TRY(to_mat(sc, &wc, p.conv1, W, K, K, W, Kp, plan, sms, st));
   EpiParams ep;
   ep.out_f32 = patches; ep.ld_f32 = W;
-  if (plan < 0) {
-    float *col, *wf;
-    IEF_TRY(sc.get(&col, size_t(Mp) * Kp));
-    IEF_TRY(sc.get(&wf, size_t(W) * Kp));
-    IEF_TRY(launch_im2col(x, dtype, Mp, R, P, G, Kp, col, sms, st));
-    clip_pad_weight_kernel<<<grid_of((long long)W * Kp, sms), 256, 0, st>>>(p.conv1, W, K, Kp, wf);
-    count_launches(1);
-    IEF_TRY(gemm_simt(col, Kp, wf, Kp, int(Mp), W, Kp, ep, st));
-  } else {
-    __half *col, *wh;
-    IEF_TRY(sc.get(&col, size_t(Mp) * Kp));
-    IEF_TRY(sc.get(&wh, size_t(W) * Kp));
-    IEF_TRY(launch_im2col(x, dtype, Mp, R, P, G, Kp, col, sms, st));
-    clip_pad_weight_kernel<<<grid_of((long long)W * Kp, sms), 256, 0, st>>>(p.conv1, W, K, Kp, wh);
-    count_launches(1);
-    GemmTcArgs g;
-    g.A_hi = reinterpret_cast<const bf16*>(col); g.W_hi = reinterpret_cast<const bf16*>(wh);
-    g.M = int(Mp); g.N = W; g.K = Kp; g.lda = Kp; g.ldw = Kp; g.fp16 = 1;
-    IEF_TRY(gemm_tc(g, ep, sms, st));
-  }
+  IEF_TRY(gemm_plan(plan, col, wc, int(Mp), W, Kp, ep, nullptr, sms, st));
   // class token, positional embedding and ln_pre -> the fp32 residual [N, T, W] (model.py:227-230)
   {
-    const int grid = grid_of(M * 32, sms);
+    const int grid = blocks_for(M * 32, sms);
 #define IEF_TOK(NV)                                                                                                  \
   case NV:                                                                                                           \
     clip_tokens_kernel<NV><<<grid, 256, 0, st>>>(patches, p.cls, p.pos, p.ln_pre_w, p.ln_pre_b, T, M, xr);          \

@@ -20,6 +20,7 @@ void keep_async_pool();              // once per device: the stream-ordered allo
 void count_launches(int n);          // kernels launched by this library (bench.py's gpu_launches)
 unsigned long long launch_count();
 int cuda_fail(cudaError_t e, const char* what, const char* file, int line);
+int device_sms(int* out);            // SM count of the current device
 
 #define IEF_CUDA(call)                                                                    \
   do {                                                                                    \

@@ -31,7 +31,7 @@ struct EpiParams {
   int ld_bf = 0;
   int hi_fp16 = 0;               // out_hi / out_lo receive fp16 instead of bf16
   // EPI_QKV: packed in-projection scattered into the attention kernel's operand layouts
-  //   q  [B, H, T, dhp]  (scaled by qscale, columns >= dh never written: kept zero by the allocator)
+  //   q  [B, H, T, dhp]  (scaled by qscale; columns >= dh are neither written nor read by the attention kernels)
   //   k  [B, H, T, dhp]
   //   vt [B, H, dh, Tpad] (transposed so that P.V is a K-major x K-major UMMA)
   bf16* q = nullptr;

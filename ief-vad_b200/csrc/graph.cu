@@ -11,7 +11,6 @@
 #include "attention.cuh"
 #include "elementwise.cuh"
 #include "gemm.cuh"
-#include "scratch.cuh"
 
 namespace iefvad {
 
@@ -176,27 +175,6 @@ simadj_softmax_kernel(const float* __restrict__ sim, int ld, const float* __rest
 }
 
 // ------------------------------------------------------------------------------------------------ copies
-// dst[r, c] = (r < rows && c < cols) ? src[r, c] : 0  for r < rows_p, c < cols_p (fp32 and/or bf16 hi / lo copies;
-// hi_fp16: dst_hi receives fp16 instead, no lo)
-__global__ void __launch_bounds__(256)
-pad2d_kernel(const float* __restrict__ src, int rows, int cols, long long ld_src, int rows_p, int cols_p,
-             float* __restrict__ dst_f32, bf16* __restrict__ dst_hi, bf16* __restrict__ dst_lo, int hi_fp16) {
-  const long long total = (long long)rows_p * cols_p;
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
-    const int r = int(i / cols_p), c = int(i - (long long)r * cols_p);
-    const float v = (r < rows && c < cols) ? src[r * ld_src + c] : 0.f;
-    if (dst_f32) dst_f32[i] = v;
-    if (dst_hi && hi_fp16) {
-      reinterpret_cast<__half*>(dst_hi)[i] = __float2half_rn(v);
-    } else if (dst_hi) {
-      bf16 h, l;
-      split_bf16(v, h, l);
-      dst_hi[i] = h;
-      if (dst_lo) dst_lo[i] = l;
-    }
-  }
-}
-
 // im2col of Conv1d(k = 5, pad = 2) along T: dst[t, k * Din + c] = x[t + k - 2, c] (0 outside [0, T)), rows t < Tp
 __global__ void __launch_bounds__(256)
 im2col5_kernel(const float* __restrict__ x, int T, int Din, int Tp, float* __restrict__ dst_f32, bf16* __restrict__ dst_hi,
@@ -258,55 +236,6 @@ add_bias_resid_kernel(const float* __restrict__ s, const float* __restrict__ bia
     }
     reinterpret_cast<float4*>(o)[i] = v;
   }
-}
-
-int blocks_for(long long n, int num_sms) {
-  long long b = (n + 255) / 256;
-  const long long cap = (long long)num_sms * 8;
-  return int(b < 1 ? 1 : (b > cap ? cap : b));
-}
-
-// one operand / result in the representation the plan needs: fp32 (plan < 0), bf16 hi (+ lo when plan == 1) or fp16
-// in `hi` (plan == 2)
-struct Mat {
-  float* f = nullptr;
-  bf16* hi = nullptr;
-  bf16* lo = nullptr;
-  int ld = 0;
-};
-
-int alloc_mat(Scratch& sc, Mat* m, size_t rows, int ld, int plan, bool zero = false) {
-  m->ld = ld;
-  if (plan < 0) return sc.get(&m->f, rows * ld, zero);
-  IEF_TRY(sc.get(&m->hi, rows * ld, zero));
-  if (plan == 1) IEF_TRY(sc.get(&m->lo, rows * ld, zero));
-  return IEFVAD_OK;
-}
-
-// C = epilogue(A . W^T) in the plan's arithmetic; `ep` carries bias / act / resid / alpha and the fp32 output, `dst`
-// (optional) receives the result in operand form for a following contraction.
-int gemm_plan(int plan, const Mat& A, const Mat& W, int M, int N, int K, EpiParams ep, const Mat* dst, int num_sms,
-              cudaStream_t st) {
-  if (dst) {
-    if (plan < 0) { ep.out_f32 = dst->f; ep.ld_f32 = dst->ld; }
-    else { ep.out_hi = dst->hi; ep.out_lo = dst->lo; ep.ld_bf = dst->ld; ep.hi_fp16 = (plan == 2); }
-  }
-  if (plan < 0) return gemm_simt(A.f, A.ld, W.f, W.ld, M, N, K, ep, st);
-  GemmTcArgs g;
-  g.A_hi = A.hi; g.A_lo = A.lo; g.W_hi = W.hi; g.W_lo = W.lo;
-  g.M = M; g.N = N; g.K = K; g.lda = A.ld; g.ldw = W.ld; g.nsplit = (plan == 1) ? 3 : 1; g.fp16 = (plan == 2);
-  return gemm_tc(g, ep, num_sms, st);
-}
-
-// src fp32 [rows, cols] (pitch ld_src) -> zero-padded operand [rows_p, cols_p]
-int to_mat(Scratch& sc, Mat* m, const float* src, int rows, int cols, long long ld_src, int rows_p, int cols_p, int plan,
-           int num_sms, cudaStream_t st) {
-  IEF_TRY(alloc_mat(sc, m, size_t(rows_p), cols_p, plan));
-  pad2d_kernel<<<blocks_for((long long)rows_p * cols_p, num_sms), 256, 0, st>>>(src, rows, cols, ld_src, rows_p, cols_p,
-                                                                                 m->f, m->hi, m->lo, plan == 2);
-  count_launches(1);
-  IEF_CUDA(cudaGetLastError());
-  return IEFVAD_OK;
 }
 
 int check_dims(const char* who, int Din, int Dout, int plan) {
@@ -411,26 +340,23 @@ int graph_convolution(const float* x, const float* adj, const float* wt, const f
   Mat w, cw;
   IEF_TRY(to_mat(sc, &w, wt, Dout, Din, Din, Dout, Din, plan, num_sms, st));
   if (residual == 2) IEF_TRY(to_mat(sc, &cw, conv_w, Dout, 5 * Din, 5 * Din, Dout, 5 * Din, plan, num_sms, st));
-  float *outp, *res32 = nullptr, *xpad = nullptr, *sup32 = nullptr;
+  float *outp, *res32 = nullptr, *sup32 = nullptr;
   IEF_TRY(sc.get(&outp, size_t(Tp) * Dout));
   if (residual == 2) IEF_TRY(sc.get(&res32, size_t(Tp) * Dout));
   for (long long b = 0; b < B; ++b) {
+    Scratch sb(st);                               // this batch element's operands, back to the pool at the end of the loop body
     const float* xb32 = x + b * T * Din;
     Mat xb;
-    IEF_TRY(to_mat(sc, &xb, xb32, T, Din, Din, Tp, Din, plan, num_sms, st));
+    IEF_TRY(to_mat(sb, &xb, xb32, T, Din, Din, Tp, Din, plan, num_sms, st));
     // residual term (layers.py:98-104): identity -> the (zero-padded) input itself; Conv1d -> one GEMM over im2col rows
     const float* resid = nullptr;
     if (residual == 1) {
-      if (plan < 0) resid = xb.f;
-      else {
-        if (!xpad) IEF_TRY(sc.get(&xpad, size_t(Tp) * Din));
-        pad2d_kernel<<<blocks_for((long long)Tp * Din, num_sms), 256, 0, st>>>(xb32, T, Din, Din, Tp, Din, xpad, nullptr, nullptr, 0);
-        count_launches(1);
-        resid = xpad;
-      }
+      Mat xf;                                     // the fp32 form of x_b (xb itself under plan -1)
+      if (plan >= 0) IEF_TRY(to_mat(sb, &xf, xb32, T, Din, Din, Tp, Din, -1, num_sms, st));
+      resid = plan < 0 ? xb.f : xf.f;
     } else if (residual == 2) {
       Mat col;
-      IEF_TRY(alloc_mat(sc, &col, size_t(Tp), 5 * Din, plan));
+      IEF_TRY(alloc_mat(sb, &col, size_t(Tp), 5 * Din, plan));
       im2col5_kernel<<<blocks_for((long long)Tp * 5 * Din, num_sms), 256, 0, st>>>(xb32, T, Din, Tp, col.f, col.hi, col.lo);
       count_launches(1);
       EpiParams ec;
@@ -454,11 +380,11 @@ int graph_convolution(const float* x, const float* adj, const float* wt, const f
     }
     // supportT [Dout, Tp] = W^T . x_b^T: C = A . W'^T with A = W^T [Dout, Din], W' = x_b [Tp, Din] -> K-major operand
     Mat supT;
-    IEF_TRY(alloc_mat(sc, &supT, size_t(Dout), Tp, plan));
+    IEF_TRY(alloc_mat(sb, &supT, size_t(Dout), Tp, plan));
     EpiParams e1;
     IEF_TRY(gemm_plan(plan, w, xb, Dout, Tp, Din, e1, &supT, num_sms, st));
     Mat ab;
-    IEF_TRY(to_mat(sc, &ab, adj + b * T * T, T, T, T, Tp, Tp, plan, num_sms, st));
+    IEF_TRY(to_mat(sb, &ab, adj + b * T * T, T, T, T, Tp, Tp, plan, num_sms, st));
     EpiParams e2;
     e2.bias = bias; e2.resid = resid; e2.ld_resid = Dout; e2.out_f32 = outp; e2.ld_f32 = Dout;
     IEF_TRY(gemm_plan(plan, ab, supT, Tp, Dout, Tp, e2, nullptr, num_sms, st));
@@ -469,29 +395,53 @@ int graph_convolution(const float* x, const float* adj, const float* wt, const f
   return IEFVAD_OK;
 }
 
+int alloc_attn_work(Scratch& sc, AttnWork* w, int plan, int N, int L, int D, int heads) {
+  const size_t M = size_t(N) * L;
+  const int dh = D / heads, dhp = (dh + 63) / 64 * 64, Tpad = (L + 7) / 8 * 8;
+  IEF_TRY(alloc_mat(sc, &w->ctx, M, D, plan == 1 ? 0 : plan));
+  if (plan < 0) return sc.get(&w->qkv32, M * 3 * D);
+  IEF_TRY(sc.get(&w->q, M * heads * dhp));
+  IEF_TRY(sc.get(&w->k, M * heads * dhp));
+  return sc.get(&w->vt, size_t(N) * heads * dh * Tpad);
+}
+
+int attention_sublayer(int plan, const Mat& x, const Mat& in_w, const float* in_b, const Mat& out_w, const float* out_b,
+                       int N, int L, int D, int heads, const float* attn_mask, const uint8_t* key_pad, const float* resid,
+                       float* out, const AttnWork& w, int num_sms, cudaStream_t st) {
+  const int M = N * L, dh = D / heads;
+  EpiParams e1;
+  e1.bias = in_b;
+  AttnTcArgs at;
+  if (plan < 0) {
+    e1.out_f32 = w.qkv32; e1.ld_f32 = 3 * D;
+  } else {
+    at.q = w.q; at.k = w.k; at.vt = w.vt; at.out = w.ctx.hi; at.ldo = D;
+    at.B = N; at.T = L; at.H = heads; at.dh = dh; at.Tpad = (L + 7) / 8 * 8;
+    at.attn_mask = attn_mask; at.key_pad = key_pad; at.fp16 = (plan == 2);
+    at.dhp = attn_qk_cols(at);
+    e1.mode = EPI_QKV; e1.q = w.q; e1.k = w.k; e1.vt = w.vt; e1.hi_fp16 = at.fp16;
+    e1.T = L; e1.H = heads; e1.dh = dh; e1.dhp = at.dhp; e1.Tpad = at.Tpad; e1.D = D; e1.qscale = 1.0f / sqrtf(float(dh));
+  }
+  IEF_TRY(gemm_plan(plan, x, in_w, M, 3 * D, D, e1, nullptr, num_sms, st));
+  IEF_TRY(plan < 0 ? attn_simt(w.qkv32, w.ctx.f, N, L, heads, dh, attn_mask, key_pad, st) : attn_tc(at, st));
+  EpiParams e2;
+  e2.bias = out_b; e2.resid = resid; e2.ld_resid = D; e2.out_f32 = out; e2.ld_f32 = D;
+  return gemm_plan(plan == 1 ? 0 : plan, w.ctx, out_w, M, D, D, e2, nullptr, num_sms, st);
+}
+
 int transformer_blocks(float* xa, const ResBlockParams* blocks, int layers, int L, int N, int D, int heads,
                        const float* attn_mask, const uint8_t* key_pad, int plan, int num_sms, cudaStream_t st) {
   if (layers == 0 || L == 0 || N == 0) return IEFVAD_OK;
   const long long M = (long long)N * L;
-  const int dh = D / heads;
-  const int dhp = (dh + 63) / 64 * 64, Tpad = (L + 7) / 8 * 8;
-  const float qscale = 1.0f / sqrtf(float(dh));
   const int f16 = (plan == 2);
   Scratch sc(st);
   float* xb;                                      // second residual buffer: x alternates xa -> xb -> xa in each block
   IEF_TRY(sc.get(&xb, size_t(M) * D));
-  Mat h, ctx, u;
+  Mat h, u;
   IEF_TRY(alloc_mat(sc, &h, size_t(M), D, plan));
-  IEF_TRY(alloc_mat(sc, &ctx, size_t(M), D, plan == 1 ? 0 : plan));
   IEF_TRY(alloc_mat(sc, &u, size_t(M), 4 * D, plan));
-  float* qkv32 = nullptr;
-  bf16 *q = nullptr, *k = nullptr, *vt = nullptr;
-  if (plan < 0) IEF_TRY(sc.get(&qkv32, size_t(M) * 3 * D));
-  else {
-    IEF_TRY(sc.get(&q, size_t(M) * heads * dhp, true));
-    IEF_TRY(sc.get(&k, size_t(M) * heads * dhp, true));
-    IEF_TRY(sc.get(&vt, size_t(N) * heads * dh * Tpad, true));
-  }
+  AttnWork aw;
+  IEF_TRY(alloc_attn_work(sc, &aw, plan, N, L, D, heads));
   std::vector<Mat> wmats(size_t(layers) * 4);
   for (int i = 0; i < layers; ++i) {
     const ResBlockParams& p = blocks[i];
@@ -504,26 +454,7 @@ int transformer_blocks(float* xa, const ResBlockParams* blocks, int layers, int 
     IEF_TRY(to_mat(sc, &wp, p.proj_w, D, 4 * D, 4 * D, D, 4 * D, plan, num_sms, st));
     // x = x + attn(ln_1(x))   (module.py:41)
     IEF_TRY(layernorm(xa, M, D, p.ln1_w, p.ln1_b, nullptr, nullptr, 1e-5f, h.f, h.hi, h.lo, num_sms, st, f16));
-    if (plan < 0) {
-      EpiParams e1;
-      e1.bias = p.in_b; e1.out_f32 = qkv32; e1.ld_f32 = 3 * D;
-      IEF_TRY(gemm_simt(h.f, D, wi.f, D, int(M), 3 * D, D, e1, st));
-      IEF_TRY(attn_simt(qkv32, ctx.f, N, L, heads, dh, attn_mask, key_pad, st));
-    } else {
-      EpiParams e1;
-      e1.mode = EPI_QKV; e1.bias = p.in_b; e1.q = q; e1.k = k; e1.vt = vt; e1.hi_fp16 = f16;
-      e1.T = L; e1.H = heads; e1.dh = dh; e1.dhp = dhp; e1.Tpad = Tpad; e1.D = D; e1.qscale = qscale;
-      IEF_TRY(gemm_plan(plan, h, wi, int(M), 3 * D, D, e1, nullptr, num_sms, st));
-      AttnTcArgs at;
-      at.q = q; at.k = k; at.vt = vt; at.out = ctx.hi; at.ldo = D;
-      at.B = N; at.T = L; at.H = heads; at.dh = dh; at.dhp = dhp; at.Tpad = Tpad;
-      at.attn_mask = attn_mask; at.key_pad = key_pad;
-      at.fp16 = f16;
-      IEF_TRY(attn_tc(at, st));
-    }
-    EpiParams e2;
-    e2.bias = p.out_b; e2.resid = xa; e2.ld_resid = D; e2.out_f32 = xb; e2.ld_f32 = D;
-    IEF_TRY(gemm_plan(plan == 1 ? 0 : plan, ctx, wo, int(M), D, D, e2, nullptr, num_sms, st));
+    IEF_TRY(attention_sublayer(plan, h, wi, p.in_b, wo, p.out_b, N, L, D, heads, attn_mask, key_pad, xa, xb, aw, num_sms, st));
     // x = x + mlp(ln_2(x))   (module.py:42): c_fc + QuickGELU, then c_proj with the residual
     IEF_TRY(layernorm(xb, M, D, p.ln2_w, p.ln2_b, nullptr, nullptr, 1e-5f, h.f, h.hi, h.lo, num_sms, st, f16));
     EpiParams e3;
@@ -540,7 +471,7 @@ int transformer_blocks(float* xa, const ResBlockParams* blocks, int layers, int 
 int transformer(const float* x, const ResBlockParams* blocks, int layers, int L, int N, int D, int heads,
                 const float* attn_mask, const uint8_t* key_pad, int plan, float* out, int num_sms, cudaStream_t st) {
   IEF_CHECK(x && out && blocks && layers >= 0 && L >= 0 && N >= 0, "transformer: bad argument");
-  IEF_CHECK(plan >= -1 && plan <= 2, "transformer: plan must be -1, 0, 1 or 2");
+  IEF_TRY(check_plan("transformer", plan));
   IEF_CHECK(D > 0 && D % 128 == 0 && heads > 0 && D % heads == 0, "transformer: width %d must be a multiple of 128 and of heads=%d", D, heads);
   const int dh = D / heads;
   IEF_CHECK(dh == 32 || dh == 64 || dh == 96 || dh == 128, "transformer: head dim %d unsupported (32, 64, 96, 128)", dh);

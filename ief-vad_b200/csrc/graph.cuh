@@ -2,7 +2,7 @@
 // model/module.py (dead code in the live reference graph, named by the north star), built from the same tcgen05
 // GEMM / attention / LayerNorm kernels as the live forward plus the kernels of graph.cu.
 #pragma once
-#include "common.cuh"
+#include "operand.cuh"
 
 namespace iefvad {
 
@@ -36,6 +36,22 @@ struct ResBlockParams {   // one ResidualAttentionBlock, model/module.py:20-43 (
 int transformer(const float* x, const ResBlockParams* blocks, int layers, int L, int N, int D, int heads,
                 const float* attn_mask, const uint8_t* key_pad, int plan, float* out, int num_sms,
                 cudaStream_t stream);
+
+// Workspace of attention_sublayer for N sequences of L tokens of width D, allocated once for any number of calls: q, k
+// and vt (16-bit plans) or the fp32 qkv (plan -1), and the context in the out-projection's operand form.
+struct AttnWork {
+  bf16 *q = nullptr, *k = nullptr, *vt = nullptr;
+  float* qkv32 = nullptr;
+  Mat ctx;
+};
+int alloc_attn_work(Scratch& sc, AttnWork* w, int plan, int N, int L, int D, int heads);
+
+// out = resid + out_proj(attention(in_proj(x))), nn.MultiheadAttention(x, x, x) in eval mode (torch/nn/functional.py:6244)
+// on batch-first x [N * L, D] in the plan's operand form; in_w [3D, D] and out_w [D, D] as operands too, resid (optional)
+// and out fp32 [N * L, D].  Plan 1 runs the out-projection single-pass on a bf16 context.
+int attention_sublayer(int plan, const Mat& x, const Mat& in_w, const float* in_b, const Mat& out_w, const float* out_b,
+                       int N, int L, int D, int heads, const float* attn_mask, const uint8_t* key_pad, const float* resid,
+                       float* out, const AttnWork& w, int num_sms, cudaStream_t stream);
 
 // The block loop of `transformer` on a BATCH-FIRST fp32 residual x [N, L, D], updated in place (the residual stays
 // fp32 under every plan).  Arguments as `transformer`, already validated by the caller.

@@ -402,9 +402,6 @@ int Model::forward(const void* img, const void* ev, int in_dtype, long long B, l
                                               (vr->chunk_start && vr->chunk_valid) ? nullptr : vr->rowmap + out0, vr->row_base + row0, status.as<int>()));
       else IEF_TRY(inverse_rowmap(vr->rowmap + out0, vr->row_base + row0, Mo, M, inv_map.as<int>(), num_sms, stream));
     }
-    // q / k rows: d_h padded to a multiple of 64 for the 128-byte-swizzled kernels; the short-sequence kernel takes
-    // 32-column chunks (64-byte swizzle), so d_h = 96 goes unpadded there (a quarter less q / k traffic)
-    const int dhq = (!fp32_plan && T <= 256 && dh % 32 == 0) ? dh : dhp;
     for (int m = 0; m < 2; ++m) {
       const bool ragged = vr && vr->chunk_start && vr->chunk_valid;
       const uint8_t* in = static_cast<const uint8_t*>(inputs[m]) + (ragged ? 0 : size_t(row0) * D * in_esize);
@@ -445,20 +442,21 @@ int Model::forward(const void* img, const void* ev, int in_dtype, long long B, l
           IEF_PROF(KC_LAYERNORM, double(M) * D * 8, layernorm(y32.as<float>(), M, D, ln_w[m][i], ln_b[m][i], last ? whiten_w[m] : nullptr,
                             last ? whiten_b[m] : nullptr, 1e-5f, x32.as<float>(), nullptr, nullptr, num_sms, stream));
         } else {
+          AttnTcArgs at;
+          at.q = qb.as<bf16>(); at.k = kb.as<bf16>(); at.vt = vtb.as<bf16>(); at.out = h_hi.as<bf16>(); at.ldo = D;
+          at.B = Bs; at.T = int(T); at.H = H; at.dh = dh; at.Tpad = Tpad;
+          if (dedup) { at.B = 1; at.T = int(Me); at.Tpad = int(Me); at.items = items_dev.as<int>(); at.n_chunks = n_items; }
+          at.fp16 = f16;
+          if (direct_compact && last && !ln_fused) at.row_out = inv_map.as<int>();
+          at.dhp = attn_qk_cols(at);
           EpiParams e1;
           e1.hi_fp16 = f16;
           e1.mode = EPI_QKV; e1.bias = ip.b; e1.q = qb.as<bf16>(); e1.k = kb.as<bf16>(); e1.vt = vtb.as<bf16>();
-          e1.T = dedup ? int(Me) : int(T); e1.H = H; e1.dh = dh; e1.dhp = dhq; e1.Tpad = dedup ? int(Me) : Tpad; e1.D = D; e1.qscale = qscale;
+          e1.T = at.T; e1.H = H; e1.dh = dh; e1.dhp = at.dhp; e1.Tpad = at.Tpad; e1.D = D; e1.qscale = qscale;
           GemmTcArgs g1;
           g1.A_hi = (i == 0) ? x16 : a_hi.as<bf16>(); g1.W_hi = f16 ? ip.w_h16 : ip.w_hi;
           g1.M = int(Me); g1.N = 3 * D; g1.K = D; g1.lda = D; g1.ldw = D; g1.fp16 = f16;
           IEF_PROF(KC_GEMM_QKV, 6.0 * Me * D * D, gemm_tc(g1, e1, num_sms, stream));
-          AttnTcArgs at;
-          at.q = qb.as<bf16>(); at.k = kb.as<bf16>(); at.vt = vtb.as<bf16>(); at.out = h_hi.as<bf16>(); at.ldo = D;
-          at.B = Bs; at.T = int(T); at.H = H; at.dh = dh; at.dhp = dhq; at.Tpad = Tpad;
-          if (dedup) { at.B = 1; at.T = int(Me); at.Tpad = int(Me); at.items = items_dev.as<int>(); at.n_chunks = n_items; }
-          at.fp16 = f16;
-          if (direct_compact && last && !ln_fused) at.row_out = inv_map.as<int>();
           IEF_PROF(KC_ATTN_TC, attn_flops, attn_tc(at, stream));
           if (ln_fused) {
             OutprojLnArgs oa;

@@ -47,6 +47,13 @@ int cuda_fail(cudaError_t e, const char* what, const char* file, int line) {
   return IEFVAD_ERR_CUDA;
 }
 
+int device_sms(int* out) {
+  int dev = 0;
+  IEF_CUDA(cudaGetDevice(&dev));
+  IEF_CUDA(cudaDeviceGetAttribute(out, cudaDevAttrMultiProcessorCount, dev));
+  return IEFVAD_OK;
+}
+
 static PFN_cuTensorMapEncodeTiled_v12000 get_encode() {
   static PFN_cuTensorMapEncodeTiled_v12000 fn = nullptr;
   static std::once_flag once;

@@ -1,5 +1,5 @@
 // Per-call device temporaries from the stream-ordered pool, released (stream-ordered) when the object goes out of scope.
-// Used by the stateless entry points of graph.cu and clip.cu.
+// Used by the stateless entry points (capi.cu, graph.cu, clip.cu).
 #pragma once
 #include <vector>
 
@@ -15,12 +15,11 @@ struct Scratch {   // stream-ordered temporaries
     for (void* p : ptrs) cudaFreeAsync(p, s);
   }
   template <typename T>
-  int get(T** out, size_t count, bool zero = false) {
+  int get(T** out, size_t count) {
     void* p = nullptr;
     const size_t bytes = (count ? count : 1) * sizeof(T);
     IEF_CUDA(cudaMallocAsync(&p, bytes, s));
     ptrs.push_back(p);
-    if (zero) IEF_CUDA(cudaMemsetAsync(p, 0, bytes, s));
     *out = static_cast<T*>(p);
     return IEFVAD_OK;
   }

@@ -183,7 +183,8 @@ int iefvad_outproj_ln(const float* ctx, const float* w, const float* bias, const
 /* nn.MultiheadAttention(batch_first=True)(x, x, x)[0] in eval mode (model/imf_vad.py:115; torch/nn/functional.py:6244).
  * x [B, T, D] fp32; in_w [3D, D], in_b [3D], out_w [D, D], out_b [D].  attn_mask: optional additive [T, T] fp32;
  * key_padding_mask: optional [B, T] uint8 (non-zero = ignore).  plan as for iefvad_linear; plan 2 runs the default model
- * plan HH's arithmetic (fp16 projections and fp16 attention, unpadded q / k rows where the model uses them). */
+ * plan HH's arithmetic (fp16 projections and fp16 attention).  Under every tensor-core plan q / k rows hold d_h columns
+ * where the short-sequence kernel runs (T <= 256 without masks), else d_h padded to a multiple of 64, as in the model. */
 int iefvad_mha(const float* x, const float* in_w, const float* in_b, const float* out_w, const float* out_b,
                int64_t B, int64_t T, int D, int num_heads, const float* attn_mask, const uint8_t* key_padding_mask,
                int plan, float* out, void* stream);
