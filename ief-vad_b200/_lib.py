@@ -14,6 +14,7 @@ ABI_VERSION = 1
 F32, F16, BF16 = 0, 1, 2
 NOISE = {"Gaussian": 0, "StudentT": 1}
 PLANS = {"fp32": -1, "B": 6, "HH": 56}
+DROPOUT_KINDS = {"philox": 0, "torch": 1}       # iefvad_dropout.kind
 
 if not os.path.exists(LIB_PATH):
     raise ImportError(
@@ -67,6 +68,9 @@ _SIGS = {
     "iefvad_process_feat": (_i, [_vp, _i, _vp, _i64, _i, _i, _vp, _vp, _i, _vp]),
     "iefvad_attention_train_fwd": (_i, [_vp, _i64, _i64, _i, _i, _f, C.c_uint64, _vp, _vp, _vp]),
     "iefvad_attention_train_bwd": (_i, [_vp, _vp, _vp, _vp, _i64, _i64, _i, _i, _f, C.c_uint64, _vp, _vp]),
+    "iefvad_attention_train_fwd_dropout": (_i, [_vp, _i64, _i64, _i, _i, _vp, _vp, _vp, _vp]),
+    "iefvad_attention_train_bwd_dropout": (_i, [_vp, _vp, _vp, _vp, _i64, _i64, _i, _i, _vp, _vp, _vp]),
+    "iefvad_dropout_mask": (_i, [_vp, _i64, _i, _i64, _vp, _vp]),
     "iefvad_layernorm_bwd": (_i, [_vp, _vp, _vp, _i64, _i, _f, _vp, _vp, _vp, _vp]),
     "iefvad_colsum": (_i, [_vp, _vp, _i64, _i, _vp, _vp]),
     "iefvad_fuse_bwd": (_i, [_vp] * 11 + [_i64, _f, _f] + [_vp] * 5),
@@ -103,6 +107,12 @@ for _name, (_res, _args) in _SIGS.items():
 
 if lib.iefvad_abi_version() != ABI_VERSION:
     raise ImportError(f"libiefvad.so ABI {lib.iefvad_abi_version()} != expected {ABI_VERSION}; rebuild it")
+
+
+class Dropout(C.Structure):
+    """struct iefvad_dropout: the mask of one training-attention call (include/iefvad.h)."""
+    _fields_ = [("kind", C.c_int32), ("p", C.c_double), ("seed", C.c_uint64), ("offset", C.c_uint64),
+                ("threads", C.c_int64)]
 
 
 class IefvadError(RuntimeError):

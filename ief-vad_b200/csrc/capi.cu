@@ -693,20 +693,78 @@ int iefvad_attention_train_fwd(const float* qkv, int64_t B, int64_t T, int heads
                                float* out, float* lse, void* stream) {
   IEF_CHECK(qkv && out && lse, "iefvad_attention_train_fwd: null argument");
   IEF_CHECK(B >= 0 && B < 65536 && T >= 0 && T < (1 << 24), "iefvad_attention_train_fwd: bad B / T");
-  return attn_train_fwd(qkv, int(B), int(T), heads, head_dim, p_drop, seed, out, lse, static_cast<cudaStream_t>(stream));
+  IEF_CHECK(p_drop >= 0.f && p_drop < 1.f, "attention dropout probability %f outside [0, 1)", p_drop);
+  return attn_train_fwd(qkv, int(B), int(T), heads, head_dim, dropout_philox(p_drop, seed, int(T)), out, lse,
+                        static_cast<cudaStream_t>(stream));
 }
 
-int iefvad_attention_train_bwd(const float* qkv, const float* out, const float* dout, const float* lse, int64_t B, int64_t T,
-                               int heads, int head_dim, float p_drop, uint64_t seed, float* dqkv, void* stream) {
-  IEF_CHECK(qkv && out && dout && lse && dqkv, "iefvad_attention_train_bwd: null argument");
-  IEF_CHECK(B >= 0 && B < 65536 && T >= 0 && T < (1 << 24), "iefvad_attention_train_bwd: bad B / T");
+static int attn_train_bwd_run(const float* qkv, const float* out, const float* dout, const float* lse, int64_t B, int64_t T,
+                              int heads, int head_dim, const DropoutDesc& drop, float* dqkv, void* stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   int sms = 0;
   IEF_TRY(device_sms(&sms));
   Scratch sc(st);
   float* delta = nullptr;
   IEF_TRY(sc.get(&delta, size_t(B) * heads * T));
-  return attn_train_bwd(qkv, out, dout, lse, int(B), int(T), heads, head_dim, p_drop, seed, delta, dqkv, sms, st);
+  return attn_train_bwd(qkv, out, dout, lse, int(B), int(T), heads, head_dim, drop, delta, dqkv, sms, st);
+}
+
+int iefvad_attention_train_bwd(const float* qkv, const float* out, const float* dout, const float* lse, int64_t B, int64_t T,
+                               int heads, int head_dim, float p_drop, uint64_t seed, float* dqkv, void* stream) {
+  IEF_CHECK(qkv && out && dout && lse && dqkv, "iefvad_attention_train_bwd: null argument");
+  IEF_CHECK(B >= 0 && B < 65536 && T >= 0 && T < (1 << 24), "iefvad_attention_train_bwd: bad B / T");
+  IEF_CHECK(p_drop >= 0.f && p_drop < 1.f, "attention dropout probability %f outside [0, 1)", p_drop);
+  return attn_train_bwd_run(qkv, out, dout, lse, B, T, heads, head_dim, dropout_philox(p_drop, seed, int(T)), dqkv, stream);
+}
+
+// iefvad_dropout -> the kernels' descriptor, every field checked (B, heads, T already range-checked by the caller)
+static int dropout_desc(const char* fn, const iefvad_dropout* d, int64_t B, int64_t heads, int64_t T, DropoutDesc* out) {
+  IEF_CHECK(d, "%s: null dropout descriptor", fn);
+  if (d->kind == IEFVAD_DROPOUT_PHILOX) {
+    IEF_CHECK(d->p >= 0.0 && d->p < 1.0, "%s: philox dropout probability %g outside [0, 1)", fn, d->p);
+    *out = dropout_philox(float(d->p), d->seed, int(T));
+    return IEFVAD_OK;
+  }
+  IEF_CHECK(d->kind == IEFVAD_DROPOUT_TORCH, "%s: dropout kind %d is neither IEFVAD_DROPOUT_PHILOX (0) nor "
+            "IEFVAD_DROPOUT_TORCH (1)", fn, int(d->kind));
+  IEF_CHECK(d->p > 0.0 && d->p < 1.0, "%s: torch dropout probability %g outside (0, 1)", fn, d->p);
+  IEF_CHECK(d->threads > 0 && d->threads < (int64_t(1) << 31), "%s: torch dropout threads %lld outside (0, 2^31)", fn,
+            (long long)d->threads);
+  IEF_CHECK(d->offset % 4 == 0, "%s: torch generator offset %llu is not a multiple of 4", fn,
+            (unsigned long long)d->offset);
+  const int64_t n = B * heads * T * T;
+  IEF_CHECK(n % 4 == 0, "%s: B*heads*T*T = %lld is not a multiple of 4 - torch's dropout draws such sizes with a narrower "
+            "vector width, which is not reproduced", fn, (long long)n);
+  *out = dropout_torch(d->p, d->seed, d->offset, unsigned(d->threads), int(T));
+  return IEFVAD_OK;
+}
+
+int iefvad_attention_train_fwd_dropout(const float* qkv, int64_t B, int64_t T, int heads, int head_dim,
+                                       const iefvad_dropout* drop, float* out, float* lse, void* stream) {
+  IEF_CHECK(qkv && out && lse, "iefvad_attention_train_fwd_dropout: null argument");
+  IEF_CHECK(B >= 0 && B < 65536 && T >= 0 && T < (1 << 24) && heads > 0, "iefvad_attention_train_fwd_dropout: bad B / T / heads");
+  DropoutDesc d;
+  IEF_TRY(dropout_desc("iefvad_attention_train_fwd_dropout", drop, B, heads, T, &d));
+  return attn_train_fwd(qkv, int(B), int(T), heads, head_dim, d, out, lse, static_cast<cudaStream_t>(stream));
+}
+
+int iefvad_attention_train_bwd_dropout(const float* qkv, const float* out, const float* dout, const float* lse, int64_t B,
+                                       int64_t T, int heads, int head_dim, const iefvad_dropout* drop, float* dqkv,
+                                       void* stream) {
+  IEF_CHECK(qkv && out && dout && lse && dqkv, "iefvad_attention_train_bwd_dropout: null argument");
+  IEF_CHECK(B >= 0 && B < 65536 && T >= 0 && T < (1 << 24) && heads > 0, "iefvad_attention_train_bwd_dropout: bad B / T / heads");
+  DropoutDesc d;
+  IEF_TRY(dropout_desc("iefvad_attention_train_bwd_dropout", drop, B, heads, T, &d));
+  return attn_train_bwd_run(qkv, out, dout, lse, B, T, heads, head_dim, d, dqkv, stream);
+}
+
+int iefvad_dropout_mask(const iefvad_dropout* drop, int64_t B, int heads, int64_t T, uint8_t* mask, void* stream) {
+  IEF_CHECK(mask, "iefvad_dropout_mask: null argument");
+  IEF_CHECK(B >= 0 && B < 65536 && T >= 0 && T < (1 << 24) && heads > 0 && B * heads * T < (int64_t(1) << 31),
+            "iefvad_dropout_mask: bad B / T / heads");
+  DropoutDesc d;
+  IEF_TRY(dropout_desc("iefvad_dropout_mask", drop, B, heads, T, &d));
+  return dropout_mask(d, int(B), heads, int(T), mask, static_cast<cudaStream_t>(stream));
 }
 
 int iefvad_layernorm_bwd(const float* x, const float* weight, const float* dy, int64_t rows, int dim, float eps, float* dx,

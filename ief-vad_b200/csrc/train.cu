@@ -6,7 +6,7 @@
 //
 //   attn_train_fwd / attn_train_bwd_{q,kv}  softmax(q k^T / sqrt(d)) v per (batch element, head) with the attention
 //                                           dropout of nn.MultiheadAttention (train mode, model/imf_vad.py:53,70) from a
-//                                           counter-based Philox4x32-10 stream keyed by (seed, head, query, key)
+//                                           counter-based Philox4x32-10 mask: the library's own or PyTorch's (philox.cuh)
 //   layernorm_bwd                           dx, dgamma, dbeta of nn.LayerNorm
 //   fuse_bwd                                backward of the uncertainty-weighted fusion (model/imf_vad.py:130-144)
 //   clas2_bwd                               backward of the MIL top-k BCE loss (train/loss.py:18-30)
@@ -36,7 +36,7 @@ constexpr int SROWS = 16;
 template <int DH>
 __global__ void __launch_bounds__(128)
 attn_train_fwd_kernel(const float* __restrict__ qkv, float* __restrict__ out, float* __restrict__ lse, int T, int H, int D,
-                      float qscale, uint32_t drop_thresh, float inv_keep, unsigned long long seed) {
+                      float qscale, DropoutDesc drop) {
   constexpr int NPL = DH / 32;
   __shared__ float Ks[32][DH + 1];
   __shared__ float Vs[32][DH];
@@ -83,7 +83,7 @@ attn_train_fwd_kernel(const float* __restrict__ qkv, float* __restrict__ out, fl
       l[i] = l[i] * alpha + warp_sum(p);         // the softmax denominator sums ALL keys; dropout acts on the weights
       m[i] = mx;
       float pd = p;
-      if (drop_thresh && key < T && tq < T) pd *= keep_scale(seed, bh, tq, key, drop_thresh, inv_keep);
+      if (drop.kind && key < T && tq < T) pd *= keep_scale(drop, bh, tq, key);
 #pragma unroll
       for (int e = 0; e < NPL; ++e) o[i][e] *= alpha;
       for (int jj = 0; jj < 32; ++jj) {
@@ -130,7 +130,7 @@ template <int DH>
 __global__ void __launch_bounds__(128)
 attn_train_bwd_q_kernel(const float* __restrict__ qkv, const float* __restrict__ dout, const float* __restrict__ lse,
                         const float* __restrict__ delta, float* __restrict__ dqkv, int T, int H, int D, float qscale,
-                        uint32_t drop_thresh, float inv_keep, unsigned long long seed) {
+                        DropoutDesc drop) {
   constexpr int NPL = DH / 32;
   __shared__ float Ks[32][DH + 1];
   __shared__ float Vs[32][DH + 1];
@@ -179,7 +179,7 @@ attn_train_bwd_q_kernel(const float* __restrict__ qkv, const float* __restrict__
       float ds = 0.f;
       if (key < T && tq < T) {
         const float p = expf(s - L[i]);
-        const float ks = drop_thresh ? keep_scale(seed, bh, tq, key, drop_thresh, inv_keep) : 1.f;
+        const float ks = drop.kind ? keep_scale(drop, bh, tq, key) : 1.f;
         ds = p * (dpd * ks - Dl[i]);
       }
       for (int jj = 0; jj < 32; ++jj) {
@@ -203,7 +203,7 @@ template <int DH>
 __global__ void __launch_bounds__(128)
 attn_train_bwd_kv_kernel(const float* __restrict__ qkv, const float* __restrict__ dout, const float* __restrict__ lse,
                          const float* __restrict__ delta, float* __restrict__ dqkv, int T, int H, int D, float qscale,
-                         uint32_t drop_thresh, float inv_keep, unsigned long long seed) {
+                         DropoutDesc drop) {
   constexpr int NPL = DH / 32;
   __shared__ float Qs[32][DH + 1];     // scaled queries of the block
   __shared__ float Gs[32][DH + 1];     // dout rows of the block
@@ -254,7 +254,7 @@ attn_train_bwd_kv_kernel(const float* __restrict__ qkv, const float* __restrict_
       float pd = 0.f, ds = 0.f;
       if (key < T && tq < T) {
         const float p = expf(s - Ls[lane]);
-        const float ks = drop_thresh ? keep_scale(seed, bh, tq, key, drop_thresh, inv_keep) : 1.f;
+        const float ks = drop.kind ? keep_scale(drop, bh, tq, key) : 1.f;
         pd = p * ks;
         ds = p * (dpd * ks - Ds[lane]);
       }
@@ -278,6 +278,16 @@ attn_train_bwd_kv_kernel(const float* __restrict__ qkv, const float* __restrict_
       dqkv[(base + key) * 3 * D + D + h * DH + lane + 32 * e] = dk[i][e];
       dqkv[(base + key) * 3 * D + 2 * D + h * DH + lane + 32 * e] = dv[i][e];
     }
+  }
+}
+
+// mask[bh, i, j] = 1 when the attention kernels keep weight (bh, query i, key j) under `drop` (the parity-test surface)
+__global__ void __launch_bounds__(kThreads)
+dropout_mask_kernel(DropoutDesc drop, long long n, uint8_t* __restrict__ mask) {
+  const long long T = drop.T;
+  for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x) {
+    const long long row = e / T;
+    mask[e] = keep_scale(drop, int(row / T), int(row % T), int(e % T)) != 0.f;
   }
 }
 
@@ -476,20 +486,18 @@ clas2_bwd_kernel(const float* __restrict__ logits, const float* __restrict__ mea
 }  // namespace
 
 // ================================================================ host wrappers
-int attn_train_fwd(const float* qkv, int B, int T, int H, int dh, float p_drop, unsigned long long seed, float* out, float* lse,
+int attn_train_fwd(const float* qkv, int B, int T, int H, int dh, DropoutDesc drop, float* out, float* lse,
                    cudaStream_t stream) {
-  IEF_CHECK(p_drop >= 0.f && p_drop < 1.f, "attention dropout probability %f outside [0, 1)", p_drop);
   const int D = H * dh;
   const dim3 grid((T + SROWS - 1) / SROWS, H, B);
   const float qs = 1.0f / sqrtf(float(dh));
-  const uint32_t thr = p_drop > 0.f ? uint32_t(double(p_drop) * 4294967296.0) : 0u;
-  const float ik = 1.f / (1.f - p_drop);
+  drop.T = T;
   if (B == 0 || T == 0) return IEFVAD_OK;
-  if (attn_train_mma_supported(dh)) return attn_train_fwd_mma(qkv, B, T, H, dh, qs, thr, ik, seed, out, lse, stream);
+  if (attn_train_mma_supported(dh)) return attn_train_fwd_mma(qkv, B, T, H, dh, qs, drop, out, lse, stream);
   switch (dh) {
-    case 32: attn_train_fwd_kernel<32><<<grid, 128, 0, stream>>>(qkv, out, lse, T, H, D, qs, thr, ik, seed); break;
-    case 64: attn_train_fwd_kernel<64><<<grid, 128, 0, stream>>>(qkv, out, lse, T, H, D, qs, thr, ik, seed); break;
-    case 96: attn_train_fwd_kernel<96><<<grid, 128, 0, stream>>>(qkv, out, lse, T, H, D, qs, thr, ik, seed); break;
+    case 32: attn_train_fwd_kernel<32><<<grid, 128, 0, stream>>>(qkv, out, lse, T, H, D, qs, drop); break;
+    case 64: attn_train_fwd_kernel<64><<<grid, 128, 0, stream>>>(qkv, out, lse, T, H, D, qs, drop); break;
+    case 96: attn_train_fwd_kernel<96><<<grid, 128, 0, stream>>>(qkv, out, lse, T, H, D, qs, drop); break;
     default: set_error("attn_train: head dim %d unsupported (32, 64, 96)", dh); return IEFVAD_ERR_INVALID;
   }
   count_launches(1);
@@ -498,22 +506,20 @@ int attn_train_fwd(const float* qkv, int B, int T, int H, int dh, float p_drop, 
 }
 
 int attn_train_bwd(const float* qkv, const float* out, const float* dout, const float* lse, int B, int T, int H, int dh,
-                   float p_drop, unsigned long long seed, float* delta_scratch, float* dqkv, int num_sms, cudaStream_t stream) {
-  IEF_CHECK(p_drop >= 0.f && p_drop < 1.f, "attention dropout probability %f outside [0, 1)", p_drop);
+                   DropoutDesc drop, float* delta_scratch, float* dqkv, int num_sms, cudaStream_t stream) {
   if (B == 0 || T == 0) return IEFVAD_OK;
   const int D = H * dh;
   const dim3 grid((T + SROWS - 1) / SROWS, H, B);
   const float qs = 1.0f / sqrtf(float(dh));
-  const uint32_t thr = p_drop > 0.f ? uint32_t(double(p_drop) * 4294967296.0) : 0u;
-  const float ik = 1.f / (1.f - p_drop);
+  drop.T = T;
   attn_delta_kernel<<<grid_for((long long)B * H * T * 32, num_sms), kThreads, 0, stream>>>(out, dout, delta_scratch, B, T, H, dh);
   if (attn_train_mma_supported(dh)) {
     count_launches(1);
-    return attn_train_bwd_mma(qkv, dout, lse, delta_scratch, B, T, H, dh, qs, thr, ik, seed, dqkv, stream);
+    return attn_train_bwd_mma(qkv, dout, lse, delta_scratch, B, T, H, dh, qs, drop, dqkv, stream);
   }
 #define IEF_BWD(DH_)                                                                                                          \
-  attn_train_bwd_q_kernel<DH_><<<grid, 128, 0, stream>>>(qkv, dout, lse, delta_scratch, dqkv, T, H, D, qs, thr, ik, seed);     \
-  attn_train_bwd_kv_kernel<DH_><<<grid, 128, 0, stream>>>(qkv, dout, lse, delta_scratch, dqkv, T, H, D, qs, thr, ik, seed);
+  attn_train_bwd_q_kernel<DH_><<<grid, 128, 0, stream>>>(qkv, dout, lse, delta_scratch, dqkv, T, H, D, qs, drop);              \
+  attn_train_bwd_kv_kernel<DH_><<<grid, 128, 0, stream>>>(qkv, dout, lse, delta_scratch, dqkv, T, H, D, qs, drop);
   switch (dh) {
     case 32: IEF_BWD(32) break;
     case 64: IEF_BWD(64) break;
@@ -522,6 +528,18 @@ int attn_train_bwd(const float* qkv, const float* out, const float* dout, const 
   }
 #undef IEF_BWD
   count_launches(3);
+  IEF_CUDA(cudaGetLastError());
+  return IEFVAD_OK;
+}
+
+int dropout_mask(DropoutDesc drop, int B, int H, int T, uint8_t* mask, cudaStream_t stream) {
+  const long long n = (long long)B * H * T * T;
+  if (n == 0) return IEFVAD_OK;
+  int sms = 0;
+  IEF_TRY(device_sms(&sms));
+  drop.T = T;
+  dropout_mask_kernel<<<grid_for(n, sms), kThreads, 0, stream>>>(drop, n, mask);
+  count_launches(1);
   IEF_CUDA(cudaGetLastError());
   return IEFVAD_OK;
 }

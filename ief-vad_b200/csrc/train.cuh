@@ -1,23 +1,25 @@
 // Internal interface of the training-step kernels (train.cu): SURVEY 8f row N3.
 #pragma once
 #include "common.cuh"
+#include "philox.cuh"
 
 namespace iefvad {
 
-// softmax(q k^T / sqrt(dh)) v with attention dropout (Philox4x32-10 keyed by seed; p_drop = 0 disables it).
-// qkv [B*T, 3*H*dh] fp32 (bias added, q unscaled) -> out [B*T, H*dh], lse [B, H, T]
-int attn_train_fwd(const float* qkv, int B, int T, int H, int dh, float p_drop, unsigned long long seed, float* out, float* lse,
-                   cudaStream_t stream);
+// softmax(q k^T / sqrt(dh)) v with attention dropout of mode `drop` (philox.cuh: dropout_philox / dropout_torch; its T is
+// set here).  qkv [B*T, 3*H*dh] fp32 (bias added, q unscaled) -> out [B*T, H*dh], lse [B, H, T]
+int attn_train_fwd(const float* qkv, int B, int T, int H, int dh, DropoutDesc drop, float* out, float* lse, cudaStream_t stream);
 // dqkv [B*T, 3*H*dh] from dout [B*T, H*dh]; delta_scratch: B*H*T floats
 int attn_train_bwd(const float* qkv, const float* out, const float* dout, const float* lse, int B, int T, int H, int dh,
-                   float p_drop, unsigned long long seed, float* delta_scratch, float* dqkv, int num_sms, cudaStream_t stream);
+                   DropoutDesc drop, float* delta_scratch, float* dqkv, int num_sms, cudaStream_t stream);
+// mask [B*H, T, T] uint8 (1 = kept) of mode `drop`: the keep decisions the attention kernels make, in torch's layout
+int dropout_mask(DropoutDesc drop, int B, int H, int T, uint8_t* mask, cudaStream_t stream);
 
-// the same on the tensor cores (mma.sync TF32, train_attn_mma.cu); qs = 1 / sqrt(dh), thr = p_drop * 2^32, ik = 1 / (1 - p_drop)
+// the same on the tensor cores (mma.sync TF32, train_attn_mma.cu); qs = 1 / sqrt(dh)
 bool attn_train_mma_supported(int dh);
-int attn_train_fwd_mma(const float* qkv, int B, int T, int H, int dh, float qs, uint32_t thr, float ik, unsigned long long seed,
+int attn_train_fwd_mma(const float* qkv, int B, int T, int H, int dh, float qs, const DropoutDesc& drop,
                        float* out, float* lse, cudaStream_t stream);
 int attn_train_bwd_mma(const float* qkv, const float* dout, const float* lse, const float* delta, int B, int T, int H, int dh,
-                       float qs, uint32_t thr, float ik, unsigned long long seed, float* dqkv, cudaStream_t stream);
+                       float qs, const DropoutDesc& drop, float* dqkv, cudaStream_t stream);
 
 int train_colsum_blocks(long long rows, int num_sms);
 // scratch: 2 * rows + 2 * train_colsum_blocks(rows) * D floats

@@ -142,7 +142,7 @@ __device__ __forceinline__ void mma_cols(float (&out)[DH / 8][4], const float (&
 template <int DH>
 __global__ void __launch_bounds__(kThreads)
 attn_fwd_mma_kernel(const float* __restrict__ qkv, float* __restrict__ out, float* __restrict__ lse, int T, int H, int D,
-                    float qscale, uint32_t drop_thresh, float inv_keep, unsigned long long seed) {
+                    float qscale, DropoutDesc drop) {
   constexpr int P = DH + 4;
   extern __shared__ uint32_t sm[];
   uint32_t* Qs = sm;                 // [BQ][P]
@@ -203,10 +203,10 @@ attn_fwd_mma_kernel(const float* __restrict__ qkv, float* __restrict__ out, floa
         s[nt][e] = expf(s[nt][e] - mx[e >> 1]);
         rs[e >> 1] += s[nt][e];                    // the softmax denominator sums ALL keys; dropout acts on the weights
       }
-      if (drop_thresh) {
+      if (drop.kind) {
         const int key = k0 + nt * 8 + 2 * t;
-        const float2 k0v = keep_scale2(seed, bh, rq[0], key, drop_thresh, inv_keep);
-        const float2 k1v = keep_scale2(seed, bh, rq[1], key, drop_thresh, inv_keep);
+        const float2 k0v = keep_scale2(drop, bh, rq[0], key);
+        const float2 k1v = keep_scale2(drop, bh, rq[1], key);
         s[nt][0] *= k0v.x; s[nt][1] *= k0v.y; s[nt][2] *= k1v.x; s[nt][3] *= k1v.y;
       }
     }
@@ -241,7 +241,7 @@ template <int DH>
 __global__ void __launch_bounds__(kThreads)
 attn_bwd_q_mma_kernel(const float* __restrict__ qkv, const float* __restrict__ dout, const float* __restrict__ lse,
                       const float* __restrict__ delta, float* __restrict__ dqkv, int T, int H, int D, float qscale,
-                      uint32_t drop_thresh, float inv_keep, unsigned long long seed) {
+                      DropoutDesc drop) {
   constexpr int P = DH + 4;
   extern __shared__ uint32_t sm[];
   uint32_t* Qs = sm;                 // [BQ][P] scaled queries
@@ -291,9 +291,9 @@ attn_bwd_q_mma_kernel(const float* __restrict__ qkv, const float* __restrict__ d
     for (int nt = 0; nt < 4; ++nt) {
       const int key = k0 + nt * 8 + 2 * t;
       float2 kv[2] = {make_float2(1.f, 1.f), make_float2(1.f, 1.f)};
-      if (drop_thresh) {
-        kv[0] = keep_scale2(seed, bh, rq[0], key, drop_thresh, inv_keep);
-        kv[1] = keep_scale2(seed, bh, rq[1], key, drop_thresh, inv_keep);
+      if (drop.kind) {
+        kv[0] = keep_scale2(drop, bh, rq[0], key);
+        kv[1] = keep_scale2(drop, bh, rq[1], key);
       }
 #pragma unroll
       for (int e = 0; e < 4; ++e) {
@@ -322,7 +322,7 @@ template <int DH>
 __global__ void __launch_bounds__(kThreads)
 attn_bwd_kv_mma_kernel(const float* __restrict__ qkv, const float* __restrict__ dout, const float* __restrict__ lse,
                        const float* __restrict__ delta, float* __restrict__ dqkv, int T, int H, int D, float qscale,
-                       uint32_t drop_thresh, float inv_keep, unsigned long long seed) {
+                       DropoutDesc drop) {
   constexpr int P = DH + 4;
   extern __shared__ uint32_t sm[];
   uint32_t* Ks = sm;                 // [BQ][P] this CTA's keys
@@ -381,7 +381,7 @@ attn_bwd_kv_mma_kernel(const float* __restrict__ qkv, const float* __restrict__ 
         const int qc = nt * 8 + 2 * t + (e & 1), tq = q0 + qc, key = rk[e >> 1];
         const bool valid = tq < T && key < T;
         const float p = valid ? expf(st[nt][e] * qscale - Ls[qc]) : 0.f;      // the streamed queries are unscaled
-        const float ks = (drop_thresh && valid) ? keep_scale(seed, bh, tq, key, drop_thresh, inv_keep) : 1.f;
+        const float ks = (drop.kind && valid) ? keep_scale(drop, bh, tq, key) : 1.f;
         st[nt][e] = p * ks;                                   // dropped weights P~^T
         dpt[nt][e] = p * (dpt[nt][e] * ks - Ds[qc]);          // dS^T
       }
@@ -414,7 +414,7 @@ bool attn_train_mma_supported(int dh) {
   return !off && (dh == 32 || dh == 64 || dh == 96 || dh == 128);
 }
 
-int attn_train_fwd_mma(const float* qkv, int B, int T, int H, int dh, float qs, uint32_t thr, float ik, unsigned long long seed,
+int attn_train_fwd_mma(const float* qkv, int B, int T, int H, int dh, float qs, const DropoutDesc& drop,
                        float* out, float* lse, cudaStream_t stream) {
   const dim3 grid((T + BQ - 1) / BQ, H, B);
 #define IEF_FWD(DH_)                                                                                                  \
@@ -422,7 +422,7 @@ int attn_train_fwd_mma(const float* qkv, int B, int T, int H, int dh, float qs, 
     const size_t smem = size_t(BQ + 4 * BC) * (DH_ + 4) * 4;                                                           \
     static bool set = false;                                                                                           \
     if (!set) { IEF_TRY(set_smem(attn_fwd_mma_kernel<DH_>, smem)); set = true; }                                       \
-    attn_fwd_mma_kernel<DH_><<<grid, kThreads, smem, stream>>>(qkv, out, lse, T, H, H * dh, qs, thr, ik, seed);         \
+    attn_fwd_mma_kernel<DH_><<<grid, kThreads, smem, stream>>>(qkv, out, lse, T, H, H * dh, qs, drop);         \
   }
   switch (dh) {
     case 32: IEF_FWD(32) break;
@@ -438,7 +438,7 @@ int attn_train_fwd_mma(const float* qkv, int B, int T, int H, int dh, float qs, 
 }
 
 int attn_train_bwd_mma(const float* qkv, const float* dout, const float* lse, const float* delta, int B, int T, int H, int dh,
-                       float qs, uint32_t thr, float ik, unsigned long long seed, float* dqkv, cudaStream_t stream) {
+                       float qs, const DropoutDesc& drop, float* dqkv, cudaStream_t stream) {
   const dim3 grid((T + BQ - 1) / BQ, H, B);
 #define IEF_BWD(DH_)                                                                                                            \
   {                                                                                                                              \
@@ -449,8 +449,8 @@ int attn_train_bwd_mma(const float* qkv, const float* dout, const float* lse, co
       IEF_TRY(set_smem(attn_bwd_kv_mma_kernel<DH_>, smem));                                                                      \
       set = true;                                                                                                                \
     }                                                                                                                            \
-    attn_bwd_q_mma_kernel<DH_><<<grid, kThreads, smem, stream>>>(qkv, dout, lse, delta, dqkv, T, H, H * dh, qs, thr, ik, seed);   \
-    attn_bwd_kv_mma_kernel<DH_><<<grid, kThreads, smem, stream>>>(qkv, dout, lse, delta, dqkv, T, H, H * dh, qs, thr, ik, seed);  \
+    attn_bwd_q_mma_kernel<DH_><<<grid, kThreads, smem, stream>>>(qkv, dout, lse, delta, dqkv, T, H, H * dh, qs, drop);   \
+    attn_bwd_kv_mma_kernel<DH_><<<grid, kThreads, smem, stream>>>(qkv, dout, lse, delta, dqkv, T, H, H * dh, qs, drop);  \
   }
   switch (dh) {
     case 32: IEF_BWD(32) break;

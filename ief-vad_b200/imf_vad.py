@@ -44,6 +44,10 @@ class MultiModal_Fusion_Attn_Iter(nn.Module):
         self.nu = nu
         self.epsilon = epsilon
         self.dropout = dropout          # attention dropout only acts in train(); this path is forward-only (eval)
+        # mask of the train() attention dropout: "philox" = the library's own counter-based mask, seeded from torch's CPU
+        # generator; "torch" = PyTorch's own mask, drawn from (and advancing) the device's CUDA generator exactly like
+        # nn.MultiheadAttention does, so a seeded run sees the reference's masks and random streams (include/iefvad.h)
+        self.dropout_rng = "philox"
         self.precision = os.environ.get("IEFVAD_PLAN", "HH")
         # valid-rows evaluation forward: compute the identical zero-pad rows of a chunk once (DESIGN.md, pad de-duplication)
         self.pad_dedup = True
@@ -208,6 +212,8 @@ class MultiModal_Fusion_Attn_Iter(nn.Module):
                 with_scores: bool = False) -> Dict[str, torch.Tensor]:
         if self.noise_model not in _lib.NOISE:
             raise ValueError("Unsupported noise_model. Choose 'Gaussian' or 'StudentT'.")
+        if self.dropout_rng not in _lib.DROPOUT_KINDS:
+            raise ValueError(f"unknown dropout_rng {self.dropout_rng!r}; choose from {sorted(_lib.DROPOUT_KINDS)}")
         if not (image_features.is_cuda and event_features.is_cuda):
             raise RuntimeError("IEF-VAD B200 path is CUDA-only: inputs must live on an sm_100a device "
                                "(there is no CPU fallback)")
@@ -259,20 +265,48 @@ class MultiModal_Fusion_Attn_Iter(nn.Module):
 
     def _forward_train(self, image_features: torch.Tensor, event_features: torch.Tensor) -> Dict[str, torch.Tensor]:
         """model/imf_vad.py:109-161 with a grad_fn (train.ForwardFn): what `loss.backward()` of train/ucf_train.py:105 needs.
-        Attention dropout (p = self.dropout) is applied in train() mode only, like nn.MultiheadAttention; every call draws a
-        fresh Philox seed from torch's CPU generator, so `torch.manual_seed` makes runs reproducible."""
+        Attention dropout (p = self.dropout) is applied in train() mode only, like nn.MultiheadAttention.  dropout_rng
+        "philox": every call draws a fresh Philox seed from torch's CPU generator, so `torch.manual_seed` makes runs
+        reproducible.  "torch": the CPU generator is left alone; the four attention layers take torch.native_dropout's
+        masks at consecutive offsets of the device's CUDA generator (image L0, L1, event L0, L1, the reference's order),
+        which is then advanced past them - the masks and every later CUDA draw are the reference's."""
         from . import train
         if image_features.dim() != 3 or image_features.shape != event_features.shape or image_features.shape[-1] != self.embed_dim:
             raise RuntimeError(f"expected two [B, T, {self.embed_dim}] tensors, got {tuple(image_features.shape)} "
                                f"and {tuple(event_features.shape)}")
         p_drop = float(self.dropout) if self.training else 0.0
-        seed = int(torch.randint(0, 2 ** 62, (1,)).item()) if p_drop > 0 else 0
+        B, T = int(image_features.shape[0]), int(image_features.shape[1])
+        seed, offsets, threads = 0, None, 0
+        if p_drop > 0 and self.dropout_rng == "torch" and B * T > 0:
+            seed, offsets, threads = self._torch_dropout_state(image_features.device, B * self.num_heads * T * T)
+        elif p_drop > 0:
+            seed = int(torch.randint(0, 2 ** 62, (1,)).item())
         cfg = dict(layers=self.num_layers, steps=self.num_refinement_steps, heads=self.num_heads, p_drop=p_drop, seed=seed,
-                   lambda_ref=float(self.lambda_ref), noise_model=self.noise_model, nu=float(self.nu),
-                   epsilon=float(self.epsilon))
+                   offsets=offsets, threads=threads, lambda_ref=float(self.lambda_ref), noise_model=self.noise_model,
+                   nu=float(self.nu), epsilon=float(self.epsilon))
         outs = train.ForwardFn.apply(cfg, image_features, event_features, *train.param_list(self))
         keys = ("fused", "logits", "image_mu", "event_mu", "image_logvar", "event_logvar", "w_i", "w_e")
         return dict(zip(keys, outs))
+
+    def _torch_dropout_state(self, device: torch.device, n: int):
+        """(seed, per-layer offsets, launch width) of torch.native_dropout on the n = B*H*T*T attention weights of each
+        layer, read from the CUDA generator of `device`, which is advanced past all of them as the reference's forward
+        would advance it."""
+        from . import ops
+        if torch.cuda.is_current_stream_capturing():
+            raise RuntimeError("dropout_rng = 'torch' reads and advances the CUDA generator on the host, which CUDA-graph "
+                               "capture does not support; capture with dropout_rng = 'philox' or in eval() mode")
+        if n % 4:
+            raise RuntimeError(f"dropout_rng = 'torch' needs B*heads*T*T to be a multiple of 4 (got {n}): torch draws other "
+                               "sizes with a narrower vector width, which the kernels do not reproduce")
+        torch.cuda.init()                                           # default_generators is filled on initialisation
+        index = device.index if device.index is not None else torch.cuda.current_device()
+        gen = torch.cuda.default_generators[index]
+        threads, advance = ops.torch_dropout_launch(n, index)
+        seed, offset = int(gen.initial_seed()), int(gen.get_offset())
+        layers = 2 * self.num_layers                                # image L0 .. L-1, then event L0 .. L-1
+        gen.set_offset(offset + layers * advance)
+        return seed, [offset + k * advance for k in range(layers)], threads
 
     def _graph_replay(self, device, B, T, D, img, ev, with_scores, launch):
         """One CUDA-graph replay of the forward for a small [B, T] problem, or None (too large, disabled, already

@@ -4,6 +4,7 @@ Every function takes CUDA tensors, allocates its outputs with torch and launches
 There is no CPU implementation: a non-CUDA tensor raises."""
 from __future__ import annotations
 
+import ctypes as C
 from typing import Optional, Tuple
 
 import torch
@@ -232,27 +233,72 @@ def auc_ap_multi(scores, pos, member, num_subsets: int, repeat: int = 16):
 
 
 # ------------------------------------------------------------------------------------------------ training step (row N3)
-def attention_train_fwd(qkv, B: int, T: int, heads: int, p_drop: float = 0.0, seed: int = 0):
-    """dropout(softmax(q k^T / sqrt(dh))) v of nn.MultiheadAttention in train mode -> (out [B*T, D], lse [B, H, T])."""
+def torch_dropout_launch(n: int, device=None) -> Tuple[int, int]:
+    """Launch width and generator advance of torch's CUDA dropout (torch.native_dropout) on n elements of `device`:
+    256-thread blocks, grid = min(SMs * (max threads per SM / 256), ceil(n / 256)) -> (threads G = grid * 256, offset
+    increment ((n - 1) / (G * 4) + 1) * 4).  G depends on the SM count, so the mask does too (include/iefvad.h)."""
+    props = torch.cuda.get_device_properties(device)
+    grid = min(props.multi_processor_count * (props.max_threads_per_multi_processor // 256), (n + 255) // 256)
+    G = grid * 256
+    return G, (((n - 1) // (G * 4) + 1) * 4 if n > 0 else 0)
+
+
+def _dropout(rng: str, p_drop: float, seed: int, offset: int, threads: int):
+    kind = _lib.DROPOUT_KINDS.get(rng)
+    if kind is None:
+        raise ValueError(f"unknown dropout rng {rng!r}; choose from {sorted(_lib.DROPOUT_KINDS)}")
+    return _lib.Dropout(kind, float(p_drop), int(seed), int(offset), int(threads))
+
+
+def attention_train_fwd(qkv, B: int, T: int, heads: int, p_drop: float = 0.0, seed: int = 0, rng: str = "philox",
+                        offset: int = 0, threads: int = 0):
+    """dropout(softmax(q k^T / sqrt(dh))) v of nn.MultiheadAttention in train mode -> (out [B*T, D], lse [B, H, T]).
+    rng "philox": the library's own mask keyed by `seed`; "torch": torch.native_dropout's mask for a CUDA generator at
+    (seed, offset), launch width `threads` (torch_dropout_launch) - the caller advances the generator."""
     qkv = _f32c(qkv, "attention_train_fwd")
     D = qkv.shape[-1] // 3
     out = torch.empty((B * T, D), dtype=torch.float32, device=qkv.device)
     lse = torch.empty((B, heads, T), dtype=torch.float32, device=qkv.device)
     with torch.cuda.device(qkv.device):
-        _lib.check(_lib.lib.iefvad_attention_train_fwd(qkv.data_ptr(), B, T, heads, D // heads, float(p_drop), int(seed),
-                                                       out.data_ptr(), lse.data_ptr(), _stream(qkv)))
+        if rng == "philox":
+            _lib.check(_lib.lib.iefvad_attention_train_fwd(qkv.data_ptr(), B, T, heads, D // heads, float(p_drop), int(seed),
+                                                           out.data_ptr(), lse.data_ptr(), _stream(qkv)))
+        else:
+            drop = _dropout(rng, p_drop, seed, offset, threads)
+            _lib.check(_lib.lib.iefvad_attention_train_fwd_dropout(qkv.data_ptr(), B, T, heads, D // heads, C.byref(drop),
+                                                                   out.data_ptr(), lse.data_ptr(), _stream(qkv)))
     return out, lse
 
 
-def attention_train_bwd(qkv, out, dout, lse, B: int, T: int, heads: int, p_drop: float = 0.0, seed: int = 0):
+def attention_train_bwd(qkv, out, dout, lse, B: int, T: int, heads: int, p_drop: float = 0.0, seed: int = 0,
+                        rng: str = "philox", offset: int = 0, threads: int = 0):
+    """dqkv of attention_train_fwd, regenerating the same mask (same p_drop / seed / rng / offset / threads)."""
     qkv, out, dout, lse = (_f32c(t, "attention_train_bwd") for t in (qkv, out, dout, lse))
     D = qkv.shape[-1] // 3
     dqkv = torch.empty_like(qkv)
     with torch.cuda.device(qkv.device):
-        _lib.check(_lib.lib.iefvad_attention_train_bwd(qkv.data_ptr(), out.data_ptr(), dout.data_ptr(), lse.data_ptr(), B, T,
-                                                       heads, D // heads, float(p_drop), int(seed), dqkv.data_ptr(),
-                                                       _stream(qkv)))
+        if rng == "philox":
+            _lib.check(_lib.lib.iefvad_attention_train_bwd(qkv.data_ptr(), out.data_ptr(), dout.data_ptr(), lse.data_ptr(),
+                                                           B, T, heads, D // heads, float(p_drop), int(seed),
+                                                           dqkv.data_ptr(), _stream(qkv)))
+        else:
+            drop = _dropout(rng, p_drop, seed, offset, threads)
+            _lib.check(_lib.lib.iefvad_attention_train_bwd_dropout(qkv.data_ptr(), out.data_ptr(), dout.data_ptr(),
+                                                                   lse.data_ptr(), B, T, heads, D // heads, C.byref(drop),
+                                                                   dqkv.data_ptr(), _stream(qkv)))
     return dqkv
+
+
+def dropout_mask(B: int, heads: int, T: int, p_drop: float, seed: int, rng: str = "torch", offset: int = 0,
+                 threads: int = 0, device=None) -> torch.Tensor:
+    """uint8 [B*heads, T, T] (1 = kept): the keep decisions of the training attention under the given mask, in the layout
+    of torch.native_dropout's mask (iefvad_dropout_mask)."""
+    drop = _dropout(rng, p_drop, seed, offset, threads)
+    device = torch.device("cuda") if device is None else torch.device(device)
+    mask = torch.empty((B * heads, T, T), dtype=torch.uint8, device=device)
+    with torch.cuda.device(mask.device):
+        _lib.check(_lib.lib.iefvad_dropout_mask(C.byref(drop), B, heads, T, mask.data_ptr(), _stream(mask)))
+    return mask
 
 
 def layernorm_bwd(x, weight, dy, eps: float = 1e-5):

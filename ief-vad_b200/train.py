@@ -12,10 +12,12 @@ csrc/train_attn_mma.cu, fp32 LayerNorm / fusion kernels) keeping what the backwa
 libiefvad.so kernels too: dgrad = linear(dY, W^T), wgrad = linear(dY^T, X^T) on the same tcgen05 GEMM, attention /
 LayerNorm / fusion / ReLU backward kernels of csrc/train.cu.  torch only owns the buffers and the autograd graph.
 
-Attention dropout (p = 0.1, active in train() mode like nn.MultiheadAttention): a counter-based Philox4x32-10 mask, a
-pure function of (seed, layer, batch element, head, query, key) documented in include/iefvad.h - regenerated, not
-stored, by the backward.  It is not PyTorch's generator stream, so train-mode runs match the reference statistically;
-in eval() mode (or with dropout = 0) forward and gradients match the reference's autograd to fp32 GEMM accuracy."""
+Attention dropout (p = 0.1, active in train() mode like nn.MultiheadAttention): a counter-based Philox4x32-10 mask,
+regenerated, not stored, by the backward (include/iefvad.h: iefvad_dropout).  With `dropout_rng = "philox"` (the default)
+it is the library's own mask, a pure function of (seed, layer, batch element, head, query, key), so train-mode runs
+match the reference statistically; with `dropout_rng = "torch"` it is torch.native_dropout's mask for the CUDA
+generator's state, bit for bit, so train-mode forward and gradients match the reference's autograd to fp32 GEMM
+accuracy, as they do in eval() mode (or with dropout = 0)."""
 from __future__ import annotations
 
 from typing import List
@@ -41,6 +43,14 @@ def _wgrad(dy, x, alpha=1.0):
     """dW [out, in] = alpha * dY^T . X from row-major dY [M, out], X [M, in] (iefvad_wgrad: both operands transposed straight
     into the GEMM's bf16 hi / lo form, split-K over the rows)."""
     return ops.wgrad(dy, x, alpha)
+
+
+def _drop(cfg, mi: int, i: int) -> dict:
+    """Dropout arguments of attention layer i of modality mi (0 image, 1 event) for ops.attention_train_fwd / _bwd."""
+    if cfg["offsets"] is not None:
+        return dict(p_drop=cfg["p_drop"], seed=cfg["seed"], rng="torch", offset=cfg["offsets"][mi * cfg["layers"] + i],
+                    threads=cfg["threads"])
+    return dict(p_drop=cfg["p_drop"], seed=cfg["seed"] + 1000 * mi + i)
 
 
 def param_list(temporal) -> List[torch.nn.Parameter]:
@@ -71,7 +81,6 @@ class ForwardFn(torch.autograd.Function):
         B, T, D = img.shape
         M = B * T
         L, R, H = cfg["layers"], cfg["steps"], cfg["heads"]
-        p_drop, seed = cfg["p_drop"], cfg["seed"]
         it = iter(params)
         saved = []                      # tensors for backward, in the order backward pops them
         enc, heads_out = {}, {}
@@ -80,7 +89,7 @@ class ForwardFn(torch.autograd.Function):
             for i in range(L):
                 w_in, b_in, w_o, b_o, g, bt = (next(it) for _ in range(6))
                 qkv = _lin(x, w_in, b_in)
-                ctx_, lse = ops.attention_train_fwd(qkv, B, T, H, p_drop, seed + 1000 * mi + i)
+                ctx_, lse = ops.attention_train_fwd(qkv, B, T, H, **_drop(cfg, mi, i))
                 y = _lin(ctx_, w_o, b_o, resid=x)                                   # x + MHA(x)        :115-116
                 saved += [x, qkv, ctx_, lse, y]
                 x = ops.layernorm(y, g, bt)
@@ -117,7 +126,7 @@ class ForwardFn(torch.autograd.Function):
         B, T, D = ctx.shape
         M = B * T
         L, R, H = cfg["layers"], cfg["steps"], cfg["heads"]
-        p_drop, seed, lam = cfg["p_drop"], cfg["seed"], cfg["lambda_ref"]
+        lam = cfg["lambda_ref"]
         saved = list(ctx.saved_tensors[:ctx.n_saved])
         params = list(ctx.saved_tensors[ctx.n_saved:])
         grads: List[torch.Tensor] = [None] * len(params)
@@ -173,7 +182,7 @@ class ForwardFn(torch.autograd.Function):
                 dy, grads[p0 + 4], grads[p0 + 5] = ops.layernorm_bwd(y, g, dxm)
                 grads[p0 + 2] = _wgrad(dy, ctx_)
                 grads[p0 + 3] = ops.colsum(dy)
-                dqkv = ops.attention_train_bwd(qkv, ctx_, _dgrad(dy, w_o), lse, B, T, H, p_drop, seed + 1000 * mi + i)
+                dqkv = ops.attention_train_bwd(qkv, ctx_, _dgrad(dy, w_o), lse, B, T, H, **_drop(cfg, mi, i))
                 grads[p0] = _wgrad(dqkv, x)
                 grads[p0 + 1] = ops.colsum(dqkv)
                 dxm = _dgrad(dqkv, w_in, resid=dy)     # residual path + attention path

@@ -350,16 +350,49 @@ int iefvad_bench_gemm(int64_t M, int N, int K, int nsplit, int tile_n, int stage
 /* nn.MultiheadAttention's core in TRAIN mode (model/imf_vad.py:53,70: dropout 0.1 on the attention weights,
  * torch/nn/functional.py:6643-6647): out = dropout(softmax(q k^T / sqrt(head_dim))) v per (batch element, head).
  * qkv [B*T, 3*heads*head_dim] (in-projection output, bias added, q unscaled); out [B*T, heads*head_dim]; lse [B, heads, T]
- * = log-sum-exp of the scores (saved for the backward).  The dropout mask is a pure function of (seed, head, query, key):
- * Philox4x32-10 with key = (seed & 0xffffffff, seed >> 32) and counter = (key >> 2, query, b * heads + h, 0), word (key & 3),
- * dropped when the word < uint32(double(p_drop) * 2^32), kept weights scaled by 1.f / (1.f - p_drop) (restated in
- * oracle/iefvad_oracle.py: attention_keep) - NOT PyTorch's generator stream (no kernel can reproduce that),
- * so train-mode parity with the reference is statistical; p_drop = 0 gives the eval-mode arithmetic. */
+ * = log-sum-exp of the scores (saved for the backward).  These two entry points use the library's own dropout mask
+ * (IEFVAD_DROPOUT_PHILOX below), a pure function of (seed, head, query, key): Philox4x32-10 with key =
+ * (seed & 0xffffffff, seed >> 32) and counter = (key >> 2, query, b * heads + h, 0), word (key & 3), dropped when the word
+ * < uint32(double(p_drop) * 2^32), kept weights scaled by 1.f / (1.f - p_drop) (restated in oracle/iefvad_oracle.py:
+ * attention_keep); p_drop = 0 gives the eval-mode arithmetic.  PyTorch's own mask for the same generator state is
+ * available too, through the *_dropout entry points below (IEFVAD_DROPOUT_TORCH). */
 int iefvad_attention_train_fwd(const float* qkv, int64_t B, int64_t T, int heads, int head_dim, float p_drop, uint64_t seed,
                                float* out, float* lse, void* stream);
 /* dqkv [B*T, 3*heads*head_dim] <- dout [B*T, heads*head_dim], recomputing the weights (and the same mask) from qkv / lse */
 int iefvad_attention_train_bwd(const float* qkv, const float* out, const float* dout, const float* lse, int64_t B, int64_t T,
                                int heads, int head_dim, float p_drop, uint64_t seed, float* dqkv, void* stream);
+
+/* The dropout mask of one training-attention call.  Both kinds are counter-based Philox4x32-10 with key
+ * (seed & 0xffffffff, seed >> 32), regenerated by the forward and both backward kernels, never stored.
+ *   IEFVAD_DROPOUT_PHILOX: the library's own mask (above); p in [0, 1); offset and threads are ignored.
+ *   IEFVAD_DROPOUT_TORCH:  PyTorch's mask, bit for bit: what torch.native_dropout (which F.multi_head_attention_forward
+ *     applies to the [B*heads, T, T] weights in train() mode with need_weights) draws on a CUDA generator whose state is
+ *     (seed, offset).  Element e = ((b * heads + h) * T + query) * T + key lies in group v = e / 4, drawn by thread
+ *     v % threads in its iteration v / threads: counter (lo64 = offset / 4 + v / threads, hi64 = v % threads), word e % 4;
+ *     kept when float(word) * 2^-32 + 2^-33 < float(1 - p), kept weights scaled by float(1 / double(float(1 - p))).
+ *     threads = G = grid * 256 of torch's launch, grid = min(SMs * (max threads per SM / 256), ceil(n / 256)) for
+ *     n = B * heads * T * T - so the mask depends on the GPU's SM count.  p in (0, 1), offset % 4 == 0, 0 < threads
+ *     < 2^31, n % 4 == 0 (torch draws other sizes with a narrower vector width, which is not reproduced).  One call
+ *     advances torch's generator by ((n - 1) / (threads * 4) + 1) * 4; the caller does that (restated in
+ *     oracle/torch_dropout.py). */
+#define IEFVAD_DROPOUT_PHILOX 0
+#define IEFVAD_DROPOUT_TORCH 1
+typedef struct iefvad_dropout {
+  int32_t kind;
+  double p;                  /* drop probability */
+  uint64_t seed;
+  uint64_t offset;
+  int64_t threads;
+} iefvad_dropout;
+/* iefvad_attention_train_fwd / _bwd with the mask given by `drop` (arguments checked before the device is touched) */
+int iefvad_attention_train_fwd_dropout(const float* qkv, int64_t B, int64_t T, int heads, int head_dim,
+                                       const iefvad_dropout* drop, float* out, float* lse, void* stream);
+int iefvad_attention_train_bwd_dropout(const float* qkv, const float* out, const float* dout, const float* lse, int64_t B,
+                                       int64_t T, int heads, int head_dim, const iefvad_dropout* drop, float* dqkv,
+                                       void* stream);
+/* mask [B*heads, T, T] uint8 (1 = kept): the keep decisions of the kernels above under `drop`, in the layout of
+ * torch.native_dropout's mask (parity-test surface) */
+int iefvad_dropout_mask(const iefvad_dropout* drop, int64_t B, int heads, int64_t T, uint8_t* mask, void* stream);
 /* nn.LayerNorm backward: x [rows, dim] = the layer's input, dy = gradient of its output -> dx, dweight [dim], dbias [dim] */
 int iefvad_layernorm_bwd(const float* x, const float* weight, const float* dy, int64_t rows, int dim, float eps, float* dx,
                          float* dweight, float* dbias, void* stream);
