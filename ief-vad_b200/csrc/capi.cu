@@ -689,10 +689,17 @@ int iefvad_profile_enable(int on) {
 
 // ------------------------------------------------------------------------------------------------ training step (N3)
 
+// the checks every training-attention entry point makes before it touches the device; `tensors`: none of its pointers is null
+static int check_train_attn(const char* fn, bool tensors, int64_t B, int64_t T, int heads, int head_dim) {
+  IEF_CHECK(tensors, "%s: null argument", fn);
+  IEF_CHECK(B >= 0 && B < 65536 && T >= 0 && T < (1 << 24) && heads > 0, "%s: bad B / T / heads", fn);
+  IEF_CHECK(attn_train_supported(head_dim), "%s: head dim %d unsupported (32, 64, 96, 128)", fn, head_dim);
+  return IEFVAD_OK;
+}
+
 int iefvad_attention_train_fwd(const float* qkv, int64_t B, int64_t T, int heads, int head_dim, float p_drop, uint64_t seed,
                                float* out, float* lse, void* stream) {
-  IEF_CHECK(qkv && out && lse, "iefvad_attention_train_fwd: null argument");
-  IEF_CHECK(B >= 0 && B < 65536 && T >= 0 && T < (1 << 24), "iefvad_attention_train_fwd: bad B / T");
+  IEF_TRY(check_train_attn("iefvad_attention_train_fwd", qkv && out && lse, B, T, heads, head_dim));
   IEF_CHECK(p_drop >= 0.f && p_drop < 1.f, "attention dropout probability %f outside [0, 1)", p_drop);
   return attn_train_fwd(qkv, int(B), int(T), heads, head_dim, dropout_philox(p_drop, seed, int(T)), out, lse,
                         static_cast<cudaStream_t>(stream));
@@ -711,8 +718,7 @@ static int attn_train_bwd_run(const float* qkv, const float* out, const float* d
 
 int iefvad_attention_train_bwd(const float* qkv, const float* out, const float* dout, const float* lse, int64_t B, int64_t T,
                                int heads, int head_dim, float p_drop, uint64_t seed, float* dqkv, void* stream) {
-  IEF_CHECK(qkv && out && dout && lse && dqkv, "iefvad_attention_train_bwd: null argument");
-  IEF_CHECK(B >= 0 && B < 65536 && T >= 0 && T < (1 << 24), "iefvad_attention_train_bwd: bad B / T");
+  IEF_TRY(check_train_attn("iefvad_attention_train_bwd", qkv && out && dout && lse && dqkv, B, T, heads, head_dim));
   IEF_CHECK(p_drop >= 0.f && p_drop < 1.f, "attention dropout probability %f outside [0, 1)", p_drop);
   return attn_train_bwd_run(qkv, out, dout, lse, B, T, heads, head_dim, dropout_philox(p_drop, seed, int(T)), dqkv, stream);
 }
@@ -741,8 +747,7 @@ static int dropout_desc(const char* fn, const iefvad_dropout* d, int64_t B, int6
 
 int iefvad_attention_train_fwd_dropout(const float* qkv, int64_t B, int64_t T, int heads, int head_dim,
                                        const iefvad_dropout* drop, float* out, float* lse, void* stream) {
-  IEF_CHECK(qkv && out && lse, "iefvad_attention_train_fwd_dropout: null argument");
-  IEF_CHECK(B >= 0 && B < 65536 && T >= 0 && T < (1 << 24) && heads > 0, "iefvad_attention_train_fwd_dropout: bad B / T / heads");
+  IEF_TRY(check_train_attn("iefvad_attention_train_fwd_dropout", qkv && out && lse, B, T, heads, head_dim));
   DropoutDesc d;
   IEF_TRY(dropout_desc("iefvad_attention_train_fwd_dropout", drop, B, heads, T, &d));
   return attn_train_fwd(qkv, int(B), int(T), heads, head_dim, d, out, lse, static_cast<cudaStream_t>(stream));
@@ -751,8 +756,7 @@ int iefvad_attention_train_fwd_dropout(const float* qkv, int64_t B, int64_t T, i
 int iefvad_attention_train_bwd_dropout(const float* qkv, const float* out, const float* dout, const float* lse, int64_t B,
                                        int64_t T, int heads, int head_dim, const iefvad_dropout* drop, float* dqkv,
                                        void* stream) {
-  IEF_CHECK(qkv && out && dout && lse && dqkv, "iefvad_attention_train_bwd_dropout: null argument");
-  IEF_CHECK(B >= 0 && B < 65536 && T >= 0 && T < (1 << 24) && heads > 0, "iefvad_attention_train_bwd_dropout: bad B / T / heads");
+  IEF_TRY(check_train_attn("iefvad_attention_train_bwd_dropout", qkv && out && dout && lse && dqkv, B, T, heads, head_dim));
   DropoutDesc d;
   IEF_TRY(dropout_desc("iefvad_attention_train_bwd_dropout", drop, B, heads, T, &d));
   return attn_train_bwd_run(qkv, out, dout, lse, B, T, heads, head_dim, d, dqkv, stream);

@@ -1,18 +1,16 @@
 // Kernels of the TRAINING step (SURVEY 8f row N3; reference: train/ucf_train.py:60-106 calls loss.backward() through
 // model/imf_vad.py:109-161 and train/loss.py:18-30): what the backward pass needs besides the GEMMs, which reuse the
 // tcgen05 kernel of the forward (dgrad = dY . W with W^T as the K-major "weight", wgrad = dY^T . X on transposed
-// activations).  Everything here is fp32 IEEE arithmetic; reductions over rows are two-stage and fixed-order, so the
-// gradients are run-to-run deterministic.
+// activations) and the attention, which has its own file (train_attn.cu).  Everything here is fp32 IEEE arithmetic;
+// reductions over rows are two-stage and fixed-order, so the gradients are run-to-run deterministic.
 //
-//   attn_train_fwd / attn_train_bwd_{q,kv}  softmax(q k^T / sqrt(d)) v per (batch element, head) with the attention
-//                                           dropout of nn.MultiheadAttention (train mode, model/imf_vad.py:53,70) from a
-//                                           counter-based Philox4x32-10 mask: the library's own or PyTorch's (philox.cuh)
 //   layernorm_bwd                           dx, dgamma, dbeta of nn.LayerNorm
+//   colsum                                  column sums (bias gradients), optionally row-weighted
 //   fuse_bwd                                backward of the uncertainty-weighted fusion (model/imf_vad.py:130-144)
+//   relu_bwd, quickgelu, axpy, outer        small elementwise helpers
+//   transpose_f32, transpose_split          transposes for the wgrad GEMMs (fp32, or straight into bf16 hi / lo operands)
 //   clas2_bwd                               backward of the MIL top-k BCE loss (train/loss.py:18-30)
-//   transpose, colsum, relu_bwd, axpy, outer
 #include "common.cuh"
-#include "philox.cuh"
 #include "train.cuh"
 
 namespace iefvad {
@@ -27,268 +25,6 @@ __host__ int grid_for(long long work_items, int num_sms, int per_sm = 8) {
   if (blocks > cap) blocks = cap;
   if (blocks < 1) blocks = 1;
   return static_cast<int>(blocks);
-}
-
-// ---------------------------------------------------------------- attention, training form (fp32, one warp per 4 rows)
-constexpr int SROWS = 16;
-
-// qkv [B*T, 3D] fp32 (bias added, q unscaled) -> out [B*T, D], lse [B, H, T] = log sum_j exp(s_ij)
-template <int DH>
-__global__ void __launch_bounds__(128)
-attn_train_fwd_kernel(const float* __restrict__ qkv, float* __restrict__ out, float* __restrict__ lse, int T, int H, int D,
-                      float qscale, DropoutDesc drop) {
-  constexpr int NPL = DH / 32;
-  __shared__ float Ks[32][DH + 1];
-  __shared__ float Vs[32][DH];
-  __shared__ float Qs[SROWS][DH];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int h = blockIdx.y, b = blockIdx.z;
-  const int bh = b * H + h;
-  const int q0 = blockIdx.x * SROWS;
-  const long long base = (long long)b * T;
-  for (int i = threadIdx.x; i < SROWS * DH; i += 128) {
-    const int rr = i / DH, d = i - rr * DH;
-    const int t = q0 + rr;
-    Qs[rr][d] = (t < T) ? qkv[(base + t) * 3 * D + h * DH + d] * qscale : 0.f;
-  }
-  float m[4], l[4], o[4][NPL];
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    m[i] = -INFINITY;
-    l[i] = 0.f;
-#pragma unroll
-    for (int e = 0; e < NPL; ++e) o[i][e] = 0.f;
-  }
-  for (int k0 = 0; k0 < T; k0 += 32) {
-    __syncthreads();
-    for (int i = threadIdx.x; i < 32 * DH; i += 128) {
-      const int kr = i / DH, d = i - kr * DH;
-      const int t = k0 + kr;
-      Ks[kr][d] = (t < T) ? qkv[(base + t) * 3 * D + D + h * DH + d] : 0.f;
-      Vs[kr][d] = (t < T) ? qkv[(base + t) * 3 * D + 2 * D + h * DH + d] : 0.f;
-    }
-    __syncthreads();
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int rr = warp * 4 + i;
-      const int tq = q0 + rr;
-      float s = 0.f;
-#pragma unroll 8
-      for (int d = 0; d < DH; ++d) s = fmaf(Qs[rr][d], Ks[lane][d], s);
-      const int key = k0 + lane;
-      if (key >= T) s = -INFINITY;
-      const float mx = fmaxf(m[i], warp_max(s));
-      const float alpha = expf(m[i] - mx);
-      const float p = expf(s - mx);
-      l[i] = l[i] * alpha + warp_sum(p);         // the softmax denominator sums ALL keys; dropout acts on the weights
-      m[i] = mx;
-      float pd = p;
-      if (drop.kind && key < T && tq < T) pd *= keep_scale(drop, bh, tq, key);
-#pragma unroll
-      for (int e = 0; e < NPL; ++e) o[i][e] *= alpha;
-      for (int jj = 0; jj < 32; ++jj) {
-        const float pj = __shfl_sync(0xffffffffu, pd, jj);
-#pragma unroll
-        for (int e = 0; e < NPL; ++e) o[i][e] = fmaf(pj, Vs[jj][lane + 32 * e], o[i][e]);
-      }
-    }
-  }
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int tq = q0 + warp * 4 + i;
-    if (tq >= T) continue;
-    const float inv = 1.f / l[i];
-#pragma unroll
-    for (int e = 0; e < NPL; ++e) out[(base + tq) * D + h * DH + lane + 32 * e] = o[i][e] * inv;
-    if (lane == 0) lse[(long long)bh * T + tq] = m[i] + logf(l[i]);
-  }
-}
-
-// delta[bh, t] = sum_d dout[t, h, d] * out[t, h, d]
-__global__ void __launch_bounds__(kThreads)
-attn_delta_kernel(const float* __restrict__ out, const float* __restrict__ dout, float* __restrict__ delta, int B, int T, int H,
-                  int dh) {
-  const int lane = threadIdx.x & 31;
-  const long long warps = ((long long)gridDim.x * blockDim.x) >> 5;
-  const long long total = (long long)B * H * T;
-  const int D = H * dh;
-  for (long long w = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5; w < total; w += warps) {
-    const long long bh = w / T;
-    const int t = int(w - bh * T);
-    const long long b = bh / H;
-    const int h = int(bh - b * H);
-    const long long off = (b * T + t) * D + h * dh;
-    float s = 0.f;
-    for (int d = lane; d < dh; d += 32) s = fmaf(out[off + d], dout[off + d], s);
-    s = warp_sum(s);
-    if (lane == 0) delta[w] = s;
-  }
-}
-
-// dq: one warp per 4 query rows, keys streamed in blocks of 32 (mirror of the forward)
-template <int DH>
-__global__ void __launch_bounds__(128)
-attn_train_bwd_q_kernel(const float* __restrict__ qkv, const float* __restrict__ dout, const float* __restrict__ lse,
-                        const float* __restrict__ delta, float* __restrict__ dqkv, int T, int H, int D, float qscale,
-                        DropoutDesc drop) {
-  constexpr int NPL = DH / 32;
-  __shared__ float Ks[32][DH + 1];
-  __shared__ float Vs[32][DH + 1];
-  __shared__ float Qs[SROWS][DH];
-  __shared__ float Gs[SROWS][DH];      // dout rows
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int h = blockIdx.y, b = blockIdx.z;
-  const int bh = b * H + h;
-  const int q0 = blockIdx.x * SROWS;
-  const long long base = (long long)b * T;
-  for (int i = threadIdx.x; i < SROWS * DH; i += 128) {
-    const int rr = i / DH, d = i - rr * DH;
-    const int t = q0 + rr;
-    Qs[rr][d] = (t < T) ? qkv[(base + t) * 3 * D + h * DH + d] * qscale : 0.f;
-    Gs[rr][d] = (t < T) ? dout[(base + t) * D + h * DH + d] : 0.f;
-  }
-  float dq[4][NPL], L[4], Dl[4];
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int tq = q0 + warp * 4 + i;
-    L[i] = (tq < T) ? lse[(long long)bh * T + tq] : 0.f;
-    Dl[i] = (tq < T) ? delta[(long long)bh * T + tq] : 0.f;
-#pragma unroll
-    for (int e = 0; e < NPL; ++e) dq[i][e] = 0.f;
-  }
-  for (int k0 = 0; k0 < T; k0 += 32) {
-    __syncthreads();
-    for (int i = threadIdx.x; i < 32 * DH; i += 128) {
-      const int kr = i / DH, d = i - kr * DH;
-      const int t = k0 + kr;
-      Ks[kr][d] = (t < T) ? qkv[(base + t) * 3 * D + D + h * DH + d] : 0.f;
-      Vs[kr][d] = (t < T) ? qkv[(base + t) * 3 * D + 2 * D + h * DH + d] : 0.f;
-    }
-    __syncthreads();
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int rr = warp * 4 + i;
-      const int tq = q0 + rr;
-      const int key = k0 + lane;
-      float s = 0.f, dpd = 0.f;
-#pragma unroll 8
-      for (int d = 0; d < DH; ++d) {
-        s = fmaf(Qs[rr][d], Ks[lane][d], s);
-        dpd = fmaf(Gs[rr][d], Vs[lane][d], dpd);
-      }
-      float ds = 0.f;
-      if (key < T && tq < T) {
-        const float p = expf(s - L[i]);
-        const float ks = drop.kind ? keep_scale(drop, bh, tq, key) : 1.f;
-        ds = p * (dpd * ks - Dl[i]);
-      }
-      for (int jj = 0; jj < 32; ++jj) {
-        const float dj = __shfl_sync(0xffffffffu, ds, jj);
-#pragma unroll
-        for (int e = 0; e < NPL; ++e) dq[i][e] = fmaf(dj, Ks[jj][lane + 32 * e], dq[i][e]);
-      }
-    }
-  }
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int tq = q0 + warp * 4 + i;
-    if (tq >= T) continue;
-#pragma unroll
-    for (int e = 0; e < NPL; ++e) dqkv[(base + tq) * 3 * D + h * DH + lane + 32 * e] = dq[i][e] * qscale;
-  }
-}
-
-// dk, dv: one warp per 4 key rows, queries streamed in blocks of 32
-template <int DH>
-__global__ void __launch_bounds__(128)
-attn_train_bwd_kv_kernel(const float* __restrict__ qkv, const float* __restrict__ dout, const float* __restrict__ lse,
-                         const float* __restrict__ delta, float* __restrict__ dqkv, int T, int H, int D, float qscale,
-                         DropoutDesc drop) {
-  constexpr int NPL = DH / 32;
-  __shared__ float Qs[32][DH + 1];     // scaled queries of the block
-  __shared__ float Gs[32][DH + 1];     // dout rows of the block
-  __shared__ float Ls[32], Ds[32];
-  __shared__ float Ks[SROWS][DH];
-  __shared__ float Vs[SROWS][DH];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int h = blockIdx.y, b = blockIdx.z;
-  const int bh = b * H + h;
-  const int k0 = blockIdx.x * SROWS;
-  const long long base = (long long)b * T;
-  for (int i = threadIdx.x; i < SROWS * DH; i += 128) {
-    const int rr = i / DH, d = i - rr * DH;
-    const int t = k0 + rr;
-    Ks[rr][d] = (t < T) ? qkv[(base + t) * 3 * D + D + h * DH + d] : 0.f;
-    Vs[rr][d] = (t < T) ? qkv[(base + t) * 3 * D + 2 * D + h * DH + d] : 0.f;
-  }
-  float dk[4][NPL], dv[4][NPL];
-#pragma unroll
-  for (int i = 0; i < 4; ++i)
-#pragma unroll
-    for (int e = 0; e < NPL; ++e) dk[i][e] = dv[i][e] = 0.f;
-  for (int q0 = 0; q0 < T; q0 += 32) {
-    __syncthreads();
-    for (int i = threadIdx.x; i < 32 * DH; i += 128) {
-      const int qr = i / DH, d = i - qr * DH;
-      const int t = q0 + qr;
-      Qs[qr][d] = (t < T) ? qkv[(base + t) * 3 * D + h * DH + d] * qscale : 0.f;
-      Gs[qr][d] = (t < T) ? dout[(base + t) * D + h * DH + d] : 0.f;
-    }
-    if (threadIdx.x < 32) {
-      const int t = q0 + threadIdx.x;
-      Ls[threadIdx.x] = (t < T) ? lse[(long long)bh * T + t] : 0.f;
-      Ds[threadIdx.x] = (t < T) ? delta[(long long)bh * T + t] : 0.f;
-    }
-    __syncthreads();
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int rr = warp * 4 + i;
-      const int key = k0 + rr;
-      const int tq = q0 + lane;         // this lane's query
-      float s = 0.f, dpd = 0.f;
-#pragma unroll 8
-      for (int d = 0; d < DH; ++d) {
-        s = fmaf(Qs[lane][d], Ks[rr][d], s);
-        dpd = fmaf(Gs[lane][d], Vs[rr][d], dpd);
-      }
-      float pd = 0.f, ds = 0.f;
-      if (key < T && tq < T) {
-        const float p = expf(s - Ls[lane]);
-        const float ks = drop.kind ? keep_scale(drop, bh, tq, key) : 1.f;
-        pd = p * ks;
-        ds = p * (dpd * ks - Ds[lane]);
-      }
-      for (int jj = 0; jj < 32; ++jj) {
-        const float pj = __shfl_sync(0xffffffffu, pd, jj);
-        const float dj = __shfl_sync(0xffffffffu, ds, jj);
-#pragma unroll
-        for (int e = 0; e < NPL; ++e) {
-          dv[i][e] = fmaf(pj, Gs[jj][lane + 32 * e], dv[i][e]);
-          dk[i][e] = fmaf(dj, Qs[jj][lane + 32 * e], dk[i][e]);      // Qs holds q * scale: d s / d k = scale * q
-        }
-      }
-    }
-  }
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int key = k0 + warp * 4 + i;
-    if (key >= T) continue;
-#pragma unroll
-    for (int e = 0; e < NPL; ++e) {
-      dqkv[(base + key) * 3 * D + D + h * DH + lane + 32 * e] = dk[i][e];
-      dqkv[(base + key) * 3 * D + 2 * D + h * DH + lane + 32 * e] = dv[i][e];
-    }
-  }
-}
-
-// mask[bh, i, j] = 1 when the attention kernels keep weight (bh, query i, key j) under `drop` (the parity-test surface)
-__global__ void __launch_bounds__(kThreads)
-dropout_mask_kernel(DropoutDesc drop, long long n, uint8_t* __restrict__ mask) {
-  const long long T = drop.T;
-  for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x) {
-    const long long row = e / T;
-    mask[e] = keep_scale(drop, int(row / T), int(row % T), int(e % T)) != 0.f;
-  }
 }
 
 // ---------------------------------------------------------------- LayerNorm backward
@@ -486,64 +222,6 @@ clas2_bwd_kernel(const float* __restrict__ logits, const float* __restrict__ mea
 }  // namespace
 
 // ================================================================ host wrappers
-int attn_train_fwd(const float* qkv, int B, int T, int H, int dh, DropoutDesc drop, float* out, float* lse,
-                   cudaStream_t stream) {
-  const int D = H * dh;
-  const dim3 grid((T + SROWS - 1) / SROWS, H, B);
-  const float qs = 1.0f / sqrtf(float(dh));
-  drop.T = T;
-  if (B == 0 || T == 0) return IEFVAD_OK;
-  if (attn_train_mma_supported(dh)) return attn_train_fwd_mma(qkv, B, T, H, dh, qs, drop, out, lse, stream);
-  switch (dh) {
-    case 32: attn_train_fwd_kernel<32><<<grid, 128, 0, stream>>>(qkv, out, lse, T, H, D, qs, drop); break;
-    case 64: attn_train_fwd_kernel<64><<<grid, 128, 0, stream>>>(qkv, out, lse, T, H, D, qs, drop); break;
-    case 96: attn_train_fwd_kernel<96><<<grid, 128, 0, stream>>>(qkv, out, lse, T, H, D, qs, drop); break;
-    default: set_error("attn_train: head dim %d unsupported (32, 64, 96)", dh); return IEFVAD_ERR_INVALID;
-  }
-  count_launches(1);
-  IEF_CUDA(cudaGetLastError());
-  return IEFVAD_OK;
-}
-
-int attn_train_bwd(const float* qkv, const float* out, const float* dout, const float* lse, int B, int T, int H, int dh,
-                   DropoutDesc drop, float* delta_scratch, float* dqkv, int num_sms, cudaStream_t stream) {
-  if (B == 0 || T == 0) return IEFVAD_OK;
-  const int D = H * dh;
-  const dim3 grid((T + SROWS - 1) / SROWS, H, B);
-  const float qs = 1.0f / sqrtf(float(dh));
-  drop.T = T;
-  attn_delta_kernel<<<grid_for((long long)B * H * T * 32, num_sms), kThreads, 0, stream>>>(out, dout, delta_scratch, B, T, H, dh);
-  if (attn_train_mma_supported(dh)) {
-    count_launches(1);
-    return attn_train_bwd_mma(qkv, dout, lse, delta_scratch, B, T, H, dh, qs, drop, dqkv, stream);
-  }
-#define IEF_BWD(DH_)                                                                                                          \
-  attn_train_bwd_q_kernel<DH_><<<grid, 128, 0, stream>>>(qkv, dout, lse, delta_scratch, dqkv, T, H, D, qs, drop);              \
-  attn_train_bwd_kv_kernel<DH_><<<grid, 128, 0, stream>>>(qkv, dout, lse, delta_scratch, dqkv, T, H, D, qs, drop);
-  switch (dh) {
-    case 32: IEF_BWD(32) break;
-    case 64: IEF_BWD(64) break;
-    case 96: IEF_BWD(96) break;
-    default: set_error("attn_train: head dim %d unsupported (32, 64, 96)", dh); return IEFVAD_ERR_INVALID;
-  }
-#undef IEF_BWD
-  count_launches(3);
-  IEF_CUDA(cudaGetLastError());
-  return IEFVAD_OK;
-}
-
-int dropout_mask(DropoutDesc drop, int B, int H, int T, uint8_t* mask, cudaStream_t stream) {
-  const long long n = (long long)B * H * T * T;
-  if (n == 0) return IEFVAD_OK;
-  int sms = 0;
-  IEF_TRY(device_sms(&sms));
-  drop.T = T;
-  dropout_mask_kernel<<<grid_for(n, sms), kThreads, 0, stream>>>(drop, n, mask);
-  count_launches(1);
-  IEF_CUDA(cudaGetLastError());
-  return IEFVAD_OK;
-}
-
 static int colsum_run(const float* a, const float* b, const float2* stats, const float* wgt, long long rows, int D, int mode,
                       float* part, float* out0, float* out1, int num_sms, cudaStream_t stream) {
   const int nblk = train_colsum_blocks(rows, num_sms);

@@ -1,10 +1,12 @@
-// Internal interface of the training-step kernels (train.cu): SURVEY 8f row N3.
+// Internal interface of the training-step kernels (train.cu, train_attn.cu, train_loss.cu): SURVEY 8f row N3.
 #pragma once
 #include "common.cuh"
 #include "philox.cuh"
 
 namespace iefvad {
 
+// Training attention (train_attn.cu).  The head sizes the kernels are built for: 32, 64, 96 and 128.
+bool attn_train_supported(int dh);
 // softmax(q k^T / sqrt(dh)) v with attention dropout of mode `drop` (philox.cuh: dropout_philox / dropout_torch; its T is
 // set here).  qkv [B*T, 3*H*dh] fp32 (bias added, q unscaled) -> out [B*T, H*dh], lse [B, H, T]
 int attn_train_fwd(const float* qkv, int B, int T, int H, int dh, DropoutDesc drop, float* out, float* lse, cudaStream_t stream);
@@ -13,13 +15,6 @@ int attn_train_bwd(const float* qkv, const float* out, const float* dout, const 
                    DropoutDesc drop, float* delta_scratch, float* dqkv, int num_sms, cudaStream_t stream);
 // mask [B*H, T, T] uint8 (1 = kept) of mode `drop`: the keep decisions the attention kernels make, in torch's layout
 int dropout_mask(DropoutDesc drop, int B, int H, int T, uint8_t* mask, cudaStream_t stream);
-
-// the same on the tensor cores (mma.sync TF32, train_attn_mma.cu); qs = 1 / sqrt(dh)
-bool attn_train_mma_supported(int dh);
-int attn_train_fwd_mma(const float* qkv, int B, int T, int H, int dh, float qs, const DropoutDesc& drop,
-                       float* out, float* lse, cudaStream_t stream);
-int attn_train_bwd_mma(const float* qkv, const float* dout, const float* lse, const float* delta, int B, int T, int H, int dh,
-                       float qs, const DropoutDesc& drop, float* dqkv, cudaStream_t stream);
 
 int train_colsum_blocks(long long rows, int num_sms);
 // scratch: 2 * rows + 2 * train_colsum_blocks(rows) * D floats

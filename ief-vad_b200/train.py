@@ -8,9 +8,10 @@ the 78 parameters and, when the image / event features require grad, of those in
 modality's first attention layer; fp32, cast by autograd to the input's dtype).  `ForwardFn` is that autograd node.
 Its forward is the model composed from the library's stand-alone operators (tcgen05 GEMMs with the 3-term bf16 split -
 gradients need fp32's exponent range, fp16 operands would flush them - the 3xTF32 tensor-core training attention of
-csrc/train_attn_mma.cu, fp32 LayerNorm / fusion kernels) keeping what the backward needs; its backward runs entirely in
-libiefvad.so kernels too: dgrad = linear(dY, W^T), wgrad = linear(dY^T, X^T) on the same tcgen05 GEMM, attention /
-LayerNorm / fusion / ReLU backward kernels of csrc/train.cu.  torch only owns the buffers and the autograd graph.
+csrc/train_attn.cu, fp32 LayerNorm / fusion kernels) keeping what the backward needs; its backward runs entirely in
+libiefvad.so kernels too: dgrad = linear(dY, W^T), wgrad = linear(dY^T, X^T) on the same tcgen05 GEMM, the attention
+backward of csrc/train_attn.cu and the LayerNorm / fusion / ReLU backward kernels of csrc/train.cu.  torch only owns the
+buffers and the autograd graph.
 
 Attention dropout (p = 0.1, active in train() mode like nn.MultiheadAttention): a counter-based Philox4x32-10 mask,
 regenerated, not stored, by the backward (include/iefvad.h: iefvad_dropout).  With `dropout_rng = "philox"` (the default)

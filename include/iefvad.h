@@ -350,7 +350,8 @@ int iefvad_bench_gemm(int64_t M, int N, int K, int nsplit, int tile_n, int stage
 /* nn.MultiheadAttention's core in TRAIN mode (model/imf_vad.py:53,70: dropout 0.1 on the attention weights,
  * torch/nn/functional.py:6643-6647): out = dropout(softmax(q k^T / sqrt(head_dim))) v per (batch element, head).
  * qkv [B*T, 3*heads*head_dim] (in-projection output, bias added, q unscaled); out [B*T, heads*head_dim]; lse [B, heads, T]
- * = log-sum-exp of the scores (saved for the backward).  These two entry points use the library's own dropout mask
+ * = log-sum-exp of the scores (saved for the backward).  head_dim 32, 64, 96 or 128; every argument is checked before
+ * the device is touched.  These two entry points use the library's own dropout mask
  * (IEFVAD_DROPOUT_PHILOX below), a pure function of (seed, head, query, key): Philox4x32-10 with key =
  * (seed & 0xffffffff, seed >> 32) and counter = (key >> 2, query, b * heads + h, 0), word (key & 3), dropped when the word
  * < uint32(double(p_drop) * 2^32), kept weights scaled by 1.f / (1.f - p_drop) (restated in oracle/iefvad_oracle.py:

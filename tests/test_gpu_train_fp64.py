@@ -1,17 +1,17 @@
 """Row N3 - the training step against float64 references built here, at shapes and configurations the reference goldens
 of tests/test_gpu_train.py do not reach.
 
-- Training attention (csrc/train_attn_mma.cu; the FFMA kernels of csrc/train.cu under IEFVAD_TRAIN_ATTN=simt): out, lse,
-  dq, dk, dv against float64 autograd of (softmax(q k^T / sqrt(dh)) * keep) v, with `keep` the documented Philox mask
-  (oracle.iefvad_oracle.attention_keep), so train-mode gradients are checked exactly, not statistically.
+- Training attention (csrc/train_attn.cu): out, lse, dq, dk, dv against float64 autograd of
+  (softmax(q k^T / sqrt(dh)) * keep) v, with `keep` the documented Philox mask (oracle.iefvad_oracle.attention_keep), so
+  train-mode gradients are checked exactly, not statistically.
 - The whole step (train.ForwardFn + train.Clas2Fn) against float64 autograd of oracle/torch_port.py with the same
   per-layer masks: loss, the 8 outputs, every parameter gradient and the gradients of the image / event features.
 - The elementwise backward operators (fuse_bwd, layernorm_bwd, colsum, clas2_bwd) at their edges.
 
 Errors are max |got - ref| / max |ref| per tensor.  Worst measured on an NVIDIA B200 (1000 W power limit):
     attention, mma.sync 3xTF32 (bound 2e-5)   dh 32: 4.3e-6   dh 64: 4.1e-6   dh 96: 4.8e-6   dh 128: 6.7e-6
-    attention, SIMT FFMA (bound 2e-5)         1.2e-6;  a wrong mask (words permuted, query / key swapped, seed's high
-                                              word lost) leaves 0.55 - 0.86 on out, dq, dk and dv
+    attention, a wrong mask                   0.55 - 0.86 on out, dq, dk and dv (words permuted, query / key swapped,
+                                              seed's high word lost)
     whole step, D = 128 (bound 1e-3)          H 4: 2.9e-5   H 2: 2.2e-5   H 1: 2.3e-5 (eval and train alike); fp16 inputs
                                               2.8e-4 (their gradient is rounded to fp16)
     whole step, D = 768, train mode           90 % quantile 4.6e-4, worst entry 0.10 (one ReLU gate flip, see the test)
@@ -19,9 +19,6 @@ Errors are max |got - ref| / max |ref| per tensor.  Worst measured on an NVIDIA 
     clas2_bwd 4.3e-7 (bound 1e-5).
 The whole file runs in about 15 s.  Needs a B200."""
 import math
-import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
@@ -34,7 +31,6 @@ from test_gpu_train import reference_loss
 
 pytestmark = pytest.mark.gpu
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SEEDS = (0, (0x00000007 << 32) | 0xDEADBEEF, 2 ** 62 - 77)      # low word only; distinct high / low words; near 2^62
 
 
@@ -142,64 +138,6 @@ def test_train_attention_distinguishes_the_documented_mask_from_wrong_ones(pkg):
         errs = attention_errors(got, attention_ref(qkv, dout, B, T, H, bad), T)
         print(f"wrong mask ({name}):", {k: f"{v:.2e}" for k, v in errs.items()})
         assert errs["out"] > 1e-2 and errs["dv"] > 1e-2, (name, errs)       # >= 500x the bound
-
-
-_SIMT_SCRIPT = r"""
-import sys
-import numpy as np
-import torch
-sys.path.insert(0, sys.argv[1])
-from iefvad_b200 import ops
-z = np.load(sys.argv[2])
-res = {}
-for name in z.files:
-    if not name.startswith("qkv:"):
-        continue
-    case = name[4:]
-    B, T, H, _, pm, seed = (int(v) for v in case.split("_"))
-    qkv, dout = torch.from_numpy(z["qkv:" + case]).cuda(), torch.from_numpy(z["dout:" + case]).cuda()
-    out, lse = ops.attention_train_fwd(qkv, B, T, H, pm / 1000, seed)
-    dqkv = ops.attention_train_bwd(qkv, out, dout, lse, B, T, H, pm / 1000, seed)
-    res["out:" + case], res["lse:" + case], res["dqkv:" + case] = out.cpu().numpy(), lse.cpu().numpy(), dqkv.cpu().numpy()
-try:                                  # head dim 128 exists only on the mma.sync path: refused here proves the SIMT path ran
-    ops.attention_train_fwd(torch.zeros(4, 3 * 128, device="cuda"), 1, 4, 1)
-    res["dh128_refused"] = np.array(0)
-except RuntimeError:
-    res["dh128_refused"] = np.array(1)
-np.savez(sys.argv[3], **res)
-"""
-
-
-def test_simt_train_attention_matches_float64_with_the_exact_mask(pkg, tmp_path):
-    """The FFMA kernels of csrc/train.cu, selected by IEFVAD_TRAIN_ATTN=simt (read once per process, hence a child
-    process with a timeout)."""
-    B, H, seed = 2, 3, SEEDS[1]
-    cases, data = [], {}
-    for dh in (32, 64, 96):
-        for T in (1, 33, 129):
-            for p in (0.0, 0.1):
-                qkv, dout = attention_inputs(B, T, H, dh, 31 * dh + T)
-                case = f"{B}_{T}_{H}_{dh}_{int(round(p * 1000))}_{seed}"
-                data[f"qkv:{case}"], data[f"dout:{case}"] = qkv.numpy(), dout.numpy()
-                cases.append((dh, T, p, qkv, dout, case))
-    np.savez(tmp_path / "in.npz", **data)
-    env = dict(os.environ, IEFVAD_TRAIN_ATTN="simt")
-    cmd = [sys.executable] + (["-s"] if sys.flags.no_user_site else []) + [
-        "-c", _SIMT_SCRIPT, ROOT, str(tmp_path / "in.npz"), str(tmp_path / "out.npz")]
-    r = subprocess.run(cmd, env=env, cwd=ROOT, capture_output=True, text=True, timeout=300)
-    assert r.returncode == 0, r.stderr[-4000:]
-    z = np.load(tmp_path / "out.npz")
-    assert int(z["dh128_refused"]) == 1
-    worst = 0.0
-    for dh, T, p, qkv, dout, case in cases:
-        D = H * dh
-        keep = O.attention_keep(seed, B, H, T, p) if p > 0 else None
-        d = torch.from_numpy(z["dqkv:" + case])
-        got = (torch.from_numpy(z["out:" + case]), torch.from_numpy(z["lse:" + case]), d[:, :D], d[:, D:2 * D], d[:, 2 * D:])
-        errs = attention_errors(got, attention_ref(qkv, dout, B, T, H, keep), T)
-        worst = max(worst, max(errs.values()))
-        assert max(errs.values()) <= 2e-5, (dh, T, p, errs)
-    print("SIMT attention worst error:", worst)
 
 
 # ------------------------------------------------------------------------------------------------ the whole training step

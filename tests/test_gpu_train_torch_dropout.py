@@ -3,16 +3,13 @@ mask, regenerated inside the kernels, and the generator stream of the reference'
 
 - iefvad_dropout_mask equals torch.native_dropout's mask bit for bit, and the generator offset after each call is torch's;
   an offset one step off, a launch width G +- 256 or swapped counter halves each give a different mask.
-- The tensor-core and SIMT training attention in torch mode against float64 autograd with torch's own mask.
+- The training attention in torch mode against float64 autograd with torch's own mask.
 - The drop-in in train() mode against a stock-torch composition (real nn.MultiheadAttention modules, need_weights at its
   default, oracle/torch_port.py for the rest) under the same torch.cuda.manual_seed: outputs, loss, every gradient, the
   CUDA generator's offset afterwards, an untouched CPU generator, and two AdamW steps.
 - The default "philox" mode is unchanged: its outputs and gradients hash to what the previous release produced.
 Worst errors measured on an NVIDIA B200 (1000 W power limit) are quoted at each bound.  Needs a B200."""
 import hashlib
-import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
@@ -24,8 +21,6 @@ from test_gpu_train import reference_loss
 from test_gpu_train_fp64 import attention_errors, attention_inputs, attention_ref, clas2_64, rel_err, small_batch, small_model
 
 pytestmark = pytest.mark.gpu
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 @pytest.fixture(scope="module")
@@ -129,64 +124,6 @@ def test_train_attention_matches_float64_with_torchs_mask(pkg, dh, B, H, T):
     assert max(errs.values()) <= 2e-5, errs
     wrong = attention_errors(got, attention_ref(qkv, dout, B, T, H, keep.transpose(2, 3)), T)
     assert wrong["out"] > 1e-2, wrong                      # non-vacuity: a transposed mask is far outside the bound
-
-
-_SIMT_SCRIPT = r"""
-import sys
-import numpy as np
-import torch
-sys.path.insert(0, sys.argv[1])
-from iefvad_b200 import ops
-z = np.load(sys.argv[2])
-res = {}
-for name in z.files:
-    if not name.startswith("qkv:"):
-        continue
-    case = name[4:]
-    B, T, H, _, pm, seed, off, G = (int(v) for v in case.split("_"))
-    qkv, dout = torch.from_numpy(z["qkv:" + case]).cuda(), torch.from_numpy(z["dout:" + case]).cuda()
-    kw = dict(rng="torch", offset=off, threads=G)
-    out, lse = ops.attention_train_fwd(qkv, B, T, H, pm / 1000, seed, **kw)
-    dqkv = ops.attention_train_bwd(qkv, out, dout, lse, B, T, H, pm / 1000, seed, **kw)
-    res["out:" + case], res["lse:" + case], res["dqkv:" + case] = out.cpu().numpy(), lse.cpu().numpy(), dqkv.cpu().numpy()
-try:                                  # head dim 128 exists only on the mma.sync path: refused here proves the SIMT path ran
-    ops.attention_train_fwd(torch.zeros(4, 3 * 128, device="cuda"), 1, 4, 1)
-    res["dh128_refused"] = np.array(0)
-except RuntimeError:
-    res["dh128_refused"] = np.array(1)
-np.savez(sys.argv[3], **res)
-"""
-
-
-def test_simt_train_attention_matches_float64_with_torchs_mask(pkg, tmp_path):
-    """The FFMA kernels of csrc/train.cu (IEFVAD_TRAIN_ATTN=simt, read once per process: a child process)."""
-    _, ops, _ = pkg
-    p, cases, data = 0.1, [], {}
-    for dh, B, H, T in ATTN_CASES:
-        qkv, dout = attention_inputs(B, T, H, dh, 11 * dh + T)
-        torch.cuda.manual_seed(3 * dh + T)
-        seed, off, keep = torch_keep(B, H, T, p)
-        G, _ = ops.torch_dropout_launch(B * H * T * T)
-        case = f"{B}_{T}_{H}_{dh}_{int(round(p * 1000))}_{seed}_{off}_{G}"
-        data[f"qkv:{case}"], data[f"dout:{case}"] = qkv.numpy(), dout.numpy()
-        cases.append((dh, B, H, T, qkv, dout, keep, case))
-    np.savez(tmp_path / "in.npz", **data)
-    env = dict(os.environ, IEFVAD_TRAIN_ATTN="simt")
-    cmd = [sys.executable] + (["-s"] if sys.flags.no_user_site else []) + [
-        "-c", _SIMT_SCRIPT, ROOT, str(tmp_path / "in.npz"), str(tmp_path / "out.npz")]
-    r = subprocess.run(cmd, env=env, cwd=ROOT, capture_output=True, text=True, timeout=300)
-    assert r.returncode == 0, r.stderr[-4000:]
-    z = np.load(tmp_path / "out.npz")
-    assert int(z["dh128_refused"]) == 1
-    worst = 0.0
-    for dh, B, H, T, qkv, dout, keep, case in cases:
-        D = H * dh
-        d = torch.from_numpy(z["dqkv:" + case])
-        got = (torch.from_numpy(z["out:" + case]), torch.from_numpy(z["lse:" + case]), d[:, :D], d[:, D:2 * D], d[:, 2 * D:])
-        errs = attention_errors(got, attention_ref(qkv, dout, B, T, H, keep), T)
-        worst = max(worst, max(errs.values()))
-        assert max(errs.values()) <= 2e-5, (dh, B, H, T, errs)
-    print("SIMT torch-mask attention worst error:", worst)
 
 
 # ------------------------------------------------------------------------------------------------ model vs stock torch

@@ -76,12 +76,16 @@ def test_new_entry_points_reject_bad_arguments_without_a_gpu():
     L = _lib.lib
     p = 1 << 20                                     # never read: every case fails its checks first
 
-    def call(fn, drop, B=2, H=4, T=48):
+    def call(fn, drop, B=2, H=4, T=48, dh=32):
         d = None if drop is None else ctypes.byref(drop)
         if fn == "fwd":
-            return L.iefvad_attention_train_fwd_dropout(p, B, T, H, 32, d, p, p, None)
+            return L.iefvad_attention_train_fwd_dropout(p, B, T, H, dh, d, p, p, None)
         if fn == "bwd":
-            return L.iefvad_attention_train_bwd_dropout(p, p, p, p, B, T, H, 32, d, p, None)
+            return L.iefvad_attention_train_bwd_dropout(p, p, p, p, B, T, H, dh, d, p, None)
+        if fn == "philox fwd":
+            return L.iefvad_attention_train_fwd(p, B, T, H, dh, 0.1, 3, p, p, None)
+        if fn == "philox bwd":
+            return L.iefvad_attention_train_bwd(p, p, p, p, B, T, H, dh, 0.1, 3, p, None)
         return L.iefvad_dropout_mask(d, B, H, T, p, None)
 
     torch_ok = dict(kind=1, p=0.1, seed=3, offset=8, threads=18432)
@@ -100,6 +104,12 @@ def test_new_entry_points_reject_bad_arguments_without_a_gpu():
             drop = None if change is None else _lib.Dropout(**{**torch_ok, **change})
             rc = call(fn, drop, **sizes)
             assert rc != 0 and word in _lib.last_error(), (fn, change, sizes, rc, _lib.last_error())
+    # sizes and head sizes the kernels are not built for, on both attention pairs (the philox pair takes no descriptor)
+    sized = [(dict(T=-1), "bad B / T"), (dict(H=0), "bad B / T"), (dict(dh=48), "head dim"), (dict(dh=0), "head dim")]
+    for fn in ("fwd", "bwd", "philox fwd", "philox bwd"):
+        for sizes, word in sized:
+            rc = call(fn, _lib.Dropout(**torch_ok), **sizes)
+            assert rc != 0 and word in _lib.last_error(), (fn, sizes, rc, _lib.last_error())
     # null tensors
     d = _lib.Dropout(**torch_ok)
     assert L.iefvad_attention_train_fwd_dropout(None, 2, 48, 4, 32, ctypes.byref(d), p, p, None) != 0
